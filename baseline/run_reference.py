@@ -18,7 +18,7 @@ pins them), so here ``available()`` is False and nothing below the guard has eve
 side is exercised through the same ``dump()`` with the oracle as the implementation (``OracleImpl``), which checks
 the file format and the consumer, not the reference.
 
-The reference is looked up in ``baseline/_ref`` (a pip --target install, git-ignored) and then ``/root/reference``.
+The reference is looked up in ``baseline/_ref`` (a pip --target install, git-ignored).
 """
 import importlib.util
 import os
@@ -28,7 +28,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DIRS = [os.path.join(ROOT, "baseline", "_ref"), "/root/reference"]
+REF_DIRS = [os.path.join(ROOT, "baseline", "_ref")]
 NEEDED = ("jax", "numpyro", "chacha")
 
 SEEDS = (0, 1, 123, (1 << 40) + 5)

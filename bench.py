@@ -11,7 +11,11 @@ A "step" = `get_batch(i, state)` (sampler kernels) followed by `DPSVI.update(sta
 mask=mask)` (fused gather / per-example gradient / clip / sum kernel(s) + (NCCL all-reduce at N > 1)
 + reduce / ChaCha noise / rescale / Adam kernel).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes, after the timed steps, what the headline path handed its caller after its last step
+(parameters, optimizer moments, state key, that step's loss and example count) as DIR/<name>.npy.  The data set and
+every key are derived from fixed seeds, so two builds run with the same arguments can be compared array by array.
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); the batch is sharded over the ranks
 (strong scaling: the global batch is fixed by the config).  `--impl reference` times the CPU
@@ -280,6 +284,36 @@ def make_family(cfg):
     return models.VAE(cfg["d"], cfg["hidden"], cfg["z"])
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def output_arrays(svi, state, loss, n_examples):
+    """Host copies of what a caller of DPSVI.update / run_epoch holds after a step: the constrained parameters, the
+    optimizer's moments, the state key (uint32 words, exact in float64), the step's loss and its example count."""
+    import re
+    import torch
+
+    def host(x):
+        a = x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
+        return a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    out = {"param_" + re.sub(r"[^0-9A-Za-z_]+", "_", k): host(v) for k, v in svi.get_params(state).items()}
+    os_ = state.optim_state
+    out.update({f"optim_{k}": host(v) for k, v in (("m", os_.m), ("v", os_.v)) if v is not None})
+    out["rng_key"] = host(state.rng_key)
+    out["loss"] = host(loss).reshape(1)
+    out["n_examples"] = host(n_examples).astype(np.float64).reshape(1)
+    return out
+
+
+def write_outputs(path, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 class LibEvents:
     """CUDA events owned by libd3p_b200 (recorded inside the C call around the dominant kernels)."""
 
@@ -444,6 +478,10 @@ def run_b200(args, cfg):
         if svi.peer_window is not None:
             svi.peer_window.check(synchronize=False)
 
+    # the headline is the C-side epoch driver where there is one for the family and collective (row f2 below), else the
+    # interpreter-driven loop
+    headline_epoch = cfg["family"] in ("logreg", "gauss", "vae") and (world == 1 or args.collective == "p2p")
+    outputs = None
     sync_all()        # ranks finish generating 41 GB of data at different times: align them before the first exchange
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -464,6 +502,8 @@ def run_b200(args, cfg):
         counts.append(nv)
     t_end.record()
     sync_all()
+    if args.dump_outputs and not headline_epoch:
+        outputs = output_arrays(svi, state, loss, counts[-1])
     svi.event_hook = None
     if args.ncu_child:      # profiled child of ncu_side_run: report which launch held how many examples, nothing else
         print(json.dumps({"per_step_examples": [int(c) if isinstance(c, int) else int(c.reshape(()).item()) for c in counts]}))
@@ -488,7 +528,7 @@ def run_b200(args, cfg):
 
     # ---- the same K steps through the C-side epoch driver (row f2): no interpreter between launches ----
     epoch_line = None
-    if cfg["family"] in ("logreg", "gauss", "vae") and (world == 1 or args.collective == "p2p"):
+    if headline_epoch:
         base = args.warmup + args.steps + 32
         state, _ = svi.run_epoch(state, get_batch, bstate, max(args.warmup, 3), first_step=base)
         sync_all()
@@ -497,6 +537,8 @@ def run_b200(args, cfg):
         state, ep_stats = svi.run_epoch(state, get_batch, bstate, args.steps, first_step=base + 8)
         p1.record()
         sync_all()
+        if args.dump_outputs:
+            outputs = output_arrays(svi, state, ep_stats[-1, 0], ep_stats[-1, 1])
         ep_ms = p0.elapsed_time(p1)
         if world > 1:
             t = torch.tensor([ep_ms], device=device)
@@ -668,6 +710,8 @@ def run_b200(args, cfg):
             v, ms, desc = cpu_run(args.workload, cfg, 4, 1, threads)
             line["cpu_baseline"] = {"value": v, "unit": "examples/s", "cores": threads, "kind": "port",
                                     "sample": "4 steps: " + desc}
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -691,7 +735,13 @@ def main():
     ap.add_argument("--ncu-child", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-other-workloads", dest="other_workloads", action="store_false",
                     help="default (c2, N = 1) run only: skip the short c3 / c5 runs reported under `workloads`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 path computed: use it with --impl b200")
     args.warmup = max(args.warmup, 3)
     cfg = dict(WORKLOADS[args.workload])
     if args.rows:

@@ -1,6 +1,6 @@
 """Writes tests/golden/reference_v1.npz from the REAL reference (d3p + jax + numpyro + jax-chacha-prng):
 
-    python tests/golden/make_reference_golden.py            # needs the packages of /root/reference/setup.py:46-49
+    python tests/golden/make_reference_golden.py            # needs the packages pinned by the reference's setup.py:46-49
 
 The vectors (baseline/run_reference.py:dump) pin what the reference's own tests leave open (SURVEY.md section 8c):
 the key-derivation rule of jax-chacha-prng, keystream word order, uniform / normal / randint transforms, Feistel and
