@@ -10,12 +10,9 @@
 // step i + 1 is queued on a second (forked) stream and runs while step i's gradient kernel drains and its finalize
 // kernel (latency-bound, a few CTAs; at N > 1 it also waits for the peers) holds the main stream.  idx / counts /
 // mask are double-buffered; events order sampler(i) -> step(i) and step(i) -> sampler(i + 2).
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <new>
-#include <vector>
 
 #include "comm.cuh"
 #include "common.cuh"
@@ -119,7 +116,7 @@ namespace {
 // a context for the duration of one call when the caller passed none
 struct CtxGuard {
   d3p_epoch_ctx* ctx; bool own = false;
-  explicit CtxGuard(d3p_epoch_ctx* c, bool needed = true) : ctx(c) {
+  CtxGuard(d3p_epoch_ctx* c, bool needed) : ctx(c) {
     if (!ctx && needed) own = d3p_epoch_ctx_create(&ctx) == D3P_OK;
   }
   ~CtxGuard() { if (own) d3p_epoch_ctx_destroy(ctx); }
@@ -128,81 +125,203 @@ struct CtxGuard {
 // rows of the batch handled by one rank of `world` (contiguous position ranges, the last one may be shorter)
 uint32_t rows_per_rank(uint32_t B, int world) { return world > 1 ? (B + (uint32_t)world - 1) / (uint32_t)world : B; }
 
-// The family-specific part of a step: launches the fused per-example-gradient / clip / sum kernels of batch positions
-// [pos_begin, pos_end) into the partial rows at `ws`.
+// The family-specific part of a step: the size of its workspace, and the launch of the fused per-example-gradient /
+// clip / sum kernels of batch positions [pos_begin, pos_end) into the partial rows at `ws`.
 struct StepLauncher {
-  size_t step_bytes;      // workspace of one step (partial rows first)
-  uint32_t n_part, P;
-  // tf_h: Threefry key on the host, or nullptr and tf_d: the key in device memory
+  const float* x; size_t stride; float* params; uint32_t P;
+  bool vae = false;       // the VAE step: side streams of a d3p_vae_ctx, a 256-byte aligned workspace
+  StepLauncher(const float* x, size_t stride, float* params, uint32_t P) : x(x), stride(stride), params(params), P(P) {}
+  // workspace of one step for `rows` batch rows per rank (partial rows first); 0 = unsupported description
+  virtual size_t workspace(uint32_t rows, uint32_t* n_part) const = 0;
+  // (tf_h, tf_d): the Threefry key of the step on the host or in device memory, one of them non-null
   virtual int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
-                         const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws,
-                         cudaStream_t s) const = 0;
+                         const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, size_t ws_bytes,
+                         d3p_vae_ctx* vae_ctx, cudaStream_t s) const = 0;
   virtual ~StepLauncher() {}
 };
 
-// keys: host words (batch_key_h, rng_key_io_h) or, for the *_dk entry points, device words (batch_key_d, rng_key_io_d)
+struct MeanfieldLauncher : StepLauncher {
+  const d3p_meanfield_desc* desc; const int32_t* y;
+  explicit MeanfieldLauncher(const d3p_meanfield_desc* d, const float* x = nullptr, size_t stride = 0,
+                             const int32_t* y = nullptr, float* params = nullptr)
+      : StepLauncher(x, stride, params, d->n_params), desc(d), y(y) {}
+  size_t workspace(uint32_t, uint32_t* n_part) const override { return d3p_meanfield_workspace_bytes(desc, n_part); }
+  int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
+                 const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, size_t ws_bytes,
+                 d3p_vae_ctx*, cudaStream_t s) const override {
+    return step_meanfield_impl(desc, params, x, stride, y, idx, mask, nullptr, B, pos_begin, pos_end, tf_h, tf_d, obs_scale,
+                               C, nullptr, nullptr, nullptr, ws, ws_bytes, s);
+  }
+};
+struct GmmLauncher : StepLauncher {
+  const d3p_gmm_desc* desc;
+  explicit GmmLauncher(const d3p_gmm_desc* d, const float* x = nullptr, size_t stride = 0, float* params = nullptr)
+      : StepLauncher(x, stride, params, d->n_params), desc(d) {}
+  size_t workspace(uint32_t, uint32_t* n_part) const override { return d3p_gmm_workspace_bytes(desc, n_part); }
+  int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
+                 const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, size_t ws_bytes,
+                 d3p_vae_ctx*, cudaStream_t s) const override {
+    return step_gmm_impl(desc, params, x, stride, idx, mask, nullptr, B, pos_begin, pos_end, tf_h, tf_d, obs_scale, C,
+                         nullptr, nullptr, nullptr, ws, ws_bytes, s);
+  }
+};
+struct VaeLauncher : StepLauncher {
+  const d3p_vae_desc* desc;
+  explicit VaeLauncher(const d3p_vae_desc* d, const float* x = nullptr, size_t stride = 0, float* params = nullptr)
+      : StepLauncher(x, stride, params, d->n_params), desc(d) { vae = true; }
+  size_t workspace(uint32_t rows, uint32_t* n_part) const override { return d3p_vae_workspace_bytes(desc, rows, n_part); }
+  int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
+                 const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, size_t ws_bytes,
+                 d3p_vae_ctx* vae_ctx, cudaStream_t s) const override {
+    return step_vae_impl(desc, params, x, stride, idx, mask, nullptr, B, pos_begin, pos_end, tf_h, tf_d, obs_scale, C,
+                         nullptr, nullptr, ws, ws_bytes, nullptr, vae_ctx, s);
+  }
+};
+
+size_t epoch_ws_bytes(const StepLauncher& fam, const d3p_sampler_desc* sampler, int32_t world) {
+  EpochWs w;
+  uint32_t n_part = 0;
+  if (!sampler_ok(sampler) || world < 1 ||
+      !layout_ws(fam.workspace(rows_per_rank(sampler->batch, world), &n_part), sampler, nullptr, w))
+    return 0;
+  return w.total;
+}
+
+// The set-up and loop shared by the d3p_dpsvi_run_epoch_* entry points.  Keys: host words (batch_key_h, rng_key_io_h)
+// or, for the *_dk entry points, device words (batch_key_d, rng_key_io_d).
 int32_t run_epoch(const StepLauncher& fam, const d3p_sampler_desc* sampler, const uint32_t* batch_key_h,
                   uint32_t* rng_key_io_h, const uint32_t* batch_key_d, uint32_t* rng_key_io_d, uint32_t first_step,
-                  uint32_t n_steps, float obs_scale, float C,
-                  float dp_scale, const d3p_leaf_table* leaves_h, d3p_optim_desc* optim_io_h, float* params_d, float* m_d,
-                  float* v_d, float* stats_out_d, d3p_comm* comm, void* ws_d, size_t ws_bytes, d3p_epoch_ctx* ctx,
-                  void* stream);
+                  uint32_t n_steps, float obs_scale, float C, float dp_scale, const d3p_leaf_table* leaves_h,
+                  d3p_optim_desc* optim_io_h, float* m_d, float* v_d, float* stats_out_d, d3p_comm* comm, void* ws_d,
+                  size_t ws_bytes, d3p_epoch_ctx* ctx, void* stream) {
+  const bool dk = rng_key_io_d != nullptr;           // keys in device memory
+  const bool split = sampler && sampler->kind == D3P_SAMPLER_SPLIT;      // pre-shuffled epoch: no sampler, no batch key
+  if (!fam.x || !fam.params || (dk ? !batch_key_d : ((!split && !batch_key_h) || !rng_key_io_h)) || !leaves_h ||
+      !optim_io_h || !ws_d)
+    return D3P_ERR_INVALID_ARGUMENT;
+  if (fam.vae && (reinterpret_cast<uintptr_t>(ws_d) & 255)) return D3P_ERR_INVALID_ARGUMENT;
+  if (split && (uint64_t)(first_step + n_steps) * sampler->batch > sampler->n_records) return D3P_ERR_INVALID_ARGUMENT;
+  if (!sampler_ok(sampler) || leaves_h->n_leaves == 0 || leaves_h->n_leaves > D3P_MAX_LEAVES)
+    return D3P_ERR_INVALID_ARGUMENT;
+  EpochWs w;
+  uint32_t n_part = 0;
+  if (!layout_ws(fam.workspace(rows_per_rank(sampler->batch, comm ? comm->world : 1), &n_part), sampler, ws_d, w))
+    return D3P_ERR_UNSUPPORTED;
+  if (ws_bytes < w.total) return D3P_ERR_WORKSPACE;
+  const uint32_t B = sampler->batch, P = fam.P;
+
+  d3p_leaf_table lt = *leaves_h;
+  // sharded batch (SURVEY 8e): this rank handles a contiguous range of batch positions; the sampler and
+  // all key derivations are replicated, the clipped sums meet inside the finalize kernel (comm.cuh)
+  uint32_t pos_begin = 0, pos_end = B;
+  if (comm && comm->world > 1) {
+    const uint32_t per = (B + comm->world - 1) / comm->world;
+    pos_begin = per * comm->rank < B ? per * comm->rank : B;
+    pos_end = pos_begin + per < B ? pos_begin + per : B;
+  }
+  const bool fork = n_steps > 1 && !split;
+  cudaStream_t main_s = (cudaStream_t)stream, samp_s = main_s;
+  cudaEvent_t ev_sampled[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr}, ev_fork = nullptr;
+  CtxGuard guard(ctx, fork || fam.vae);          // a context only for the sampler stream or the VAE's side streams
+  if ((fork || fam.vae) && !guard.ctx) return D3P_ERR_CUDA;
+  if (fam.vae && !guard.ctx->vae && d3p_vae_ctx_create(&guard.ctx->vae) != D3P_OK) return D3P_ERR_CUDA;
+  d3p_vae_ctx* const vae_ctx = fam.vae ? guard.ctx->vae : nullptr;
+  if (fork) {
+    samp_s = guard.ctx->samp;
+    ev_fork = guard.ctx->ev_fork;
+    for (int b = 0; b < 2; ++b) { ev_sampled[b] = guard.ctx->ev_sampled[b]; ev_consumed[b] = guard.ctx->ev_consumed[b]; }
+    // the sampler stream starts after everything already queued on the caller's stream
+    if (cudaEventRecord(ev_fork, main_s) != cudaSuccess || cudaStreamWaitEvent(samp_s, ev_fork, 0) != cudaSuccess)
+      return D3P_ERR_CUDA;
+  }
+  // get_batch(i, batchifier_state): fold_in, then the index sampler (minibatch.py:103-131,217-237), into buffer i & 1
+  auto queue_sampler = [&](uint32_t s) -> int32_t {
+    const int b = s & 1;
+    const bool poisson = sampler->kind == D3P_SAMPLER_POISSON;
+    uint32_t bkey[16], rcs[30];
+    int32_t r = D3P_OK;
+    if (!dk && (r = d3p_chacha_fold_in_h(batch_key_h, first_step + s, bkey)) != D3P_OK) return r;
+    if (fork && s >= 2 && cudaStreamWaitEvent(samp_s, ev_consumed[b], 0) != cudaSuccess) return D3P_ERR_CUDA;
+    if (dk) {
+      // the same keys made by one-block kernels, into the buffers of parity b (free once step s - 2 has consumed them)
+      if ((r = d3p_chacha_fold_in_dk(batch_key_d, nullptr, first_step + s, w.bkey[b], samp_s)) != D3P_OK) return r;
+      if (!poisson && (r = d3p_feistel_round_constants_dk(w.bkey[b], w.rc[b], samp_s)) != D3P_OK) return r;
+    } else if (!poisson && (r = d3p_feistel_round_constants_h(bkey, rcs)) != D3P_OK) {
+      return r;
+    }
+    const uint32_t* key_h = dk ? nullptr : bkey;
+    const uint32_t* key_d = dk ? w.bkey[b] : nullptr;
+    if (poisson) {
+      r = D3P_ERR_UNSUPPORTED;
+      if (comm && comm->world > 1)             // selector draw split over the ranks (samplers.cu)
+        r = poisson_sample_sharded_impl(comm, key_h, key_d, sampler->q, sampler->n_records, B, sampler->suppress,
+                                        pos_begin, pos_end, w.idx[b], w.counts[b], w.mask[b], w.poisson, w.poisson_bytes,
+                                        samp_s);
+      if (r == D3P_ERR_UNSUPPORTED)            // same decision on every rank (window size, tiles >= ranks)
+        r = poisson_sample_impl(key_h, key_d, sampler->q, sampler->n_records, B, sampler->suppress, w.idx[b], w.counts[b],
+                                w.mask[b], w.poisson, w.poisson_bytes, samp_s);
+    } else {
+      r = feistel_sample_impl(dk ? nullptr : rcs, dk ? w.rc[b] : nullptr, sampler->n_records, 0, B, w.idx[b], samp_s);
+    }
+    if (r == D3P_OK && fork && cudaEventRecord(ev_sampled[b], samp_s) != cudaSuccess) r = D3P_ERR_CUDA;
+    return r;
+  };
+  int32_t rc = D3P_OK;
+  if (fork) rc = queue_sampler(0);
+  for (uint32_t s = 0; s < n_steps && rc == D3P_OK; ++s) {
+    const int b = s & 1;
+    if (split) {
+      // nothing to sample: this step's records are a slice of the epoch's shuffle
+    } else if (fork) {
+      if (s + 1 < n_steps && (rc = queue_sampler(s + 1)) != D3P_OK) break;      // runs ahead on the sampler stream
+      if (cudaStreamWaitEvent(main_s, ev_sampled[b], 0) != cudaSuccess) { rc = D3P_ERR_CUDA; break; }
+    } else if ((rc = queue_sampler(s)) != D3P_OK) {
+      break;
+    }
+    const uint8_t* mask = sampler->kind == D3P_SAMPLER_POISSON ? w.mask[b] : nullptr;
+    const int32_t* idx = split ? sampler->perm_d + (size_t)(first_step + s) * B : w.idx[b];
+    // ---- DPSVI.update (svi.py:395-434) ----------------------------------------------------------------------
+    // carry / k_grad -> Threefry key / k_noise -> per-leaf keys: in host C, or all on the device with the state key
+    // advanced in place
+    uint32_t keys[3][16], tf[2];
+    if (dk) {
+      if ((rc = d3p_dpsvi_keys_dk(rng_key_io_d, lt.n_leaves, w.tf, w.sites, main_s)) != D3P_OK) break;
+    } else {
+      if ((rc = d3p_chacha_split_h(rng_key_io_h, 3, &keys[0][0])) != D3P_OK) break;           // carry, k_grad, k_noise
+      if ((rc = d3p_chacha_random_bits_h(keys[1], 0, tf, 2)) != D3P_OK) break;                // convert_to_jax_rng_key
+    }
+    rc = fam.launch(idx, mask, B, pos_begin, pos_end, dk ? nullptr : tf, dk ? w.tf : nullptr, obs_scale, C, w.step,
+                    w.step_bytes, vae_ctx, main_s);
+    if (rc != D3P_OK) break;
+    if (!dk && (rc = d3p_chacha_split_h(keys[2], (int32_t)lt.n_leaves, &lt.site_state[0][0])) != D3P_OK) break;
+    rc = perturb_finalize_impl(w.step, n_part, P, B, &lt, dk ? w.sites : nullptr, dp_scale, C, obs_scale, 1, nullptr,
+                               optim_io_h, fam.params, m_d, v_d, stats_out_d ? stats_out_d + 3 * (size_t)s : nullptr,
+                               nullptr, comm, main_s);
+    if (rc != D3P_OK) break;
+    // recorded after the finalize launch so that nothing sits between the step kernel and its programmatic dependent
+    if (fork && cudaEventRecord(ev_consumed[b], main_s) != cudaSuccess) { rc = D3P_ERR_CUDA; break; }
+    if (optim_io_h->kind == D3P_OPT_ADADP && (optim_io_h->step & 1))
+      if ((rc = d3p_adadp_finish_f32(optim_io_h, P, fam.params, v_d, main_s)) != D3P_OK) break;
+    optim_io_h->step += 1;
+    if (!dk) memcpy(rng_key_io_h, keys[0], sizeof(keys[0]));
+  }
+  if (fork) {
+    // join: whatever is still queued on the sampler stream (only after an error) precedes later work of the caller
+    if (cudaEventRecord(ev_fork, samp_s) == cudaSuccess) cudaStreamWaitEvent(main_s, ev_fork, 0);
+  }
+  return rc;
+}
 
 }  // namespace
 
 extern "C" size_t d3p_dpsvi_epoch_workspace_bytes(const d3p_meanfield_desc* desc, const d3p_sampler_desc* sampler) {
-  EpochWs w;
-  uint32_t n_part = 0;
-  if (!desc || !sampler_ok(sampler) || !layout_ws(d3p_meanfield_workspace_bytes(desc, &n_part), sampler, nullptr, w)) return 0;
-  return w.total;
+  return desc ? epoch_ws_bytes(MeanfieldLauncher(desc), sampler, 1) : 0;
 }
 
 extern "C" size_t d3p_dpsvi_epoch_vae_workspace_bytes(const d3p_vae_desc* desc, const d3p_sampler_desc* sampler,
                                                       int32_t world) {
-  EpochWs w;
-  if (!desc || !sampler_ok(sampler) || world < 1) return 0;
-  if (!layout_ws(d3p_vae_workspace_bytes(desc, rows_per_rank(sampler->batch, world), nullptr), sampler, nullptr, w)) return 0;
-  return w.total;
+  return desc ? epoch_ws_bytes(VaeLauncher(desc), sampler, world) : 0;
 }
-
-namespace {
-struct MeanfieldLauncher : StepLauncher {
-  const d3p_meanfield_desc* desc; const float* x; size_t stride; const int32_t* y;
-  int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
-                 const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, cudaStream_t s) const override {
-    if (tf_h)
-      return d3p_dpsvi_step_meanfield(desc, params, x, stride, y, idx, mask, nullptr, B, pos_begin, pos_end, tf_h, obs_scale,
-                                      C, nullptr, nullptr, nullptr, ws, step_bytes, s);
-    return d3p_dpsvi_step_meanfield_dk(desc, params, x, stride, y, idx, mask, nullptr, B, pos_begin, pos_end, tf_d, obs_scale,
-                                       C, nullptr, nullptr, nullptr, ws, step_bytes, s);
-  }
-  const float* params;
-};
-struct GmmLauncher : StepLauncher {
-  const d3p_gmm_desc* desc; const float* x; size_t stride; const float* params;
-  int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
-                 const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, cudaStream_t s) const override {
-    if (tf_h)
-      return d3p_dpsvi_step_gmm(desc, params, x, stride, idx, mask, nullptr, B, pos_begin, pos_end, tf_h, obs_scale, C,
-                                nullptr, nullptr, nullptr, ws, step_bytes, s);
-    return d3p_dpsvi_step_gmm_dk(desc, params, x, stride, idx, mask, nullptr, B, pos_begin, pos_end, tf_d, obs_scale, C,
-                                 nullptr, nullptr, nullptr, ws, step_bytes, s);
-  }
-};
-struct VaeLauncher : StepLauncher {
-  const d3p_vae_desc* desc; const float* x; size_t stride; const float* params;
-  d3p_vae_ctx* ctx = nullptr;      // side streams of the step: owned by the d3p_epoch_ctx
-  int32_t launch(const int32_t* idx, const uint8_t* mask, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
-                 const uint32_t* tf_h, const uint32_t* tf_d, float obs_scale, float C, void* ws, cudaStream_t s) const override {
-    if (tf_h)
-      return d3p_dpsvi_step_vae(desc, params, x, stride, idx, mask, nullptr, B, pos_begin, pos_end, tf_h, obs_scale, C,
-                                nullptr, nullptr, ws, step_bytes, nullptr, ctx, s);
-    return d3p_dpsvi_step_vae_dk(desc, params, x, stride, idx, mask, nullptr, B, pos_begin, pos_end, tf_d, obs_scale, C,
-                                 nullptr, nullptr, ws, step_bytes, nullptr, ctx, s);
-  }
-};
-}  // namespace
-
 
 extern "C" int32_t d3p_dpsvi_run_epoch_meanfield(const d3p_meanfield_desc* desc, const d3p_sampler_desc* sampler,
                                                  const float* x_d, size_t x_row_stride, const int32_t* y_d,
@@ -212,13 +331,10 @@ extern "C" int32_t d3p_dpsvi_run_epoch_meanfield(const d3p_meanfield_desc* desc,
                                                  d3p_optim_desc* optim_io_h, float* params_d, float* m_d, float* v_d,
                                                  float* stats_out_d, d3p_comm* comm, void* ws_d, size_t ws_bytes,
                                                  d3p_epoch_ctx* ctx, void* stream) {
-  if (!desc || !x_d || !params_d) return D3P_ERR_INVALID_ARGUMENT;
-  MeanfieldLauncher fam;
-  fam.desc = desc; fam.x = x_d; fam.stride = x_row_stride; fam.y = y_d; fam.params = params_d;
-  fam.step_bytes = d3p_meanfield_workspace_bytes(desc, &fam.n_part);
-  fam.P = desc->n_params;
-  return run_epoch(fam, sampler, batch_key_h, rng_key_io_h, nullptr, nullptr, first_step, n_steps, obs_scale, C, dp_scale,
-                   leaves_h, optim_io_h, params_d, m_d, v_d, stats_out_d, comm, ws_d, ws_bytes, ctx, stream);
+  if (!desc) return D3P_ERR_INVALID_ARGUMENT;
+  return run_epoch(MeanfieldLauncher(desc, x_d, x_row_stride, y_d, params_d), sampler, batch_key_h, rng_key_io_h, nullptr,
+                   nullptr, first_step, n_steps, obs_scale, C, dp_scale, leaves_h, optim_io_h, m_d, v_d, stats_out_d, comm,
+                   ws_d, ws_bytes, ctx, stream);
 }
 
 // Device-key form: the batchifier key and the DPSVI state key live in device memory (rng_key_io_d is advanced in place),
@@ -232,21 +348,15 @@ extern "C" int32_t d3p_dpsvi_run_epoch_meanfield_dk(const d3p_meanfield_desc* de
                                                     d3p_optim_desc* optim_io_h, float* params_d, float* m_d, float* v_d,
                                                     float* stats_out_d, d3p_comm* comm, void* ws_d, size_t ws_bytes,
                                                     d3p_epoch_ctx* ctx, void* stream) {
-  if (!desc || !x_d || !params_d || !batch_key_d || !rng_key_io_d) return D3P_ERR_INVALID_ARGUMENT;
-  MeanfieldLauncher fam;
-  fam.desc = desc; fam.x = x_d; fam.stride = x_row_stride; fam.y = y_d; fam.params = params_d;
-  fam.step_bytes = d3p_meanfield_workspace_bytes(desc, &fam.n_part);
-  fam.P = desc->n_params;
-  return run_epoch(fam, sampler, nullptr, nullptr, batch_key_d, rng_key_io_d, first_step, n_steps, obs_scale, C, dp_scale,
-                   leaves_h, optim_io_h, params_d, m_d, v_d, stats_out_d, comm, ws_d, ws_bytes, ctx, stream);
+  if (!desc) return D3P_ERR_INVALID_ARGUMENT;
+  return run_epoch(MeanfieldLauncher(desc, x_d, x_row_stride, y_d, params_d), sampler, nullptr, nullptr, batch_key_d,
+                   rng_key_io_d, first_step, n_steps, obs_scale, C, dp_scale, leaves_h, optim_io_h, m_d, v_d, stats_out_d,
+                   comm, ws_d, ws_bytes, ctx, stream);
 }
 
 // The same loop for the mixture model (examples/gaussian_mixture_model.py:205-218).
 extern "C" size_t d3p_dpsvi_epoch_gmm_workspace_bytes(const d3p_gmm_desc* desc, const d3p_sampler_desc* sampler) {
-  EpochWs w;
-  uint32_t n_part = 0;
-  if (!desc || !sampler_ok(sampler) || !layout_ws(d3p_gmm_workspace_bytes(desc, &n_part), sampler, nullptr, w)) return 0;
-  return w.total;
+  return desc ? epoch_ws_bytes(GmmLauncher(desc), sampler, 1) : 0;
 }
 
 extern "C" int32_t d3p_dpsvi_run_epoch_gmm(const d3p_gmm_desc* desc, const d3p_sampler_desc* sampler, const float* x_d,
@@ -256,13 +366,10 @@ extern "C" int32_t d3p_dpsvi_run_epoch_gmm(const d3p_gmm_desc* desc, const d3p_s
                                            d3p_optim_desc* optim_io_h, float* params_d, float* m_d, float* v_d,
                                            float* stats_out_d, d3p_comm* comm, void* ws_d, size_t ws_bytes, d3p_epoch_ctx* ctx,
                                            void* stream) {
-  if (!desc || !x_d || !params_d) return D3P_ERR_INVALID_ARGUMENT;
-  GmmLauncher fam;
-  fam.desc = desc; fam.x = x_d; fam.stride = x_row_stride; fam.params = params_d;
-  fam.step_bytes = d3p_gmm_workspace_bytes(desc, &fam.n_part);
-  fam.P = desc->n_params;
-  return run_epoch(fam, sampler, batch_key_h, rng_key_io_h, nullptr, nullptr, first_step, n_steps, obs_scale, C, dp_scale,
-                   leaves_h, optim_io_h, params_d, m_d, v_d, stats_out_d, comm, ws_d, ws_bytes, ctx, stream);
+  if (!desc) return D3P_ERR_INVALID_ARGUMENT;
+  return run_epoch(GmmLauncher(desc, x_d, x_row_stride, params_d), sampler, batch_key_h, rng_key_io_h, nullptr, nullptr,
+                   first_step, n_steps, obs_scale, C, dp_scale, leaves_h, optim_io_h, m_d, v_d, stats_out_d, comm, ws_d,
+                   ws_bytes, ctx, stream);
 }
 
 // The same loop for the VAE family (examples/vae.py:216-233 runs fori_loop(get_batch -> update) per epoch).
@@ -273,18 +380,10 @@ extern "C" int32_t d3p_dpsvi_run_epoch_vae(const d3p_vae_desc* desc, const d3p_s
                                            d3p_optim_desc* optim_io_h, float* params_d, float* m_d, float* v_d,
                                            float* stats_out_d, d3p_comm* comm, void* ws_d, size_t ws_bytes, d3p_epoch_ctx* ctx,
                                            void* stream) {
-  if (!desc || !x_d || !params_d || !sampler_ok(sampler)) return D3P_ERR_INVALID_ARGUMENT;
-  if (reinterpret_cast<uintptr_t>(ws_d) & 255) return D3P_ERR_INVALID_ARGUMENT;   // the VAE step wants 256-byte alignment
-  VaeLauncher fam;
-  fam.desc = desc; fam.x = x_d; fam.stride = x_row_stride; fam.params = params_d;
-  fam.step_bytes = d3p_vae_workspace_bytes(desc, rows_per_rank(sampler->batch, comm ? comm->world : 1), &fam.n_part);
-  fam.P = desc->n_params;
-  CtxGuard g(ctx);
-  if (!g.ctx || (!g.ctx->vae && d3p_vae_ctx_create(&g.ctx->vae) != D3P_OK)) return D3P_ERR_CUDA;
-  fam.ctx = g.ctx->vae;
-  ctx = g.ctx;
-  return run_epoch(fam, sampler, batch_key_h, rng_key_io_h, nullptr, nullptr, first_step, n_steps, obs_scale, C, dp_scale,
-                   leaves_h, optim_io_h, params_d, m_d, v_d, stats_out_d, comm, ws_d, ws_bytes, ctx, stream);
+  if (!desc) return D3P_ERR_INVALID_ARGUMENT;
+  return run_epoch(VaeLauncher(desc, x_d, x_row_stride, params_d), sampler, batch_key_h, rng_key_io_h, nullptr, nullptr,
+                   first_step, n_steps, obs_scale, C, dp_scale, leaves_h, optim_io_h, m_d, v_d, stats_out_d, comm, ws_d,
+                   ws_bytes, ctx, stream);
 }
 
 extern "C" int32_t d3p_dpsvi_run_epoch_vae_dk(const d3p_vae_desc* desc, const d3p_sampler_desc* sampler, const float* x_d,
@@ -292,181 +391,9 @@ extern "C" int32_t d3p_dpsvi_run_epoch_vae_dk(const d3p_vae_desc* desc, const d3
                                               uint32_t first_step, uint32_t n_steps, float obs_scale, float C,
                                               float dp_scale, const d3p_leaf_table* leaves_h, d3p_optim_desc* optim_io_h,
                                               float* params_d, float* m_d, float* v_d, float* stats_out_d, d3p_comm* comm,
-                                              void* ws_d, size_t ws_bytes, d3p_epoch_ctx* ctx,
-                                           void* stream) {
-  if (!desc || !x_d || !params_d || !sampler_ok(sampler) || !batch_key_d || !rng_key_io_d) return D3P_ERR_INVALID_ARGUMENT;
-  if (reinterpret_cast<uintptr_t>(ws_d) & 255) return D3P_ERR_INVALID_ARGUMENT;
-  VaeLauncher fam;
-  fam.desc = desc; fam.x = x_d; fam.stride = x_row_stride; fam.params = params_d;
-  fam.step_bytes = d3p_vae_workspace_bytes(desc, rows_per_rank(sampler->batch, comm ? comm->world : 1), &fam.n_part);
-  fam.P = desc->n_params;
-  CtxGuard g(ctx);
-  if (!g.ctx || (!g.ctx->vae && d3p_vae_ctx_create(&g.ctx->vae) != D3P_OK)) return D3P_ERR_CUDA;
-  fam.ctx = g.ctx->vae;
-  ctx = g.ctx;
-  return run_epoch(fam, sampler, nullptr, nullptr, batch_key_d, rng_key_io_d, first_step, n_steps, obs_scale, C, dp_scale,
-                   leaves_h, optim_io_h, params_d, m_d, v_d, stats_out_d, comm, ws_d, ws_bytes, ctx, stream);
+                                              void* ws_d, size_t ws_bytes, d3p_epoch_ctx* ctx, void* stream) {
+  if (!desc) return D3P_ERR_INVALID_ARGUMENT;
+  return run_epoch(VaeLauncher(desc, x_d, x_row_stride, params_d), sampler, nullptr, nullptr, batch_key_d, rng_key_io_d,
+                   first_step, n_steps, obs_scale, C, dp_scale, leaves_h, optim_io_h, m_d, v_d, stats_out_d, comm, ws_d,
+                   ws_bytes, ctx, stream);
 }
-
-namespace {
-int32_t run_epoch(const StepLauncher& fam, const d3p_sampler_desc* sampler, const uint32_t* batch_key_h,
-                  uint32_t* rng_key_io_h, const uint32_t* batch_key_d, uint32_t* rng_key_io_d, uint32_t first_step,
-                  uint32_t n_steps, float obs_scale, float C,
-                  float dp_scale, const d3p_leaf_table* leaves_h, d3p_optim_desc* optim_io_h, float* params_d, float* m_d,
-                  float* v_d, float* stats_out_d, d3p_comm* comm, void* ws_d, size_t ws_bytes, d3p_epoch_ctx* ctx,
-                  void* stream) {
-  const bool dk = rng_key_io_d != nullptr;           // keys in device memory
-  const bool split = sampler && sampler->kind == D3P_SAMPLER_SPLIT;      // pre-shuffled epoch: no sampler, no batch key
-  if ((dk ? (!split && !batch_key_d) : ((!split && !batch_key_h) || !rng_key_io_h)) || !leaves_h || !optim_io_h ||
-      !params_d || !ws_d)
-    return D3P_ERR_INVALID_ARGUMENT;
-  if (split && (uint64_t)(first_step + n_steps) * sampler->batch > sampler->n_records) return D3P_ERR_INVALID_ARGUMENT;
-  if (!sampler_ok(sampler) || leaves_h->n_leaves == 0 || leaves_h->n_leaves > D3P_MAX_LEAVES)
-    return D3P_ERR_INVALID_ARGUMENT;
-  EpochWs w;
-  if (!layout_ws(fam.step_bytes, sampler, ws_d, w)) return D3P_ERR_UNSUPPORTED;
-  if (ws_bytes < w.total) return D3P_ERR_WORKSPACE;
-  const uint32_t B = sampler->batch, P = fam.P;
-  const uint32_t n_part = fam.n_part;
-
-  d3p_leaf_table lt = *leaves_h;
-  // sharded batch (SURVEY 8e): this rank handles a contiguous range of batch positions; the sampler and
-  // all key derivations are replicated, the clipped sums meet inside the finalize kernel (comm.cuh)
-  uint32_t pos_begin = 0, pos_end = B;
-  if (comm && comm->world > 1) {
-    const uint32_t per = (B + comm->world - 1) / comm->world;
-    pos_begin = per * comm->rank < B ? per * comm->rank : B;
-    pos_end = pos_begin + per < B ? pos_begin + per : B;
-  }
-  // D3P_EPOCH_PROFILE=1: per-phase CUDA-event timings of this call on stderr (synchronises at the end; the
-  // sampler then stays on the main stream so that the three phases are disjoint in time)
-#ifdef D3P_DEV_SWITCHES      // development builds only (D3P_NVCC_DEFINES=D3P_DEV_SWITCHES): the product reads no environment
-  const bool prof = getenv("D3P_EPOCH_PROFILE") != nullptr;
-  const bool fork = !prof && getenv("D3P_EPOCH_SERIAL") == nullptr && n_steps > 1;
-#else
-  const bool prof = false;
-  const bool fork = n_steps > 1 && !split;
-#endif
-  cudaStream_t main_s = (cudaStream_t)stream, samp_s = main_s;
-  cudaEvent_t ev_sampled[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr}, ev_fork = nullptr;
-  CtxGuard guard(ctx, fork);          // no context needed without the fork
-  if (fork) {
-    if (!guard.ctx) return D3P_ERR_CUDA;
-    samp_s = guard.ctx->samp;
-    ev_fork = guard.ctx->ev_fork;
-    for (int b = 0; b < 2; ++b) { ev_sampled[b] = guard.ctx->ev_sampled[b]; ev_consumed[b] = guard.ctx->ev_consumed[b]; }
-    // the sampler stream starts after everything already queued on the caller's stream
-    if (cudaEventRecord(ev_fork, main_s) != cudaSuccess || cudaStreamWaitEvent(samp_s, ev_fork, 0) != cudaSuccess)
-      return D3P_ERR_CUDA;
-  }
-  std::vector<cudaEvent_t> ev;
-  auto mark = [&]() {
-    if (!prof) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, main_s);
-    ev.push_back(e);
-  };
-  // get_batch(i, batchifier_state): fold_in, then the index sampler (minibatch.py:103-131,217-237), into buffer i & 1
-  auto queue_sampler = [&](uint32_t s) -> int32_t {
-    const int b = s & 1;
-    uint32_t bkey[16];
-    int32_t r = D3P_OK;
-    if (!dk && (r = d3p_chacha_fold_in_h(batch_key_h, first_step + s, bkey)) != D3P_OK) return r;
-    if (fork && s >= 2 && cudaStreamWaitEvent(samp_s, ev_consumed[b], 0) != cudaSuccess) return D3P_ERR_CUDA;
-    if (dk) {
-      // the same get_batch with the key derived on the device (buffers of parity b: free once step s - 2 has consumed them)
-      if ((r = d3p_chacha_fold_in_dk(batch_key_d, nullptr, first_step + s, w.bkey[b], samp_s)) != D3P_OK) return r;
-      if (sampler->kind == D3P_SAMPLER_POISSON) {
-        r = D3P_ERR_UNSUPPORTED;
-        if (comm && comm->world > 1)
-          r = d3p_poisson_sample_sharded_dk(comm, w.bkey[b], sampler->q, sampler->n_records, B, sampler->suppress, pos_begin,
-                                            pos_end, w.idx[b], w.counts[b], w.mask[b], w.poisson, w.poisson_bytes, samp_s);
-        if (r == D3P_ERR_UNSUPPORTED)
-          r = d3p_poisson_sample_dk(w.bkey[b], sampler->q, sampler->n_records, B, sampler->suppress, w.idx[b], w.counts[b],
-                                    w.mask[b], w.poisson, w.poisson_bytes, samp_s);
-      } else {
-        if ((r = d3p_feistel_round_constants_dk(w.bkey[b], w.rc[b], samp_s)) != D3P_OK) return r;
-        r = d3p_feistel_sample_dk(w.rc[b], sampler->n_records, 0, B, w.idx[b], samp_s);
-      }
-    } else if (sampler->kind == D3P_SAMPLER_POISSON) {
-      r = D3P_ERR_UNSUPPORTED;
-      if (comm && comm->world > 1)             // selector draw split over the ranks (samplers.cu)
-        r = d3p_poisson_sample_sharded(comm, bkey, sampler->q, sampler->n_records, B, sampler->suppress, pos_begin,
-                                       pos_end, w.idx[b], w.counts[b], w.mask[b], w.poisson, w.poisson_bytes, samp_s);
-      if (r == D3P_ERR_UNSUPPORTED)            // same decision on every rank (window size, tiles >= ranks)
-        r = d3p_poisson_sample(bkey, sampler->q, sampler->n_records, B, sampler->suppress, w.idx[b], w.counts[b],
-                               w.mask[b], w.poisson, w.poisson_bytes, samp_s);
-    } else {
-      uint32_t rcs[30];
-      if ((r = d3p_feistel_round_constants_h(bkey, rcs)) != D3P_OK) return r;
-      r = d3p_feistel_sample(rcs, sampler->n_records, 0, B, w.idx[b], samp_s);
-    }
-    if (r == D3P_OK && fork && cudaEventRecord(ev_sampled[b], samp_s) != cudaSuccess) r = D3P_ERR_CUDA;
-    return r;
-  };
-  int32_t rc = D3P_OK;
-  if (fork) rc = queue_sampler(0);
-  for (uint32_t s = 0; s < n_steps && rc == D3P_OK; ++s) {
-    const int b = s & 1;
-    mark();
-    if (split) {
-      // nothing to sample: this step's records are a slice of the epoch's shuffle
-    } else if (fork) {
-      if (s + 1 < n_steps && (rc = queue_sampler(s + 1)) != D3P_OK) break;      // runs ahead on the sampler stream
-      if (cudaStreamWaitEvent(main_s, ev_sampled[b], 0) != cudaSuccess) { rc = D3P_ERR_CUDA; break; }
-    } else if ((rc = queue_sampler(s)) != D3P_OK) {
-      break;
-    }
-    const uint8_t* mask = sampler->kind == D3P_SAMPLER_POISSON ? w.mask[b] : nullptr;
-    const int32_t* idx = split ? sampler->perm_d + (size_t)(first_step + s) * B : w.idx[b];
-    mark();
-    // ---- DPSVI.update (svi.py:395-434) ----------------------------------------------------------------------
-    uint32_t keys[3][16], tf[2];
-    if (dk) {
-      // carry / k_grad -> Threefry key / k_noise -> per-leaf keys, all on the device, the state key advanced in place
-      if ((rc = d3p_dpsvi_keys_dk(rng_key_io_d, lt.n_leaves, w.tf, w.sites, main_s)) != D3P_OK) break;
-      if ((rc = fam.launch(idx, mask, B, pos_begin, pos_end, nullptr, w.tf, obs_scale, C, w.step, main_s)) != D3P_OK) break;
-      mark();
-      rc = d3p_perturb_finalize_dk_f32(w.step, n_part, P, B, &lt, w.sites, dp_scale, C, obs_scale, nullptr, optim_io_h,
-                                       params_d, m_d, v_d, stats_out_d ? stats_out_d + 3 * (size_t)s : nullptr, comm, main_s);
-    } else {
-      if ((rc = d3p_chacha_split_h(rng_key_io_h, 3, &keys[0][0])) != D3P_OK) break;           // carry, k_grad, k_noise
-      if ((rc = d3p_chacha_random_bits_h(keys[1], 0, tf, 2)) != D3P_OK) break;                // convert_to_jax_rng_key
-      rc = fam.launch(idx, mask, B, pos_begin, pos_end, tf, nullptr, obs_scale, C, w.step, main_s);
-      if (rc != D3P_OK) break;
-      mark();
-      if ((rc = d3p_chacha_split_h(keys[2], (int32_t)lt.n_leaves, &lt.site_state[0][0])) != D3P_OK) break;
-      rc = d3p_perturb_finalize_p2p_f32(w.step, n_part, P, B, &lt, dp_scale, C, obs_scale, 1, nullptr, optim_io_h,
-                                        params_d, m_d, v_d, stats_out_d ? stats_out_d + 3 * (size_t)s : nullptr, nullptr,
-                                        comm, main_s);
-    }
-    if (rc != D3P_OK) break;
-    // recorded after the finalize launch so that nothing sits between the step kernel and its programmatic dependent
-    if (fork && cudaEventRecord(ev_consumed[b], main_s) != cudaSuccess) { rc = D3P_ERR_CUDA; break; }
-    if (optim_io_h->kind == D3P_OPT_ADADP && (optim_io_h->step & 1))
-      if ((rc = d3p_adadp_finish_f32(optim_io_h, P, params_d, v_d, main_s)) != D3P_OK) break;
-    optim_io_h->step += 1;
-    if (!dk) memcpy(rng_key_io_h, keys[0], sizeof(keys[0]));
-    mark();
-  }
-  if (fork) {
-    // join: whatever is still queued on the sampler stream (only after an error) precedes later work of the caller
-    if (cudaEventRecord(ev_fork, samp_s) == cudaSuccess) cudaStreamWaitEvent(main_s, ev_fork, 0);
-  }
-  if (prof && rc == D3P_OK && ev.size() == 4 * (size_t)n_steps) {
-    cudaStreamSynchronize((cudaStream_t)stream);
-    double t[3] = {0, 0, 0};
-    for (uint32_t s = 0; s < n_steps; ++s)
-      for (int k = 0; k < 3; ++k) {
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, ev[4 * s + k], ev[4 * s + k + 1]);
-        t[k] += ms;
-      }
-    fprintf(stderr, "[d3p epoch profile] rank %d: %u steps, mean ms: sampler %.4f  step kernel %.4f  finalize %.4f\n",
-            comm ? comm->rank : 0, n_steps, t[0] / n_steps, t[1] / n_steps, t[2] / n_steps);
-  }
-  for (cudaEvent_t e : ev) cudaEventDestroy(e);
-  return rc;
-}
-}  // namespace

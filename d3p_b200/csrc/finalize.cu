@@ -433,12 +433,12 @@ extern "C" int32_t d3p_perturb_finalize_f32(const float* partials_d, uint32_t n_
                                       grad_out_d, optim_h, params_d, m_d, v_d, stats_d, nf_override_h, nullptr, stream);
 }
 
-static int32_t perturb_finalize_impl(const float* partials_d, uint32_t n_partials, uint32_t P, uint32_t B,
-                                     const d3p_leaf_table* leaves_h, const uint32_t* site_states_d, float dp_scale, float C,
-                                     float obs_scale, int32_t add_noise, float* grad_out_d,
-                                     const d3p_optim_desc* optim_h, float* params_d, float* m_d,
-                                     float* v_d, float* stats_d, const float* nf_override_h,
-                                     d3p_comm* comm, void* stream) {
+int32_t d3p::perturb_finalize_impl(const float* partials_d, uint32_t n_partials, uint32_t P, uint32_t B,
+                                   const d3p_leaf_table* leaves_h, const uint32_t* site_states_d, float dp_scale, float C,
+                                   float obs_scale, int32_t add_noise, float* grad_out_d,
+                                   const d3p_optim_desc* optim_h, float* params_d, float* m_d,
+                                   float* v_d, float* stats_d, const float* nf_override_h,
+                                   d3p_comm* comm, void* stream) {
   if (!partials_d || n_partials == 0 || B == 0) return D3P_ERR_INVALID_ARGUMENT;
   if (add_noise && !leaves_h) return D3P_ERR_INVALID_ARGUMENT;
   if (leaves_h && leaves_h->n_leaves > D3P_MAX_LEAVES) return D3P_ERR_UNSUPPORTED;

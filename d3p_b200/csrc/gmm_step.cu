@@ -529,11 +529,11 @@ extern "C" size_t d3p_gmm_workspace_bytes(const d3p_gmm_desc* desc, uint32_t* n_
   return (size_t)n_part * (desc->n_params + 2) * sizeof(float);
 }
 
-static int32_t step_gmm_impl(const d3p_gmm_desc* desc, const float* params_d, const float* x_d, size_t x_row_stride,
-                             const int32_t* idx_d, const uint8_t* mask_d, const int32_t* num_valid_d, uint32_t B,
-                             uint32_t pos_begin, uint32_t pos_end, const uint32_t* threefry_key_h,
-                             const uint32_t* threefry_key_d, float obs_scale, float C, float* px_norms_d,
-                             float* px_grads_d, float* px_loss_d, void* ws_d, size_t ws_bytes, void* stream) {
+int32_t d3p::step_gmm_impl(const d3p_gmm_desc* desc, const float* params_d, const float* x_d, size_t x_row_stride,
+                           const int32_t* idx_d, const uint8_t* mask_d, const int32_t* num_valid_d, uint32_t B,
+                           uint32_t pos_begin, uint32_t pos_end, const uint32_t* threefry_key_h,
+                           const uint32_t* threefry_key_d, float obs_scale, float C, float* px_norms_d,
+                           float* px_grads_d, float* px_loss_d, void* ws_d, size_t ws_bytes, void* stream) {
   if (!desc || !params_d || !x_d || (!threefry_key_h && !threefry_key_d) || !ws_d) return D3P_ERR_INVALID_ARGUMENT;
   if (!gmm_supported(desc)) return D3P_ERR_UNSUPPORTED;
   if (pos_end > B || pos_begin > pos_end || !(C > 0.f) || !(obs_scale != 0.f)) return D3P_ERR_INVALID_ARGUMENT;

@@ -341,12 +341,14 @@ size_t d3p_meanfield_workspace_bytes(const d3p_meanfield_desc* desc, uint32_t* n
   return (size_t)n_partials * (desc->n_params + 2) * sizeof(float);
 }
 
-static int32_t step_meanfield_impl(const d3p_meanfield_desc* desc, const float* params_d, const float* x_d,
-                                   size_t x_row_stride, const int32_t* y_d, const int32_t* idx_d,
-                                   const uint8_t* mask_d, const int32_t* num_valid_d, uint32_t B,
-                                   uint32_t pos_begin, uint32_t pos_end, const uint32_t* threefry_key_h,
-                                   const uint32_t* threefry_key_d, float obs_scale, float C, float* px_norms_d,
-                                   float* px_grads_d, float* px_loss_d, void* ws_d, size_t ws_bytes, void* stream) {
+}  // extern "C"
+
+int32_t d3p::step_meanfield_impl(const d3p_meanfield_desc* desc, const float* params_d, const float* x_d,
+                                 size_t x_row_stride, const int32_t* y_d, const int32_t* idx_d,
+                                 const uint8_t* mask_d, const int32_t* num_valid_d, uint32_t B,
+                                 uint32_t pos_begin, uint32_t pos_end, const uint32_t* threefry_key_h,
+                                 const uint32_t* threefry_key_d, float obs_scale, float C, float* px_norms_d,
+                                 float* px_grads_d, float* px_loss_d, void* ws_d, size_t ws_bytes, void* stream) {
   if (!desc_ok(desc) || !params_d || !x_d || (!threefry_key_h && !threefry_key_d) || !ws_d) return D3P_ERR_INVALID_ARGUMENT;
   if (desc->family == D3P_FAMILY_LOGREG && !y_d) return D3P_ERR_INVALID_ARGUMENT;
   if (C == 0.f || obs_scale == 0.f || B == 0 || pos_begin > pos_end || pos_end > B || x_row_stride < desc->d)
@@ -386,6 +388,8 @@ static int32_t step_meanfield_impl(const d3p_meanfield_desc* desc, const float* 
   if (desc->link == D3P_LINK_EXP) return launch_shape<D3P_FAMILY_GAUSS, D3P_LINK_EXP>(sh, a, smem, n_partials, s);
   return launch_shape<D3P_FAMILY_GAUSS, D3P_LINK_SOFTPLUS>(sh, a, smem, n_partials, s);
 }
+
+extern "C" {
 
 int32_t d3p_dpsvi_step_meanfield(const d3p_meanfield_desc* desc, const float* params_d, const float* x_d,
                                  size_t x_row_stride, const int32_t* y_d, const int32_t* idx_d,

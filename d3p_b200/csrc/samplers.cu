@@ -390,8 +390,10 @@ int32_t d3p_feistel_round_constants_h(const uint32_t state_h[16], uint32_t rc_h[
   return D3P_OK;
 }
 
-static int32_t feistel_sample_impl(const uint32_t* rc_h, const uint32_t* rc_d, uint32_t capacity, uint32_t first_pos,
-                                   uint32_t n, int32_t* idx_d, void* stream) {
+}  // extern "C"
+
+int32_t d3p::feistel_sample_impl(const uint32_t* rc_h, const uint32_t* rc_d, uint32_t capacity, uint32_t first_pos,
+                                 uint32_t n, int32_t* idx_d, void* stream) {
   if ((!rc_h && !rc_d) || capacity == 0 || (!idx_d && n)) return D3P_ERR_INVALID_ARGUMENT;
   if ((uint64_t)first_pos + n > (uint64_t)capacity) return D3P_ERR_INVALID_ARGUMENT;
   if (n == 0) return D3P_OK;
@@ -410,6 +412,8 @@ static int32_t feistel_sample_impl(const uint32_t* rc_h, const uint32_t* rc_d, u
   feistel_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(p, rc_d, first_pos, n, idx_d);
   return check_launch();
 }
+
+extern "C" {
 
 int32_t d3p_feistel_sample(const uint32_t rc_h[30], uint32_t capacity, uint32_t first_pos, uint32_t n,
                            int32_t* idx_d, void* stream) {
@@ -432,9 +436,11 @@ int32_t d3p_feistel_sample_dk(const uint32_t* rc_d, uint32_t capacity, uint32_t 
 
 size_t d3p_poisson_workspace_bytes(uint32_t n_records) { return carve_poisson_ws(nullptr, n_records).bytes; }
 
-static int32_t poisson_sample_impl(const uint32_t* state_h, const uint32_t* state_d, float q, uint32_t n_records,
-                                   uint32_t max_b, int32_t suppress, int32_t* idx_d, int32_t* counts_d, uint8_t* mask_d,
-                                   void* ws_d, size_t ws_bytes, void* stream) {
+}  // extern "C"
+
+int32_t d3p::poisson_sample_impl(const uint32_t* state_h, const uint32_t* state_d, float q, uint32_t n_records,
+                                 uint32_t max_b, int32_t suppress, int32_t* idx_d, int32_t* counts_d, uint8_t* mask_d,
+                                 void* ws_d, size_t ws_bytes, void* stream) {
   if ((!state_h && !state_d) || !counts_d || !ws_d || (!idx_d && max_b) || n_records == 0 || max_b > n_records)
     return D3P_ERR_INVALID_ARGUMENT;
   const ChaChaArg key = chacha_arg(state_h, state_d);
@@ -452,6 +458,8 @@ static int32_t poisson_sample_impl(const uint32_t* state_h, const uint32_t* stat
   return check_launch();
 }
 
+extern "C" {
+
 int32_t d3p_poisson_sample(const uint32_t state_h[16], float q, uint32_t n_records, uint32_t max_b,
                            int32_t suppress, int32_t* idx_d, int32_t* counts_d, uint8_t* mask_d, void* ws_d,
                            size_t ws_bytes, void* stream) {
@@ -466,10 +474,12 @@ int32_t d3p_poisson_sample_dk(const uint32_t* state_d, float q, uint32_t n_recor
   return poisson_sample_impl(nullptr, state_d, q, n_records, max_b, suppress, idx_d, counts_d, mask_d, ws_d, ws_bytes, stream);
 }
 
-static int32_t poisson_sample_sharded_impl(d3p_comm* comm, const uint32_t* state_h, const uint32_t* state_d, float q,
-                                           uint32_t n_records, uint32_t max_b, int32_t suppress, uint32_t pos_begin,
-                                           uint32_t pos_end, int32_t* idx_d, int32_t* counts_d, uint8_t* mask_d,
-                                           void* ws_d, size_t ws_bytes, void* stream) {
+}  // extern "C"
+
+int32_t d3p::poisson_sample_sharded_impl(d3p_comm* comm, const uint32_t* state_h, const uint32_t* state_d, float q,
+                                         uint32_t n_records, uint32_t max_b, int32_t suppress, uint32_t pos_begin,
+                                         uint32_t pos_end, int32_t* idx_d, int32_t* counts_d, uint8_t* mask_d,
+                                         void* ws_d, size_t ws_bytes, void* stream) {
   const ChaChaArg key = chacha_arg(state_h, state_d);
   if (!comm || (!state_h && !state_d) || !counts_d || !ws_d || (!idx_d && max_b) || n_records == 0 || max_b > n_records ||
       pos_begin > pos_end || pos_end > max_b)
@@ -500,6 +510,8 @@ static int32_t poisson_sample_sharded_impl(d3p_comm* comm, const uint32_t* state
                                                                 key, q, cov_lo, cov_hi);
   return check_launch();
 }
+
+extern "C" {
 
 int32_t d3p_poisson_sample_sharded(d3p_comm* comm, const uint32_t state_h[16], float q, uint32_t n_records,
                                    uint32_t max_b, int32_t suppress, uint32_t pos_begin, uint32_t pos_end,

@@ -7,7 +7,6 @@ import numpy as np
 import torch
 
 from . import _native as _n
-from .models import VAE, GaussianMixture, MeanFieldFamily
 
 
 def _threefry_split_second(key):
@@ -39,33 +38,11 @@ def evaluate_elbo(svi, svi_state, jax_key, args):
     # (d3p/minibatch.py:126-131), so those are materialised rather than read through the index list
     from .minibatch import BatchView
     args = tuple(a.tensor() if (isinstance(a, BatchView) and a.num_valid is not None) else a for a in args)
-    Xsrc, stride, ysrc, idx, B = svi._resolve_args(args)
-    if getattr(svi, "_local_rows", None) is not None:
+    b = svi._resolve_args(args)
+    if b.local_rows is not None:
         raise NotImplementedError("DPSVI.evaluate takes whole batches (LocalRows are a sharded-update input)")
     desc = fam.desc(svi._num_obs_total())
     key = _threefry_split_second(np.asarray(jax_key, dtype=np.uint32).reshape(2))    # SVI.evaluate: _, rng_key_eval
-    lib = _n.lib()
-    kp = key.ctypes.data_as(C.POINTER(C.c_uint32))
-    loss = torch.empty(1, dtype=torch.float32, device=Xsrc.device)
-    flat = svi_state.optim_state.flat
-    if isinstance(fam, VAE):
-        need = lib.d3p_vae_workspace_bytes(C.byref(desc), B, None)
-        ws = svi._workspace(need + 256)
-        ws_al = ws[((-ws.data_ptr()) % 256) // 4:]
-        _n.check(lib.d3p_elbo_evaluate_vae(C.byref(desc), _n.ptr(flat), _n.ptr(Xsrc), stride, _n.ptr(idx), B, kp, _n.ptr(loss),
-                                           _n.ptr(ws_al), need, fam._side_streams(), _n.stream_ptr()), "elbo_evaluate_vae")
-        return loss[0]
-    if isinstance(fam, GaussianMixture):
-        need = lib.d3p_elbo_evaluate_gmm_workspace_bytes(C.byref(desc))
-        ws = torch.empty((need + 3) // 4, dtype=torch.float32, device=Xsrc.device)
-        _n.check(lib.d3p_elbo_evaluate_gmm(C.byref(desc), _n.ptr(flat), _n.ptr(Xsrc), stride, _n.ptr(idx), B, kp, _n.ptr(loss),
-                                           _n.ptr(ws), need, _n.stream_ptr()), "elbo_evaluate_gmm")
-        return loss[0]
-    if not isinstance(fam, MeanFieldFamily):
-        raise NotImplementedError(f"DPSVI.evaluate: unknown family {type(fam).__name__}")
-    need = lib.d3p_elbo_evaluate_workspace_bytes()
-    ws = torch.empty((need + 3) // 4, dtype=torch.float32, device=Xsrc.device)
-    _n.check(lib.d3p_elbo_evaluate_meanfield(C.byref(desc), _n.ptr(svi_state.optim_state.flat), _n.ptr(Xsrc), stride,
-                                             _n.ptr(ysrc), _n.ptr(idx), B, key.ctypes.data_as(C.POINTER(C.c_uint32)),
-                                             _n.ptr(loss), _n.ptr(ws), need, _n.stream_ptr()), "elbo_evaluate")
+    loss = torch.empty(1, dtype=torch.float32, device=b.x.device)
+    fam._evaluate(svi, desc, _n.ptr(svi_state.optim_state.flat), b, key.ctypes.data_as(C.POINTER(C.c_uint32)), loss)
     return loss[0]

@@ -13,6 +13,8 @@ Parameters are the *unconstrained* variational parameters, stored as one flat fl
 whose leaf order is the jax pytree order of the reference's param dict (sorted site names).
 Arbitrary models go through the materialised-gradient stage methods of ``DPSVI``.
 """
+import ctypes as C
+
 import numpy as np
 import torch
 
@@ -42,7 +44,11 @@ class _Handle:
 
 
 class Family:
-    """What ``DPSVI`` needs from a fused model/guide family."""
+    """What ``DPSVI`` needs from a fused model/guide family.  A subclass supplies the calls of its entry points of the
+    library (``_step_workspace_bytes`` / ``_step``, ``_evaluate``, ``_epoch_workspace_bytes`` / ``_epoch``)."""
+    # DPSVI.run_epoch has a C driver with device keys / for a batch sharded over NVLink peers (else: step by step)
+    epoch_device_keys = True
+    epoch_sharded = True
 
     def layout(self):
         """[(name, offset, shape)] in pytree (sorted-name) order."""
@@ -65,25 +71,6 @@ class Family:
     def constrain(self, name, value):
         return value
 
-    @staticmethod
-    def _local_row_pointers(svi, Xsrc, stride, mask_t, pos_begin, pos_end):
-        """Base pointers of X and of the mask as the step kernels want them.  With ``minibatch.LocalRows`` the tensors
-        hold only rows [first, first + n) of the batch: the pointers are shifted back so that the kernel's global
-        position p addresses local row p - first (the kernels touch positions [pos_begin, pos_end) only)."""
-        import ctypes as C
-        x_p, m_p = _n.ptr(Xsrc), _n.ptr(mask_t)
-        if getattr(svi, "_local_rows", None) is not None:
-            first, n_local = svi._local_rows
-            if (first, first + n_local) != (pos_begin, pos_end):
-                raise ValueError(f"LocalRows [{first}, {first + n_local}) is not this rank's position range "
-                                 f"[{pos_begin}, {pos_end})")
-            x_p = C.c_void_p(Xsrc.data_ptr() - first * stride * 4)
-            if mask_t is not None:
-                if mask_t.numel() != n_local:
-                    raise ValueError("with LocalRows the mask must be the matching LocalRows slice")
-                m_p = C.c_void_p(mask_t.data_ptr() - first)
-        return x_p, m_p
-
     def observation_scale(self, num_obs_total):
         """``get_observations_scale`` (d3p/svi.py:43-65) on a one-element batch: the plate scale N / 1."""
         return float(num_obs_total)
@@ -97,8 +84,61 @@ class Family:
     def check_args(self, args):
         raise NotImplementedError
 
-    def run_step(self, svi, state, tf_key, args, mask, B, pos_begin, pos_end, px_norms, px_grads, px_loss):
-        """-> (partials tensor [n_partials, P + 2], n_partials, B, P)"""
+    def run_step(self, svi, state, tf_key, args, mask, pos_begin, pos_end, px_norms, px_grads, px_loss):
+        """The fused per-example-gradient / clip / sum kernels of batch positions [pos_begin, pos_end)
+        -> (partials tensor [n_partials, P + 2], n_partials, B, P)"""
+        b = svi._resolve_args(args)
+        desc = self.desc(svi._num_obs_total())
+        n_part = C.c_uint32(0)
+        need = self._step_workspace_bytes(desc, pos_end - pos_begin, n_part)
+        ws = svi._workspace(need)
+        mask_t, _ = svi._mask_arg(mask, b.B)
+        x_p, y_p, m_p = _n.ptr(b.x), _n.ptr(b.y), _n.ptr(mask_t)
+        if b.local_rows is not None:
+            # minibatch.LocalRows: the tensors hold only rows [first, first + n) of the batch; shift the base
+            # pointers so that the kernel's global position p addresses local row p - first
+            first, n_local = b.local_rows
+            if (first, first + n_local) != (pos_begin, pos_end):
+                raise ValueError(f"LocalRows [{first}, {first + n_local}) is not this rank's position range "
+                                 f"[{pos_begin}, {pos_end})")
+            x_p = C.c_void_p(b.x.data_ptr() - first * b.stride * 4)
+            y_p = C.c_void_p(b.y.data_ptr() - first * 4) if b.y is not None else None
+            if mask_t is not None:
+                if mask_t.numel() != n_local:
+                    raise ValueError("with LocalRows the mask must be the matching LocalRows slice")
+                m_p = C.c_void_p(mask_t.data_ptr() - first)
+        # the arguments idx_d .. C, which every family's step entry point takes in this order
+        rows = (_n.ptr(b.idx), m_p, _n.ptr(b.num_valid), b.B, pos_begin, pos_end,
+                tf_key.ctypes.data_as(C.POINTER(C.c_uint32)), float(state.observation_scale),
+                float(svi._clipping_threshold))
+        if svi.event_hook is not None:
+            svi.event_hook("step_begin")
+        self._step(desc, _n.ptr(state.optim_state.flat), x_p, b.stride, y_p, rows, px_norms, px_grads, px_loss, ws, need)
+        if svi.event_hook is not None:
+            svi.event_hook("step_end")
+        return ws, n_part.value, b.B, desc.n_params
+
+    def desc(self, num_obs_total):
+        """The family's descriptor struct of the library."""
+        raise NotImplementedError
+
+    def _step_workspace_bytes(self, desc, rows, n_part):
+        """Workspace of one step over ``rows`` batch rows; sets ``n_part`` (c_uint32) to the number of partial rows."""
+        raise NotImplementedError
+
+    def _step(self, desc, params, x, stride, y, rows, px_norms, px_grads, px_loss, ws, need):
+        """The family's ``d3p_dpsvi_step_*`` call (``y``: labels, read by the families that have them)."""
+        raise NotImplementedError
+
+    def _evaluate(self, svi, desc, params, b, key, loss):
+        """``DPSVI.evaluate`` of the ``ResolvedBatch`` b with the Threefry key ``key`` into the device scalar ``loss``."""
+        raise NotImplementedError(f"DPSVI.evaluate: unknown family {type(self).__name__}")
+
+    def _epoch_workspace_bytes(self, desc, sampler, world):
+        raise NotImplementedError
+
+    def _epoch(self, device_keys, desc, sampler, x, stride, y, batch_key, rng_key, rest):
+        """One ``d3p_dpsvi_run_epoch_*`` call; ``rest`` = the arguments from ``first_step`` on."""
         raise NotImplementedError
 
 
@@ -129,42 +169,29 @@ class MeanFieldFamily(Family):
             return torch.nn.functional.softplus(value)
         return value
 
-    def desc(self, num_obs_total):
-        raise NotImplementedError
+    def _step_workspace_bytes(self, desc, rows, n_part):
+        return _n.lib().d3p_meanfield_workspace_bytes(C.byref(desc), C.byref(n_part))
 
-    def run_step(self, svi, state, tf_key, args, mask, B, pos_begin, pos_end, px_norms, px_grads, px_loss):
-        import ctypes as C
-        Xsrc, stride, ysrc, idx, B = svi._resolve_args(args)
-        desc = self.desc(svi._num_obs_total())
-        n_part = C.c_uint32(0)
-        need = _n.lib().d3p_meanfield_workspace_bytes(C.byref(desc), C.byref(n_part))
-        ws = svi._workspace(need)
-        mask_t, _ = svi._mask_arg(mask, B)
-        flat = state.optim_state.flat
-        x_p, y_p, m_p = _n.ptr(Xsrc), _n.ptr(ysrc), _n.ptr(mask_t)
-        if getattr(svi, "_local_rows", None) is not None:
-            # minibatch.LocalRows: the tensors hold only rows [first, first + n) of the batch; shift the base
-            # pointers so that the kernel's global position p addresses local row p - first
-            first, n_local = svi._local_rows
-            if (first, first + n_local) != (pos_begin, pos_end):
-                raise ValueError(f"LocalRows [{first}, {first + n_local}) is not this rank's position range "
-                                 f"[{pos_begin}, {pos_end})")
-            x_p = C.c_void_p(Xsrc.data_ptr() - first * stride * 4)
-            y_p = C.c_void_p(ysrc.data_ptr() - first * 4) if ysrc is not None else None
-            if mask_t is not None:
-                if mask_t.numel() != n_local:
-                    raise ValueError("with LocalRows the mask must be the matching LocalRows slice")
-                m_p = C.c_void_p(mask_t.data_ptr() - first)
-        if svi.event_hook is not None:
-            svi.event_hook("step_begin")
+    def _step(self, desc, params, x, stride, y, rows, px_norms, px_grads, px_loss, ws, need):
         _n.check(_n.lib().d3p_dpsvi_step_meanfield(
-            C.byref(desc), _n.ptr(flat), x_p, stride, y_p, _n.ptr(idx), m_p, _n.ptr(getattr(svi, "_num_valid", None)),
-            B, pos_begin, pos_end, tf_key.ctypes.data_as(C.POINTER(C.c_uint32)), float(state.observation_scale),
-            float(svi._clipping_threshold), _n.ptr(px_norms), _n.ptr(px_grads), _n.ptr(px_loss), _n.ptr(ws), need,
-            _n.stream_ptr()), "dpsvi_step_meanfield")
-        if svi.event_hook is not None:
-            svi.event_hook("step_end")
-        return ws, n_part.value, B, desc.n_params
+            C.byref(desc), params, x, stride, y, *rows, _n.ptr(px_norms), _n.ptr(px_grads), _n.ptr(px_loss), _n.ptr(ws),
+            need, _n.stream_ptr()), "dpsvi_step_meanfield")
+
+    def _evaluate(self, svi, desc, params, b, key, loss):
+        need = _n.lib().d3p_elbo_evaluate_workspace_bytes()
+        ws = svi._workspace(need)
+        _n.check(_n.lib().d3p_elbo_evaluate_meanfield(C.byref(desc), params, _n.ptr(b.x), b.stride, _n.ptr(b.y),
+                                                      _n.ptr(b.idx), b.B, key, _n.ptr(loss), _n.ptr(ws), need,
+                                                      _n.stream_ptr()), "elbo_evaluate")
+
+    def _epoch_workspace_bytes(self, desc, sampler, world):
+        return _n.lib().d3p_dpsvi_epoch_workspace_bytes(C.byref(desc), C.byref(sampler))
+
+    def _epoch(self, device_keys, desc, sampler, x, stride, y, batch_key, rng_key, rest):
+        lib = _n.lib()
+        run = lib.d3p_dpsvi_run_epoch_meanfield_dk if device_keys else lib.d3p_dpsvi_run_epoch_meanfield
+        _n.check(run(C.byref(desc), C.byref(sampler), x, stride, y, batch_key, rng_key, *rest),
+                 "run_epoch_dk" if device_keys else "run_epoch")
 
 
 class LogisticRegression(MeanFieldFamily):
@@ -293,7 +320,6 @@ class VAE(Family):
     def _side_streams(self):
         """This family object's ``d3p_vae_ctx`` on the current device (caller-owned side streams: the four clipped-sum
         GEMMs of a step run concurrently on them); created on first use, released with the object."""
-        import ctypes as C
         dev = torch.cuda.current_device()
         ctxs = self.__dict__.setdefault("_ctx", {})
         if dev not in ctxs:
@@ -318,31 +344,31 @@ class VAE(Family):
         except Exception:
             pass
 
-    def run_step(self, svi, state, tf_key, args, mask, B, pos_begin, pos_end, px_norms, px_grads, px_loss):
-        import ctypes as C
+    def _step_workspace_bytes(self, desc, rows, n_part):
+        return _n.lib().d3p_vae_workspace_bytes(C.byref(desc), rows, C.byref(n_part))
+
+    def _step(self, desc, params, x, stride, y, rows, px_norms, px_grads, px_loss, ws, need):
         if px_grads is not None:
             raise NotImplementedError("the VAE path never materialises [B, P] per-example gradients")
-        Xsrc, stride, _, idx, B = svi._resolve_args(args)
-        desc = self.desc(svi._num_obs_total())
-        n_part = C.c_uint32(0)
-        need = _n.lib().d3p_vae_workspace_bytes(C.byref(desc), pos_end - pos_begin, C.byref(n_part))
-        ws = svi._workspace(need + 256)
-        base = ws.data_ptr()
-        shift = (-base) % 256                    # the library wants a 256-byte aligned workspace
-        ws_al = ws[shift // 4:]
-        mask_t, _ = svi._mask_arg(mask, B)
-        x_p, m_p = self._local_row_pointers(svi, Xsrc, stride, mask_t, pos_begin, pos_end)
-        if svi.event_hook is not None:
-            svi.event_hook("step_begin")
         _n.check(_n.lib().d3p_dpsvi_step_vae(
-            C.byref(desc), _n.ptr(state.optim_state.flat), x_p, stride, _n.ptr(idx), m_p,
-            _n.ptr(getattr(svi, "_num_valid", None)), B,
-            pos_begin, pos_end, tf_key.ctypes.data_as(C.POINTER(C.c_uint32)), float(state.observation_scale),
-            float(svi._clipping_threshold), _n.ptr(px_norms), _n.ptr(px_loss), _n.ptr(ws_al), need,
+            C.byref(desc), params, x, stride, *rows, _n.ptr(px_norms), _n.ptr(px_loss), _n.ptr(ws), need,
             self.profile_events, self._side_streams(), _n.stream_ptr()), "dpsvi_step_vae")
-        if svi.event_hook is not None:
-            svi.event_hook("step_end")
-        return ws_al, n_part.value, B, desc.n_params
+
+    def _evaluate(self, svi, desc, params, b, key, loss):
+        need = _n.lib().d3p_vae_workspace_bytes(C.byref(desc), b.B, None)
+        ws = svi._workspace(need)
+        _n.check(_n.lib().d3p_elbo_evaluate_vae(C.byref(desc), params, _n.ptr(b.x), b.stride, _n.ptr(b.idx), b.B, key,
+                                                _n.ptr(loss), _n.ptr(ws), need, self._side_streams(), _n.stream_ptr()),
+                 "elbo_evaluate_vae")
+
+    def _epoch_workspace_bytes(self, desc, sampler, world):
+        return _n.lib().d3p_dpsvi_epoch_vae_workspace_bytes(C.byref(desc), C.byref(sampler), world)
+
+    def _epoch(self, device_keys, desc, sampler, x, stride, y, batch_key, rng_key, rest):
+        lib = _n.lib()
+        run = lib.d3p_dpsvi_run_epoch_vae_dk if device_keys else lib.d3p_dpsvi_run_epoch_vae
+        _n.check(run(C.byref(desc), C.byref(sampler), x, stride, batch_key, rng_key, *rest),
+                 "run_epoch_vae_dk" if device_keys else "run_epoch_vae")
 
 
 class GaussianMixture(Family):
@@ -351,6 +377,8 @@ class GaussianMixture(Family):
     pis ~ Dir(exp(alpha_log)), mus ~ N(mus_loc, 1), sigs ~ InvGamma(1, 1), every site drawn per
     example; ``update(state, X)`` with X of shape [B, d] (the example's ``k`` positional argument is
     the constructor's ``K``)."""
+    epoch_device_keys = False       # the mixture's epoch driver: host keys, one GPU
+    epoch_sharded = False
 
     def __init__(self, K, d):
         self.K, self.d = int(K), int(d)
@@ -376,23 +404,23 @@ class GaussianMixture(Family):
         g.num_obs_total = float(num_obs_total)
         return g
 
-    def run_step(self, svi, state, tf_key, args, mask, B, pos_begin, pos_end, px_norms, px_grads, px_loss):
-        import ctypes as C
-        Xsrc, stride, _, idx, B = svi._resolve_args(args)
-        desc = self.desc(svi._num_obs_total())
-        n_part = C.c_uint32(0)
-        need = _n.lib().d3p_gmm_workspace_bytes(C.byref(desc), C.byref(n_part))
-        ws = svi._workspace(need)
-        mask_t, _ = svi._mask_arg(mask, B)
-        x_p, m_p = self._local_row_pointers(svi, Xsrc, stride, mask_t, pos_begin, pos_end)
-        if svi.event_hook is not None:
-            svi.event_hook("step_begin")
+    def _step_workspace_bytes(self, desc, rows, n_part):
+        return _n.lib().d3p_gmm_workspace_bytes(C.byref(desc), C.byref(n_part))
+
+    def _step(self, desc, params, x, stride, y, rows, px_norms, px_grads, px_loss, ws, need):
         _n.check(_n.lib().d3p_dpsvi_step_gmm(
-            C.byref(desc), _n.ptr(state.optim_state.flat), x_p, stride, _n.ptr(idx), m_p,
-            _n.ptr(getattr(svi, "_num_valid", None)), B,
-            pos_begin, pos_end, tf_key.ctypes.data_as(C.POINTER(C.c_uint32)), float(state.observation_scale),
-            float(svi._clipping_threshold), _n.ptr(px_norms), _n.ptr(px_grads), _n.ptr(px_loss), _n.ptr(ws), need,
-            _n.stream_ptr()), "dpsvi_step_gmm")
-        if svi.event_hook is not None:
-            svi.event_hook("step_end")
-        return ws, n_part.value, B, desc.n_params
+            C.byref(desc), params, x, stride, *rows, _n.ptr(px_norms), _n.ptr(px_grads), _n.ptr(px_loss), _n.ptr(ws),
+            need, _n.stream_ptr()), "dpsvi_step_gmm")
+
+    def _evaluate(self, svi, desc, params, b, key, loss):
+        need = _n.lib().d3p_elbo_evaluate_gmm_workspace_bytes(C.byref(desc))
+        ws = svi._workspace(need)
+        _n.check(_n.lib().d3p_elbo_evaluate_gmm(C.byref(desc), params, _n.ptr(b.x), b.stride, _n.ptr(b.idx), b.B, key,
+                                                _n.ptr(loss), _n.ptr(ws), need, _n.stream_ptr()), "elbo_evaluate_gmm")
+
+    def _epoch_workspace_bytes(self, desc, sampler, world):
+        return _n.lib().d3p_dpsvi_epoch_gmm_workspace_bytes(C.byref(desc), C.byref(sampler))
+
+    def _epoch(self, device_keys, desc, sampler, x, stride, y, batch_key, rng_key, rest):
+        _n.check(_n.lib().d3p_dpsvi_run_epoch_gmm(C.byref(desc), C.byref(sampler), x, stride, batch_key, rng_key, *rest),
+                 "run_epoch_gmm")

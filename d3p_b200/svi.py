@@ -30,6 +30,17 @@ class DPSVIState(NamedTuple):
     observation_scale: float
 
 
+class ResolvedBatch(NamedTuple):
+    """A batch as the step / evaluate / epoch kernels take it (``DPSVI._resolve_args``)."""
+    x: torch.Tensor      # float32 rows on the device
+    stride: int          # row stride of x in elements
+    y: Any               # int32 labels read at the same rows as x, or None
+    idx: Any             # int32 row indices of a BatchView into x, or None: row p of x is batch position p
+    B: int               # batch size
+    num_valid: Any       # device count of the real rows of a Poisson BatchView (the kernels skip the rest), or None
+    local_rows: Any      # (first, n_local) of a LocalRows slice, or None
+
+
 # ---- pytree helpers (dict leaves in sorted-key order, like jax) ----------------------------------
 def tree_leaves(tree):
     if tree is None:
@@ -85,6 +96,27 @@ def _concat_rows(leaves, batched):
         flat = [t.reshape(1, -1) for t in ts]
     sizes = [f.shape[1] for f in flat]
     return torch.cat(flat, dim=1).contiguous(), sizes, [tuple(t.shape) for t in ts]
+
+
+def _aligned_scratch(ws, need):
+    """The cached float32 scratch tensor ``ws`` if it holds ``need`` bytes on the device, else a new one; 256-byte
+    aligned (the VAE kernels require it)."""
+    if ws is None or ws.numel() * 4 < need or ws.device != _dev():
+        buf = torch.empty((need + 256 + 3) // 4, dtype=torch.float32, device=_dev())
+        ws = buf[((-buf.data_ptr()) % 256) // 4:]
+    return ws
+
+
+def _leaf_layout(layout):
+    """A ``LeafTable`` with the offsets and lengths of the leaves of ``layout`` (site states zero)."""
+    if len(layout) > _n.MAX_LEAVES:
+        raise _n.D3PNativeError(f"more than {_n.MAX_LEAVES} parameter leaves are not supported")
+    lt = _n.LeafTable()
+    lt.n_leaves = len(layout)
+    for l, (name, off, shape) in enumerate(layout):
+        lt.leaf_off[l] = off
+        lt.leaf_len[l] = int(np.prod(shape)) if len(shape) else 1
+    return lt
 
 
 def _split_rows(mat, sizes, shapes):
@@ -210,37 +242,34 @@ class DPSVI:
 
     # ---- fused path ------------------------------------------------------------------------------
     def _workspace(self, need):
-        """A cached, 256-byte aligned float32 scratch tensor of at least ``need`` bytes."""
+        """A 256-byte aligned float32 view of at least ``need`` bytes into a cached scratch tensor."""
         if need == 0:
             raise _n.D3PNativeError("unsupported model family configuration")
-        if self._ws is None or self._ws.numel() * 4 < need or self._ws.device != _dev():
-            self._ws = torch.empty((need + 3) // 4, dtype=torch.float32, device=_dev())
+        self._ws = _aligned_scratch(self._ws, need)
         return self._ws
 
     def _resolve_args(self, args):
-        """-> (x, x_stride, y, idx, B) for the step kernel."""
+        """-> ``ResolvedBatch`` of the batch arrays ``args``."""
         fam = self.family
         fam.check_args(args)
         X = args[0]
         idx = None
-        self._local_rows = None
         # a Poisson BatchView knows how many of its slots are real: the kernels skip the padding slots even when the
         # caller does not pass mask= (the reference zero-fills those rows, d3p/minibatch.py:126-131)
-        self._num_valid = X.num_valid if isinstance(X, BatchView) else None
+        num_valid = X.num_valid if isinstance(X, BatchView) else None
         if isinstance(X, LocalRows):
             # rank-local slice of the batch: (first, n_local); the step kernel addresses rows by global
             # position, so the family shifts the base pointers back by `first` rows
             if any(not isinstance(a, LocalRows) or a.first != X.first or a.tensor.shape[0] != X.tensor.shape[0]
                    for a in args):
                 raise ValueError("all batch arrays must be LocalRows of the same slice")
-            self._local_rows = (X.first, int(X.tensor.shape[0]))
             B = X.batch_size
             Xsrc = X.tensor.to(device=_dev(), dtype=torch.float32)
             if Xsrc.dim() > 2:
                 Xsrc = Xsrc.reshape(Xsrc.shape[0], -1)
             Xsrc = Xsrc.contiguous()
             ysrc = args[1].tensor.to(device=_dev(), dtype=torch.int32).contiguous() if len(args) > 1 else None
-            return Xsrc, int(Xsrc.stride(0)), ysrc, None, B
+            return ResolvedBatch(Xsrc, int(Xsrc.stride(0)), ysrc, None, B, num_valid, (X.first, int(X.tensor.shape[0])))
         if isinstance(X, BatchView):
             idx, Xsrc = X.idx, X.source
             ysrc = None
@@ -250,7 +279,7 @@ class DPSVI:
                     ysrc = Y.source
                 else:   # mixed: materialise everything
                     idx, Xsrc = None, X.tensor()
-                    self._num_valid = None          # the gather zero-filled the padding rows
+                    num_valid = None          # the gather zero-filled the padding rows
                     ysrc = Y.tensor() if isinstance(Y, BatchView) else Y
         else:
             Xsrc = X
@@ -278,7 +307,7 @@ class DPSVI:
                                  f"{rows_needed} are needed")
         if idx is None and Xsrc.shape[0] < B:
             raise ValueError(f"the batch array has {Xsrc.shape[0]} rows, {B} are needed")
-        return Xsrc, int(Xsrc.stride(0)), ysrc, idx, B
+        return ResolvedBatch(Xsrc, int(Xsrc.stride(0)), ysrc, idx, B, num_valid, None)
 
     @staticmethod
     def _mask_arg(mask, B):
@@ -309,18 +338,13 @@ class DPSVI:
             rank, world = self.shard[0], self.shard[1]
             per = (B + world - 1) // world
             pos_begin, pos_end = min(B, rank * per), min(B, (rank + 1) * per)
-        return fam.run_step(self, state, tf_key, args, mask, B, pos_begin, pos_end, px_norms, px_grads, px_loss)
+        return fam.run_step(self, state, tf_key, args, mask, pos_begin, pos_end, px_norms, px_grads, px_loss)
 
     def _leaf_table(self, layout, rng_key):
         """Per-leaf site keys: ``rng_suite.split(rng, n_leaves)`` (svi.py:490-491)."""
-        if len(layout) > _n.MAX_LEAVES:
-            raise _n.D3PNativeError(f"more than {_n.MAX_LEAVES} parameter leaves are not supported")
-        lt = _n.LeafTable()
-        lt.n_leaves = len(layout)
+        lt = _leaf_layout(layout)
         site_keys = np.asarray(self._rng_suite.split(rng_key, len(layout)), dtype=np.uint32).reshape(len(layout), 16)
-        for l, (name, off, shape) in enumerate(layout):
-            lt.leaf_off[l] = off
-            lt.leaf_len[l] = int(np.prod(shape)) if len(shape) else 1
+        for l in range(len(layout)):
             for i in range(16):
                 lt.site_state[l][i] = int(site_keys[l, i])
         return lt
@@ -408,24 +432,22 @@ class DPSVI:
         (``examples/logistic_regression.py:149-160``): returns ``(new_state, stats)`` where
         ``stats[num_steps, 3]`` holds ``(loss, n, f)`` per step on the device.
 
-        For the mean-field families and the VAE fed by ``poisson_batchify_data`` /
-        ``subsample_batchify_data`` the whole loop runs inside ``d3p_dpsvi_run_epoch_meanfield`` /
-        ``d3p_dpsvi_run_epoch_vae`` (no interpreter between launches); the result is bit-identical to
-        the step-by-step calls, which remain the path for everything else (NCCL-backend sharded runs,
-        GMM, custom batchifiers).
+        For the model families fed by ``poisson_batchify_data`` / ``subsample_batchify_data`` /
+        ``split_batchify_data`` the whole loop runs inside the family's ``d3p_dpsvi_run_epoch_*`` driver (no
+        interpreter between launches); the result is bit-identical to the step-by-step calls, which remain the path for
+        everything else (NCCL-backend sharded runs, custom batchifiers, and the key modes or sharded runs a family has
+        no driver for: ``Family.epoch_device_keys`` / ``Family.epoch_sharded``).
 
         ``device_keys=True`` drives the ``*_dk`` entry points: the batchifier key and the state key are uploaded once
         and every per-step key is derived on the device (what a jitted caller with traced keys binds to, see
         INTEGRATION.md); the results are bit-identical.  This facade then reads the final state key back, which
         synchronises; a binding that keeps its keys on the device does not."""
-        from .models import GaussianMixture, MeanFieldFamily, VAE
+        fam = self.family
         spec = getattr(get_batch, "spec", None)
-        is_vae, is_gmm = isinstance(self.family, VAE), isinstance(self.family, GaussianMixture)
         is_split = spec is not None and spec["kind"] == _n.SAMPLER_SPLIT
-        if is_gmm and (device_keys or self.shard is not None):
-            spec = None         # the mixture's epoch driver: single GPU, host keys
-        fused = (spec is not None and (isinstance(self.family, MeanFieldFamily) or is_vae or is_gmm)
-                 and (self.shard is None or self.shard[2] is None) and self._rng_suite is strong_rng and spec["rng_suite"] is strong_rng and self.event_hook is None
+        fused = (spec is not None and fam is not None and (fam.epoch_device_keys or not device_keys)
+                 and (self.shard is None or (fam.epoch_sharded and self.shard[2] is None))
+                 and self._rng_suite is strong_rng and spec["rng_suite"] is strong_rng and self.event_hook is None
                  and num_steps > 0)
         if not fused:
             stats = torch.zeros(max(num_steps, 0), 3, dtype=torch.float32, device=_dev())
@@ -435,28 +457,22 @@ class DPSVI:
                 svi_state, loss = self.update(svi_state, *batch, mask=mask)
                 stats[s, 0] = loss
             return svi_state, stats
-        fam = self.family
         dev = _dev()
         world = self.shard[1] if self.shard is not None else 1
         # everything about an epoch call that depends only on (batchifier, family, device) is worked out once
         plan_key = (id(spec), dev.index, world, self._num_obs_total())
         plan = getattr(self, "_epoch_plan", None)
         if plan is None or plan[0] != plan_key:
-            Xsrc, stride, ysrc, _, _ = self._resolve_args(spec["dataset"])
+            data = self._resolve_args(spec["dataset"])
             desc = fam.desc(self._num_obs_total())
             sd = _n.SamplerDesc(spec["kind"], spec["q"], spec["n_records"], spec["batch"], 1 if spec["suppress"] else 0, None)
             probe = sd
             if is_split:        # the size query wants a non-null shuffle pointer; the real one is set per call
                 probe = _n.SamplerDesc(spec["kind"], spec["q"], spec["n_records"], spec["batch"], 0, 256)
-            if is_gmm:
-                need = _n.lib().d3p_dpsvi_epoch_gmm_workspace_bytes(C.byref(desc), C.byref(probe))
-            elif is_vae:
-                need = _n.lib().d3p_dpsvi_epoch_vae_workspace_bytes(C.byref(desc), C.byref(probe), world)
-            else:
-                need = _n.lib().d3p_dpsvi_epoch_workspace_bytes(C.byref(desc), C.byref(probe))
+            need = fam._epoch_workspace_bytes(desc, probe, world)
             if need == 0:
                 raise _n.D3PNativeError("unsupported family / sampler configuration for run_epoch")
-            plan = (plan_key, spec, Xsrc, stride, ysrc, desc, sd, need)      # keeps `spec` (and its id) alive
+            plan = (plan_key, spec, data.x, data.stride, data.y, desc, sd, need)      # keeps `spec` (and its id) alive
             self._epoch_plan = plan
         _, _, Xsrc, stride, ysrc, desc, sd, need = plan
         perm = None
@@ -465,9 +481,7 @@ class DPSVI:
             if (first_step + num_steps) * spec["batch"] > perm.numel():
                 raise ValueError("run_epoch: the split batchifier has only num_records // batch_size batches per epoch")
             sd = _n.SamplerDesc(spec["kind"], spec["q"], spec["n_records"], spec["batch"], 0, perm.data_ptr())
-        if getattr(self, "_epoch_ws", None) is None or self._epoch_ws.numel() < need + 256 or self._epoch_ws.device != dev:
-            self._epoch_ws = torch.empty(need + 256, dtype=torch.uint8, device=dev)
-        ws_al = self._epoch_ws[(-self._epoch_ws.data_ptr()) % 256:]          # the VAE step wants 256-byte alignment
+        self._epoch_ws = ws = _aligned_scratch(getattr(self, "_epoch_ws", None), need)
         if self.peer_window is not None and spec["kind"] == _n.SAMPLER_POISSON:
             self.peer_window = self.peer_window.with_records(spec["n_records"])   # sharded selector draw
         ectx = self._epoch_ctx(dev.index)
@@ -481,54 +495,26 @@ class DPSVI:
             lr = os_.lr.clone() if os_.lr is not None else None
         lt_c = getattr(self, "_epoch_lt", None)
         if lt_c is None or lt_c[0] is not os_.layout:
-            lt = _n.LeafTable()
-            lt.n_leaves = len(os_.layout)
-            for l, (name, off, shape) in enumerate(os_.layout):
-                lt.leaf_off[l] = off
-                lt.leaf_len[l] = int(np.prod(shape)) if len(shape) else 1
-            self._epoch_lt = lt_c = (os_.layout, lt)
+            self._epoch_lt = lt_c = (os_.layout, _leaf_layout(os_.layout))
         lt = lt_c[1]
         od = self.optim.desc(os_.step, lr, desc.n_params)
         stats = torch.empty(num_steps, 3, dtype=torch.float32, device=dev)
         bkey = (np.zeros(16, np.uint32) if is_split else
                 np.ascontiguousarray(np.asarray(batchifier_state, dtype=np.uint32).reshape(16)))
         rkey = np.array(np.asarray(svi_state.rng_key, dtype=np.uint32).reshape(16), copy=True)
-        u32p = C.POINTER(C.c_uint32)
         comm = self.peer_window.ptr if self.shard is not None else None
+        rest = (int(first_step), int(num_steps), float(svi_state.observation_scale), float(self._clipping_threshold),
+                float(self._dp_scale), C.byref(lt), C.byref(od), _n.ptr(flat), _n.ptr(m), _n.ptr(v), _n.ptr(stats), comm,
+                _n.ptr(ws), need, ectx, _n.stream_ptr())
         if device_keys:
             bkey_d = torch.as_tensor(bkey.view(np.int32)).to(dev)
             rkey_d = torch.as_tensor(rkey.view(np.int32)).to(dev)
-            if is_vae:
-                _n.check(_n.lib().d3p_dpsvi_run_epoch_vae_dk(
-                    C.byref(desc), C.byref(sd), _n.ptr(Xsrc), stride, _n.ptr(bkey_d), _n.ptr(rkey_d), int(first_step),
-                    int(num_steps), float(svi_state.observation_scale), float(self._clipping_threshold),
-                    float(self._dp_scale), C.byref(lt), C.byref(od), _n.ptr(flat), _n.ptr(m), _n.ptr(v), _n.ptr(stats), comm,
-                    _n.ptr(ws_al), need, ectx, _n.stream_ptr()), "run_epoch_vae_dk")
-            else:
-                _n.check(_n.lib().d3p_dpsvi_run_epoch_meanfield_dk(
-                    C.byref(desc), C.byref(sd), _n.ptr(Xsrc), stride, _n.ptr(ysrc), _n.ptr(bkey_d), _n.ptr(rkey_d),
-                    int(first_step), int(num_steps), float(svi_state.observation_scale), float(self._clipping_threshold),
-                    float(self._dp_scale), C.byref(lt), C.byref(od), _n.ptr(flat), _n.ptr(m), _n.ptr(v), _n.ptr(stats), comm,
-                    _n.ptr(ws_al), need, ectx, _n.stream_ptr()), "run_epoch_dk")
+            fam._epoch(True, desc, sd, _n.ptr(Xsrc), stride, _n.ptr(ysrc), _n.ptr(bkey_d), _n.ptr(rkey_d), rest)
             rkey = rkey_d.cpu().numpy().view(np.uint32).copy()
-        elif is_gmm:
-            _n.check(_n.lib().d3p_dpsvi_run_epoch_gmm(
-                C.byref(desc), C.byref(sd), _n.ptr(Xsrc), stride, bkey.ctypes.data_as(u32p),
-                rkey.ctypes.data_as(u32p), int(first_step), int(num_steps), float(svi_state.observation_scale),
-                float(self._clipping_threshold), float(self._dp_scale), C.byref(lt), C.byref(od), _n.ptr(flat), _n.ptr(m),
-                _n.ptr(v), _n.ptr(stats), comm, _n.ptr(ws_al), need, ectx, _n.stream_ptr()), "run_epoch_gmm")
-        elif is_vae:
-            _n.check(_n.lib().d3p_dpsvi_run_epoch_vae(
-                C.byref(desc), C.byref(sd), _n.ptr(Xsrc), stride, bkey.ctypes.data_as(u32p),
-                rkey.ctypes.data_as(u32p), int(first_step), int(num_steps), float(svi_state.observation_scale),
-                float(self._clipping_threshold), float(self._dp_scale), C.byref(lt), C.byref(od), _n.ptr(flat), _n.ptr(m),
-                _n.ptr(v), _n.ptr(stats), comm, _n.ptr(ws_al), need, ectx, _n.stream_ptr()), "run_epoch_vae")
         else:
-            _n.check(_n.lib().d3p_dpsvi_run_epoch_meanfield(
-                C.byref(desc), C.byref(sd), _n.ptr(Xsrc), stride, _n.ptr(ysrc), bkey.ctypes.data_as(u32p),
-                rkey.ctypes.data_as(u32p), int(first_step), int(num_steps), float(svi_state.observation_scale),
-                float(self._clipping_threshold), float(self._dp_scale), C.byref(lt), C.byref(od), _n.ptr(flat), _n.ptr(m),
-                _n.ptr(v), _n.ptr(stats), comm, _n.ptr(ws_al), need, ectx, _n.stream_ptr()), "run_epoch")
+            u32p = C.POINTER(C.c_uint32)
+            fam._epoch(False, desc, sd, _n.ptr(Xsrc), stride, _n.ptr(ysrc), bkey.ctypes.data_as(u32p),
+                       rkey.ctypes.data_as(u32p), rest)
         new_os = OptimState(os_.step + num_steps, flat, m, v, os_.layout, lr)
         return DPSVIState(new_os, rkey.reshape(np.asarray(svi_state.rng_key).shape), svi_state.observation_scale), stats
 
