@@ -9,7 +9,9 @@ Two jobs, both guarded by ``available()``:
 * ``dump_golden(path)``      — outputs of the reference on fixed seeds (``tests/golden/make_reference_golden.py``
   writes ``tests/golden/reference_v1.npz``): ChaCha key plumbing (``PRNGKey/split/fold_in/random_bits/uniform/normal/
   randint/convert_to_jax_rng_key``), Feistel and Poisson indices, per-example Threefry keys and guide normals, jax
-  gamma draws, and 3-step ``DPSVI.update`` trajectories per model family.  ``tests/test_reference_golden.py`` holds the
+  gamma draws, 3-step ``DPSVI.update`` trajectories per model family, and 3-step logistic-regression trajectories with
+  numpyro's other optimizers and a scheduled Adam (``OPTIM_CASES``, keys ``optraj_*``).
+  ``tests/test_reference_golden.py`` (and ``tests/test_reference_optimizers.py`` for the ``optraj_*`` keys) holds the
   oracle and the CUDA path to that file: this is the one command that turns "parity unpinned" (the key-derivation rule
   of jax-chacha-prng, numpyro's seed plumbing, jax's gamma sampler: DESIGN.md section 8) into a pinned statement.
 
@@ -32,6 +34,28 @@ REF_DIRS = [os.path.join(ROOT, "baseline", "_ref")]
 NEEDED = ("jax", "numpyro", "chacha")
 
 SEEDS = (0, 1, 123, (1 << 40) + 5)
+
+# Optimizer cases of the short logistic-regression trajectories under the ``optraj_*`` keys: numpyro.optim class name,
+# positional and keyword arguments.  A step size given as (schedule name, args) is that schedule of
+# jax.example_libraries.optimizers (the oracle side: oracle/optim.py, same names).
+OPTIM_CASES = {
+    "momentum": ("Momentum", (1e-3, 0.9), {}),
+    "adagrad": ("Adagrad", (1e-2,), {"momentum": 0.8}),
+    "rmsprop": ("RMSProp", (1e-3,), {"gamma": 0.8}),
+    "rmsprop_momentum": ("RMSPropMomentum", (1e-3,), {"gamma": 0.8, "momentum": 0.7}),
+    "clipped_adam": ("ClippedAdam", (1e-3,), {"clip_norm": 10.0}),
+    "adam_exponential_decay": ("Adam", (("exponential_decay", (1e-3, 2, 0.5)),), {}),
+}
+
+
+def make_optim(spec, optim_module, schedule_module):
+    """An optimizer of ``OPTIM_CASES`` from ``optim_module`` (numpyro.optim or oracle.optim), its schedule (if any)
+    from ``schedule_module`` (jax.example_libraries.optimizers or oracle.optim)."""
+    cls, args, kwargs = spec
+    if args and isinstance(args[0], tuple):
+        name, sargs = args[0]
+        args = (getattr(schedule_module, name)(*sargs),) + tuple(args[1:])
+    return getattr(optim_module, cls)(*args, **kwargs)
 FOLD_DATA = (0, 1, 7, 1 << 31)
 
 
@@ -124,9 +148,11 @@ class ReferenceImpl:
             return ex.model, ex.guide, {}, 10.0
         raise ValueError(fam)
 
-    def trajectory(self, fam, data, mask, steps, seed, N, **shape):
+    def trajectory(self, fam, data, mask, steps, seed, N, optim=None, **shape):
         """3 masked ``DPSVI.update`` steps from ``svi.init`` on a fixed batch.  Returns the flat initial parameters
-        (jax pytree leaf order of the unconstrained param dict), and per step: loss, flat parameters, rng key."""
+        (jax pytree leaf order of the unconstrained param dict), and per step: loss, flat parameters, rng key.
+        ``optim``: an ``OPTIM_CASES`` entry (default: Adam(1e-3), as the examples)."""
+        import jax.example_libraries.optimizers as schedules
         import numpyro.optim as optimizers
         from numpyro.handlers import scale
         from numpyro.infer import Trace_ELBO
@@ -142,7 +168,8 @@ class ReferenceImpl:
         if fam == "vae":
             model, guide = scale(model, scale=1 / N), scale(guide, scale=1 / N)       # examples/vae.py:193-194
             kw = {"z_dim": shape["z_dim"], "hidden_dim": shape["hidden_dim"]}
-        svi = self.svi.DPSVI(model, guide, optimizers.Adam(1e-3), Trace_ELBO(), dp_scale=1.0, clipping_threshold=clip,
+        opt = optimizers.Adam(1e-3) if optim is None else make_optim(optim, optimizers, schedules)
+        svi = self.svi.DPSVI(model, guide, opt, Trace_ELBO(), dp_scale=1.0, clipping_threshold=clip,
                              num_obs_total=N, rng_suite=self.rng, **kw)
         batch = tuple(jnp.asarray(a) for a in data)
         state = svi.init(self.rng.PRNGKey(seed), *batch)
@@ -184,8 +211,8 @@ class OracleImpl:
     def threefry_normal(self, key2, n): return self.t.normal(np.asarray(key2, np.uint32), (n,))
     def threefry_gamma(self, key2, alpha): return self.g.gamma(np.asarray(key2, np.uint32), np.asarray(alpha, np.float32))
 
-    def trajectory(self, fam, data, mask, steps, seed, N, **shape):
-        from oracle import families, gmm, svi, vae
+    def trajectory(self, fam, data, mask, steps, seed, N, optim=None, **shape):
+        from oracle import families, gmm, optim as ooptim, svi, vae
         if fam == "logreg":
             f, clip = families.LogisticRegression(data[0].shape[1], N), 1.0
         elif fam == "gauss":
@@ -194,7 +221,8 @@ class OracleImpl:
             f, clip = gmm.GaussianMixture(shape["K"], data[0].shape[1], N), 20.0
         else:
             f, clip = vae.VAE(int(np.prod(data[0].shape[1:])), shape["hidden_dim"], shape["z_dim"], N), 10.0
-        s = svi.DPSVI(f, None, svi.Adam(1e-3), None, clip, 1.0)
+        opt = svi.Adam(1e-3) if optim is None else make_optim(optim, ooptim, ooptim)
+        s = svi.DPSVI(f, None, opt, None, clip, 1.0)
         p0 = f.init_params(0, 0.05) if fam == "vae" else f.init_params()
         st = s.init(self.c.PRNGKey(seed), *data, params=p0)
         order = f.flat_param_order()
@@ -276,6 +304,19 @@ def dump(impl, path, families=("logreg", "gauss", "gmm", "vae")):
         for s, leaves in enumerate(tr["params"]):
             for i, l in enumerate(leaves):
                 out[f"traj_{fam}_step{s}_{i}"] = l
+    # the other numpyro optimizers and one scheduled Adam, on the logistic-regression case
+    data, mask, N, shape = trajectory_inputs("logreg")
+    for name, spec in OPTIM_CASES.items():
+        try:
+            tr = impl.trajectory("logreg", data, mask, 3, 7, N, optim=spec, **shape)
+        except Exception as e:
+            skipped.append(f"optim {name}: {type(e).__name__}: {e}")
+            continue
+        out[f"optraj_{name}_loss"] = np.array(tr["loss"], np.float32)
+        out[f"optraj_{name}_rng_key"] = np.stack(tr["rng_key"])
+        for s, leaves in enumerate(tr["params"]):
+            for i, l in enumerate(leaves):
+                out[f"optraj_{name}_step{s}_{i}"] = l
     out["skipped"] = np.array("; ".join(skipped))
     np.savez_compressed(path, **out)
     return sorted(out)

@@ -16,6 +16,10 @@ ERR_PEER_TIMEOUT = -5
 FAMILY_LOGREG, FAMILY_GAUSS = 0, 1
 LINK_EXP, LINK_SOFTPLUS = 0, 1
 OPT_NONE, OPT_SGD, OPT_ADAM, OPT_ADADP = 0, 1, 2, 3
+OPT_MOMENTUM, OPT_ADAGRAD, OPT_RMSPROP, OPT_RMSPROP_MOMENTUM, OPT_CLIPPED_ADAM = 4, 5, 6, 7, 8
+OPT_SCHEDULED = 0x100
+SCHED_CONSTANT, SCHED_EXPONENTIAL, SCHED_INVERSE_TIME, SCHED_POLYNOMIAL, SCHED_PIECEWISE = 0, 1, 2, 3, 4
+MAX_BOUNDARIES = 16
 
 
 class MeanfieldDesc(C.Structure):
@@ -45,7 +49,12 @@ class LeafTable(C.Structure):
 class OptimDesc(C.Structure):
     _fields_ = [("kind", C.c_int32), ("step_size", C.c_float), ("b1", C.c_float), ("b2", C.c_float),
                 ("eps", C.c_float), ("step", C.c_int32), ("tol", C.c_float), ("stability_check", C.c_int32),
-                ("lr_d", C.c_void_p), ("err_ws_d", C.c_void_p)]
+                ("lr_d", C.c_void_p), ("err_ws_d", C.c_void_p),
+                # appended: read only for kinds OPT_MOMENTUM .. OPT_CLIPPED_ADAM or with OPT_SCHEDULED
+                ("momentum", C.c_float), ("gamma", C.c_float), ("clip_norm", C.c_float), ("schedule", C.c_int32),
+                ("decay_steps", C.c_float), ("decay_rate", C.c_float), ("staircase", C.c_int32),
+                ("final_step_size", C.c_float), ("power", C.c_float), ("n_boundaries", C.c_uint32),
+                ("boundaries", C.c_float * MAX_BOUNDARIES), ("values", C.c_float * (MAX_BOUNDARIES + 1))]
 
 
 class SamplerDesc(C.Structure):
@@ -94,6 +103,7 @@ _SIGNATURES = {
                                              C.c_float, C.c_float, C.c_float, C.c_int32, _vp,
                                              C.POINTER(OptimDesc), _vp, _vp, _vp, _vp,
                                              C.POINTER(C.c_float), _vp]),
+    "d3p_optim_step_size": (C.c_int32, [C.POINTER(OptimDesc), C.c_int32, C.POINTER(C.c_float)]),
     "d3p_adadp_workspace_floats": (C.c_size_t, [C.c_uint32]),
     "d3p_adadp_finish_f32": (C.c_int32, [C.POINTER(OptimDesc), C.c_uint32, _vp, _vp, _vp]),
     "d3p_dpsvi_epoch_workspace_bytes": (C.c_size_t, [C.POINTER(MeanfieldDesc), C.POINTER(SamplerDesc)]),

@@ -199,6 +199,8 @@ int32_t run_epoch(const StepLauncher& fam, const d3p_sampler_desc* sampler, cons
   if (!fam.x || !fam.params || (dk ? !batch_key_d : ((!split && !batch_key_h) || !rng_key_io_h)) || !leaves_h ||
       !optim_io_h || !ws_d)
     return D3P_ERR_INVALID_ARGUMENT;
+  // a descriptor the finalize would refuse is refused before the first step kernel is queued
+  if (const int32_t rc = optim_check(optim_io_h, fam.params, m_d, v_d); rc != D3P_OK) return rc;
   if (fam.vae && (reinterpret_cast<uintptr_t>(ws_d) & 255)) return D3P_ERR_INVALID_ARGUMENT;
   if (split && (uint64_t)(first_step + n_steps) * sampler->batch > sampler->n_records) return D3P_ERR_INVALID_ARGUMENT;
   if (!sampler_ok(sampler) || leaves_h->n_leaves == 0 || leaves_h->n_leaves > D3P_MAX_LEAVES)

@@ -1,7 +1,8 @@
 // K8: fixed-order reduction of the per-CTA partial sums + mean + ChaCha20 Gaussian perturbation
 // + rescale + optimizer step, in one launch.  Replaces DPSVI._combine_gradients
 // (d3p/svi.py:327-348), _perturb_and_reassemble_gradients (:350-377), perturbation_function
-// (:470-498) and _apply_gradient (:379-393) with numpyro.optim.SGD / Adam.
+// (:470-498) and _apply_gradient (:379-393) with numpyro.optim.SGD / Adam / Momentum / Adagrad / RMSProp /
+// RMSPropMomentum / ClippedAdam and d3p's ADADP.
 #include "comm.cuh"
 #include "common.cuh"
 #include "launch.cuh"
@@ -20,8 +21,10 @@ struct FinalizeArgs {
   float dp_scale, C, obs_scale;
   int add_noise;
   float* grad_out;
-  int opt_kind;
-  float step_size, b1, b2, eps;
+  int opt_kind;        // D3P_OPT_* without D3P_OPT_SCHEDULED
+  float step_size;     // lr of this step: the schedule is evaluated on the host, once per launch
+  float b1, b2, eps;
+  float mom, gamma, clip;   // MOMENTUM .. CLIPPED_ADAM (header)
   int step;
   float* params;
   float* m;
@@ -48,6 +51,61 @@ D3P_D float adadp_element(const FinalizeArgs& a, float lr, uint32_t j, float x, 
   return e * e;
 }
 
+// Which old state an optimizer kind reads (ADADP's is handled by adadp_element).
+__host__ __device__ inline bool opt_uses_x(int k) { return k != D3P_OPT_NONE && k != D3P_OPT_ADADP; }
+__host__ __device__ inline bool opt_uses_m(int k) {
+  return k == D3P_OPT_ADAM || k == D3P_OPT_MOMENTUM || k == D3P_OPT_ADAGRAD || k == D3P_OPT_RMSPROP_MOMENTUM ||
+         k == D3P_OPT_CLIPPED_ADAM;
+}
+__host__ __device__ inline bool opt_uses_v(int k) {
+  return k == D3P_OPT_ADAM || k == D3P_OPT_ADAGRAD || k == D3P_OPT_RMSPROP || k == D3P_OPT_RMSPROP_MOMENTUM ||
+         k == D3P_OPT_CLIPPED_ADAM;
+}
+
+// One element of the numpyro optimizers (jax.example_libraries.optimizers; header, D3P_OPT_*): x, m, v are the old
+// state, loaded by the kernel's prologue; bc1 / bc2 are Adam's bias corrections of this step.
+D3P_D void optim_element(const FinalizeArgs& a, float bc1, float bc2, uint32_t j, float g, float x, float m, float v,
+                         float* __restrict__ prm, float* __restrict__ pm, float* __restrict__ pv) {
+  // (an if-chain; NONE and ADADP do nothing here.  finalize_quad_kernel keeps its own SGD and Adam branches, which
+  // compile to exactly the arithmetic they had before the other kinds existed, and calls this after them: written as
+  // a switch, or ahead of its ADADP branch, it costs that kernel 21 registers and one CTA per SM)
+  const int k = a.opt_kind;
+  if (k == D3P_OPT_SGD) {
+    prm[j] = x - a.step_size * g;
+  } else if (k == D3P_OPT_ADAM || k == D3P_OPT_CLIPPED_ADAM) {
+    // jnp.clip (a NaN stays NaN); only the moments see the clipped value, grad_out got g already
+    if (k == D3P_OPT_CLIPPED_ADAM) g = g < -a.clip ? -a.clip : (g > a.clip ? a.clip : g);
+    m = (1.0f - a.b1) * g + a.b1 * m;
+    v = (1.0f - a.b2) * (g * g) + a.b2 * v;
+    float mhat = m / bc1;
+    float vhat = v / bc2;
+    prm[j] = x - a.step_size * mhat / (sqrtf(vhat) + a.eps);
+    pm[j] = m;
+    pv[j] = v;
+  } else if (k == D3P_OPT_MOMENTUM) {
+    m = a.mom * m + g;
+    prm[j] = x - a.step_size * m;
+    pm[j] = m;
+  } else if (k == D3P_OPT_ADAGRAD) {
+    v = v + g * g;
+    const float r = v > 0.f ? 1.0f / sqrtf(v) : 0.f;     // an element that never had a gradient: 0, not 0 * inf
+    m = (1.0f - a.mom) * (g * r) + a.mom * m;
+    prm[j] = x - a.step_size * m;
+    pm[j] = m;
+    pv[j] = v;
+  } else if (k == D3P_OPT_RMSPROP) {
+    v = v * a.gamma + (g * g) * (1.0f - a.gamma);
+    prm[j] = x - a.step_size * g / sqrtf(v + a.eps);     // eps inside the root
+    pv[j] = v;
+  } else if (k == D3P_OPT_RMSPROP_MOMENTUM) {
+    v = v * a.gamma + (g * g) * (1.0f - a.gamma);
+    m = a.mom * m + a.step_size * g / sqrtf(v + a.eps);
+    prm[j] = x - m;
+    pm[j] = m;
+    pv[j] = v;
+  }
+}
+
 constexpr int kFinThreads = 512;   // 16 warps share the partial rows of a 32-column strip: the row loop is latency-bound
 
 // site states live in constant-bank kernel parameters next to the leaf table
@@ -66,7 +124,8 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const __grid_cons
   // Launched as a programmatic dependent of the step kernel, this CTA is resident while that kernel is still running.
   // Everything that does not depend on its partial rows happens NOW, under the producer's tail instead of behind it:
   // the column's Gaussian draw (a ChaCha block: keys only), the Adam bias corrections and the loads of the parameter
-  // and its moments (written by the previous finalize, which completed before the step kernel started).
+  // and the optimizer state its kind keeps (written by the previous finalize, which completed before the step kernel
+  // started).
   float xi_pre = 0.f, x_pre = 0.f, m_pre = 0.f, v_pre = 0.f, bc1 = 1.f, bc2 = 1.f;
   bool have_xi = false;
   {
@@ -90,9 +149,10 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const __grid_cons
           have_xi = true;
         }
       }
-      if (a.opt_kind == D3P_OPT_SGD || a.opt_kind == D3P_OPT_ADAM) x_pre = a.params[jp];
-      if (a.opt_kind == D3P_OPT_ADAM) {
-        m_pre = a.m[jp]; v_pre = a.v[jp];
+      if (opt_uses_x(a.opt_kind)) x_pre = a.params[jp];
+      if (opt_uses_m(a.opt_kind)) m_pre = a.m[jp];
+      if (opt_uses_v(a.opt_kind)) v_pre = a.v[jp];
+      if (a.opt_kind == D3P_OPT_ADAM || a.opt_kind == D3P_OPT_CLIPPED_ADAM) {
         const float t = (float)(a.step + 1);
         bc1 = 1.0f - powf(a.b1, t); bc2 = 1.0f - powf(a.b2, t);
       }
@@ -171,19 +231,8 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const __grid_cons
     if (have_xi) g = __fadd_rn(g, __fmul_rn(xi_pre, sigma));          // svi.py:485-486 (drawn in the prologue)
     g = __fmul_rn(__fmul_rn(g, a.obs_scale), f);                       // svi.py:374-375
     if (a.grad_out) a.grad_out[j] = g;
-    if (a.opt_kind == D3P_OPT_SGD) {
-      a.params[j] = x_pre - a.step_size * g;
-    } else if (a.opt_kind == D3P_OPT_ADAM) {
-      float m = (1.0f - a.b1) * g + a.b1 * m_pre;
-      float v = (1.0f - a.b2) * (g * g) + a.b2 * v_pre;
-      float mhat = m / bc1;
-      float vhat = v / bc2;
-      a.params[j] = x_pre - a.step_size * mhat / (sqrtf(vhat) + a.eps);
-      a.m[j] = m;
-      a.v[j] = v;
-    } else if (a.opt_kind == D3P_OPT_ADADP) {
-      err2 = adadp_element(a, *a.lr, j, a.params[j], g);
-    }
+    optim_element(a, bc1, bc2, j, g, x_pre, m_pre, v_pre, a.params, a.m, a.v);
+    if (a.opt_kind == D3P_OPT_ADADP) err2 = adadp_element(a, *a.lr, j, a.params[j], g);
   }
   if (a.opt_kind == D3P_OPT_ADADP && (a.step & 1)) {
     err2 = group_sum<32>(err2);
@@ -256,8 +305,8 @@ __global__ void __launch_bounds__(256) finalize_quad_kernel(const __grid_constan
     jj[i] = off + (ok[i] ? e : 0u);
     sum[i] = 0.f;
     x[i] = (ok[i] && a.opt_kind != D3P_OPT_NONE) ? prm[jj[i]] : 0.f;
-    m0[i] = (ok[i] && a.opt_kind == D3P_OPT_ADAM) ? pm[jj[i]] : 0.f;
-    v0[i] = (ok[i] && a.opt_kind == D3P_OPT_ADAM) ? pv[jj[i]] : 0.f;
+    m0[i] = (ok[i] && opt_uses_m(a.opt_kind)) ? pm[jj[i]] : 0.f;
+    v0[i] = (ok[i] && opt_uses_v(a.opt_kind)) ? pv[jj[i]] : 0.f;
   }
   // The partial rows are requested before the ChaCha rounds below.  Up to 4 rows (the VAE's concurrent wave writes 4)
   // are only LOADED here and added after the rounds, so that the 200 dependent instructions of the rounds run under
@@ -346,8 +395,9 @@ __global__ void __launch_bounds__(256) finalize_quad_kernel(const __grid_constan
       prm[j] = x[i] - a.step_size * mhat / (sqrtf(vhat) + a.eps);
       pm[j] = m;
       pv[j] = v;
-    } else if (a.opt_kind == D3P_OPT_ADADP) {
-      err2 += adadp_element(a, lr_adadp, j, x[i], g);
+    } else {                                                     // the other kinds (and ADADP)
+      optim_element(a, bc1, bc2, j, g, x[i], m0[i], v0[i], prm, pm, pv);
+      if (a.opt_kind == D3P_OPT_ADADP) err2 += adadp_element(a, lr_adadp, j, x[i], g);
     }
   }
   if (adadp_odd) {                                              // fixed-order CTA sum of the error terms
@@ -424,6 +474,58 @@ extern "C" int32_t d3p_reduce_partials_f32(const float* partials_d, uint32_t n_p
   return check_launch();
 }
 
+// jax.example_libraries.optimizers' schedules (constant, exponential_decay, inverse_time_decay, polynomial_decay,
+// piecewise_constant), restated in float32.
+extern "C" int32_t d3p_optim_step_size(const d3p_optim_desc* o, int32_t step, float* out_h) {
+  if (!o || !out_h) return D3P_ERR_INVALID_ARGUMENT;
+  const int32_t kind = o->kind & ~D3P_OPT_SCHEDULED;
+  if (kind < D3P_OPT_NONE || kind > D3P_OPT_CLIPPED_ADAM) return D3P_ERR_UNSUPPORTED;
+  if (kind == D3P_OPT_CLIPPED_ADAM && !(o->clip_norm > 0.f)) return D3P_ERR_INVALID_ARGUMENT;
+  if (!(o->kind & D3P_OPT_SCHEDULED)) { *out_h = o->step_size; return D3P_OK; }
+  if (kind == D3P_OPT_NONE || kind == D3P_OPT_ADADP || step < 0) return D3P_ERR_INVALID_ARGUMENT;
+  const float s = o->step_size, i = (float)step, ds = o->decay_steps;
+  switch (o->schedule) {
+    case D3P_SCHED_CONSTANT:
+      *out_h = s;
+      return D3P_OK;
+    case D3P_SCHED_EXPONENTIAL:
+    case D3P_SCHED_INVERSE_TIME:
+    case D3P_SCHED_POLYNOMIAL:
+      if (!(ds > 0.f)) return D3P_ERR_INVALID_ARGUMENT;
+      break;
+    case D3P_SCHED_PIECEWISE:
+      if (o->n_boundaries > D3P_MAX_BOUNDARIES) return D3P_ERR_INVALID_ARGUMENT;
+      break;
+    default:
+      return D3P_ERR_UNSUPPORTED;
+  }
+  if (o->schedule == D3P_SCHED_EXPONENTIAL) {
+    *out_h = s * powf(o->decay_rate, i / ds);
+  } else if (o->schedule == D3P_SCHED_INVERSE_TIME) {
+    *out_h = o->staircase ? s / (1.f + o->decay_rate * floorf(i / ds)) : s / (1.f + o->decay_rate * i / ds);
+  } else if (o->schedule == D3P_SCHED_POLYNOMIAL) {
+    const float n = fminf(i, ds);
+    const float mult = powf(1.f - n / ds, o->power);
+    *out_h = mult * (s - o->final_step_size) + o->final_step_size;
+  } else {
+    uint32_t k = 0;
+    for (uint32_t b = 0; b < o->n_boundaries; ++b) k += i > o->boundaries[b] ? 1u : 0u;
+    *out_h = o->values[k];
+  }
+  return D3P_OK;
+}
+
+int32_t d3p::optim_check(const d3p_optim_desc* o, const float* params_d, const float* m_d, const float* v_d) {
+  if (!o) return D3P_OK;
+  const int32_t kind = o->kind & ~D3P_OPT_SCHEDULED;
+  if (kind != D3P_OPT_NONE && !params_d) return D3P_ERR_INVALID_ARGUMENT;
+  if ((opt_uses_m(kind) && !m_d) || (opt_uses_v(kind) && !v_d)) return D3P_ERR_INVALID_ARGUMENT;
+  if (kind == D3P_OPT_ADADP && (!m_d || !v_d || !o->lr_d || !o->err_ws_d || o->step < 0))
+    return D3P_ERR_INVALID_ARGUMENT;
+  float lr;
+  return d3p_optim_step_size(o, o->step, &lr);
+}
+
 extern "C" int32_t d3p_perturb_finalize_f32(const float* partials_d, uint32_t n_partials, uint32_t P, uint32_t B,
                                             const d3p_leaf_table* leaves_h, float dp_scale, float C, float obs_scale,
                                             int32_t add_noise, float* grad_out_d, const d3p_optim_desc* optim_h,
@@ -446,22 +548,22 @@ int32_t d3p::perturb_finalize_impl(const float* partials_d, uint32_t n_partials,
   a.partials = partials_d; a.n_partials = n_partials; a.P = P; a.B = B;
   a.dp_scale = dp_scale; a.C = C; a.obs_scale = obs_scale; a.add_noise = add_noise;
   a.grad_out = grad_out_d;
-  a.opt_kind = optim_h ? optim_h->kind : D3P_OPT_NONE;
-  a.step_size = optim_h ? optim_h->step_size : 0.f;
+  if (const int32_t rc = optim_check(optim_h, params_d, m_d, v_d); rc != D3P_OK) return rc;
+  a.opt_kind = optim_h ? optim_h->kind & ~D3P_OPT_SCHEDULED : D3P_OPT_NONE;
+  a.step_size = 0.f;
+  if (optim_h) d3p_optim_step_size(optim_h, optim_h->step, &a.step_size);   // validated by optim_check
   a.b1 = optim_h ? optim_h->b1 : 0.f; a.b2 = optim_h ? optim_h->b2 : 0.f; a.eps = optim_h ? optim_h->eps : 0.f;
+  const bool appended = a.opt_kind >= D3P_OPT_MOMENTUM;     // fields past err_ws_d exist only for the new kinds
+  a.mom = appended ? optim_h->momentum : 0.f;
+  a.gamma = appended ? optim_h->gamma : 0.f;
+  a.clip = appended ? optim_h->clip_norm : 0.f;
   a.step = optim_h ? optim_h->step : 0;
   a.params = params_d; a.m = m_d; a.v = v_d; a.stats = stats_d;
   a.use_override = nf_override_h ? 1 : 0;
   a.n_override = nf_override_h ? nf_override_h[0] : 0.f;
   a.f_override = nf_override_h ? nf_override_h[1] : 0.f;
-  if (a.opt_kind != D3P_OPT_NONE && !params_d) return D3P_ERR_INVALID_ARGUMENT;
-  if (a.opt_kind == D3P_OPT_ADAM && (!m_d || !v_d)) return D3P_ERR_INVALID_ARGUMENT;
   a.lr = nullptr; a.err_ws = nullptr;
-  if (a.opt_kind == D3P_OPT_ADADP) {
-    if (!m_d || !v_d || !optim_h->lr_d || !optim_h->err_ws_d || a.step < 0) return D3P_ERR_INVALID_ARGUMENT;
-    a.lr = optim_h->lr_d; a.err_ws = optim_h->err_ws_d;
-  }
-  if (a.opt_kind < D3P_OPT_NONE || a.opt_kind > D3P_OPT_ADADP) return D3P_ERR_UNSUPPORTED;
+  if (a.opt_kind == D3P_OPT_ADADP) { a.lr = optim_h->lr_d; a.err_ws = optim_h->err_ws_d; }
   LeafTable lt;
   SiteStates ss;
   CommDev cd;

@@ -58,5 +58,8 @@ int32_t perturb_finalize_impl(const float* partials_d, uint32_t n_partials, uint
                               float obs_scale, int32_t add_noise, float* grad_out_d, const d3p_optim_desc* optim_h,
                               float* params_d, float* m_d, float* v_d, float* stats_d, const float* nf_override_h,
                               d3p_comm* comm, void* stream);
+// The optimizer checks of perturb_finalize_impl (descriptor as d3p_optim_step_size, plus the state buffers its kind
+// needs), for callers that want to refuse a bad descriptor before they launch anything.
+int32_t optim_check(const d3p_optim_desc* optim_h, const float* params_d, const float* m_d, const float* v_d);
 
 }  // namespace d3p

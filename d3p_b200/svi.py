@@ -435,8 +435,10 @@ class DPSVI:
         For the model families fed by ``poisson_batchify_data`` / ``subsample_batchify_data`` /
         ``split_batchify_data`` the whole loop runs inside the family's ``d3p_dpsvi_run_epoch_*`` driver (no
         interpreter between launches); the result is bit-identical to the step-by-step calls, which remain the path for
-        everything else (NCCL-backend sharded runs, custom batchifiers, and the key modes or sharded runs a family has
-        no driver for: ``Family.epoch_device_keys`` / ``Family.epoch_sharded``).
+        everything else (NCCL-backend sharded runs, custom batchifiers, the key modes or sharded runs a family has
+        no driver for: ``Family.epoch_device_keys`` / ``Family.epoch_sharded``, and an optimizer whose step size is a
+        Python callable other than the named schedules of ``d3p_b200.optimizers``, which the C driver cannot call).
+        Either way a schedule is evaluated at the optimizer's own step counter, not at ``first_step``.
 
         ``device_keys=True`` drives the ``*_dk`` entry points: the batchifier key and the state key are uploaded once
         and every per-step key is derived on the device (what a jitted caller with traced keys binds to, see
@@ -448,7 +450,7 @@ class DPSVI:
         fused = (spec is not None and fam is not None and (fam.epoch_device_keys or not device_keys)
                  and (self.shard is None or (fam.epoch_sharded and self.shard[2] is None))
                  and self._rng_suite is strong_rng and spec["rng_suite"] is strong_rng and self.event_hook is None
-                 and num_steps > 0)
+                 and getattr(self.optim, "fused_epoch", True) and num_steps > 0)
         if not fused:
             stats = torch.zeros(max(num_steps, 0), 3, dtype=torch.float32, device=_dev())
             for s in range(num_steps):

@@ -187,6 +187,28 @@ int32_t d3p_dpsvi_step_meanfield(const d3p_meanfield_desc* desc, const float* pa
 #define D3P_OPT_SGD 1
 #define D3P_OPT_ADAM 2
 #define D3P_OPT_ADADP 3 /* d3p.optimizers.ADADP (d3p/optimizers.py:29-131) */
+/* numpyro.optim wrappers of jax.example_libraries.optimizers; g = the released noisy gradient, lr = step_size(i):
+ *   MOMENTUM          m = momentum * m + g;                           x -= lr * m            (momentum = numpyro's mass)
+ *   ADAGRAD           v += g^2; r = v > 0 ? 1 / sqrt(v) : 0;
+ *                     m = (1 - momentum) * (g * r) + momentum * m;     x -= lr * m
+ *   RMSPROP           v = v * gamma + g^2 * (1 - gamma);               x -= lr * g / sqrt(v + eps)
+ *   RMSPROP_MOMENTUM  v as RMSPROP; m = momentum * m + lr * g / sqrt(v + eps);  x -= m
+ *   CLIPPED_ADAM      Adam (b1, b2, eps) on clip(g, -clip_norm, clip_norm); grad_out_d still receives g */
+#define D3P_OPT_MOMENTUM 4
+#define D3P_OPT_ADAGRAD 5
+#define D3P_OPT_RMSPROP 6
+#define D3P_OPT_RMSPROP_MOMENTUM 7
+#define D3P_OPT_CLIPPED_ADAM 8
+/* OR-ed into `kind`: step_size is the schedule `schedule` (fields below) evaluated at `step`, not a constant.  Not
+ * valid with NONE or ADADP (whose step size is device state). */
+#define D3P_OPT_SCHEDULED 0x100
+/* Step-size schedules of jax.example_libraries.optimizers, s = step_size, i = step, float32 arithmetic: */
+#define D3P_SCHED_CONSTANT 0     /* s                                                                              */
+#define D3P_SCHED_EXPONENTIAL 1  /* s * decay_rate ** (i / decay_steps)                                            */
+#define D3P_SCHED_INVERSE_TIME 2 /* s / (1 + decay_rate * i / decay_steps); staircase: i / decay_steps floored     */
+#define D3P_SCHED_POLYNOMIAL 3   /* n = min(i, decay_steps): (1 - n / decay_steps) ** power * (s - final) + final  */
+#define D3P_SCHED_PIECEWISE 4    /* values[#{b in boundaries : i > b}]                                             */
+#define D3P_MAX_BOUNDARIES 16
 
 typedef struct {
   uint32_t n_leaves;
@@ -206,7 +228,28 @@ typedef struct {
   int32_t stability_check; /* reject the odd step when err > tol (optimizers.py:92-97)       */
   float* lr_d;             /* device scalar: current step size, updated by d3p_adadp_finish  */
   float* err_ws_d;         /* device scratch, >= d3p_adadp_workspace_floats(P) floats        */
+  /* Appended fields: read only when `kind` names MOMENTUM .. CLIPPED_ADAM or carries D3P_OPT_SCHEDULED, so a caller
+   * that knows only the fields above never has them read. */
+  float momentum;          /* MOMENTUM: mass; ADAGRAD, RMSPROP_MOMENTUM: momentum             */
+  float gamma;             /* RMSPROP, RMSPROP_MOMENTUM: decay of the squared-gradient average */
+  float clip_norm;         /* CLIPPED_ADAM: element-wise clip bound (> 0)                     */
+  int32_t schedule;        /* D3P_SCHED_* (with D3P_OPT_SCHEDULED)                            */
+  float decay_steps;       /* EXPONENTIAL, INVERSE_TIME, POLYNOMIAL (> 0)                     */
+  float decay_rate;        /* EXPONENTIAL, INVERSE_TIME                                       */
+  int32_t staircase;       /* INVERSE_TIME                                                    */
+  float final_step_size;   /* POLYNOMIAL                                                      */
+  float power;             /* POLYNOMIAL                                                      */
+  uint32_t n_boundaries;   /* PIECEWISE: <= D3P_MAX_BOUNDARIES                                */
+  float boundaries[D3P_MAX_BOUNDARIES];
+  float values[D3P_MAX_BOUNDARIES + 1]; /* PIECEWISE: n_boundaries + 1 step sizes            */
 } d3p_optim_desc;
+
+/* The step size of `optim_h` at optimizer step `step` (its own counter, starting at 0): step_size, or with
+ * D3P_OPT_SCHEDULED the schedule, evaluated in float32 on the host.  d3p_perturb_finalize_* evaluate it this way once
+ * per launch.  Also validates the descriptor: unknown kind or schedule -> D3P_ERR_UNSUPPORTED; D3P_OPT_SCHEDULED on
+ * NONE / ADADP, step < 0, decay_steps <= 0, n_boundaries > D3P_MAX_BOUNDARIES or a clip_norm that is not > 0 ->
+ * D3P_ERR_INVALID_ARGUMENT. */
+int32_t d3p_optim_step_size(const d3p_optim_desc* optim_h, int32_t step, float* out_h);
 
 /* ADADP needs the global error norm before an odd step can be accepted, so an odd step is two
  * launches: d3p_perturb_finalize_f32 (kind = D3P_OPT_ADADP, odd `step`) stores the tentative
@@ -270,7 +313,9 @@ int32_t d3p_dpsvi_run_epoch_meanfield(const d3p_meanfield_desc* desc, const d3p_
  *   loss = (loss_sum / B) * f                                          (d3p/svi.py:306,342)
  * xi ~ N(0, 1) from the ChaCha stream of the leaf's site state (counter from 0).
  * grad_out_d[P] (may be NULL) receives grad; if optim->kind != NONE, params_d / m_d / v_d are
- * updated in place (numpyro.optim.SGD / Adam, d3p/svi.py:379-393).
+ * updated in place (d3p/svi.py:379-393 with numpyro.optim.SGD / Adam / Momentum / Adagrad / RMSProp /
+ * RMSPropMomentum / ClippedAdam or d3p's ADADP; m_d holds the first-moment / velocity / momentum state, v_d the
+ * squared-gradient state, and a kind that keeps one of them needs its pointer).
  * stats_d[3] (may be NULL) = { loss, n, f }.
  * nf_override_h (may be NULL) = { n, f } supplied by the caller instead of the counts in the
  * partials — the stage-method form DPSVI._perturb_and_reassemble_gradients(state, key,
