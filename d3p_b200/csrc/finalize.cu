@@ -63,20 +63,25 @@ __host__ __device__ inline bool opt_uses_v(int k) {
 }
 
 // One element of the numpyro optimizers (jax.example_libraries.optimizers; header, D3P_OPT_*): x, m, v are the old
-// state, loaded by the kernel's prologue; bc1 / bc2 are Adam's bias corrections of this step.
+// state, loaded by the kernel's prologue; bc1 / bc2 are Adam's bias corrections of this step.  quad_adam: Adam's
+// moments are rounded as finalize_quad_kernel has always rounded them, fma(g, 1 - b1, b1 * m) and
+// fma(g * g, 1 - b2, b2 * v).  Everywhere else (finalize_kernel, and ClippedAdam in both kernels) the compiler
+// contracts the plain expressions the other way round, fma(m, b1, (1 - b1) * g): the two differ in the last bit.
 D3P_D void optim_element(const FinalizeArgs& a, float bc1, float bc2, uint32_t j, float g, float x, float m, float v,
-                         float* __restrict__ prm, float* __restrict__ pm, float* __restrict__ pv) {
-  // (an if-chain; NONE and ADADP do nothing here.  finalize_quad_kernel keeps its own SGD and Adam branches, which
-  // compile to exactly the arithmetic they had before the other kinds existed, and calls this after them: written as
-  // a switch, or ahead of its ADADP branch, it costs that kernel 21 registers and one CTA per SM)
-  const int k = a.opt_kind;
+                         float* __restrict__ prm, float* __restrict__ pm, float* __restrict__ pv, bool quad_adam) {
+  const int k = a.opt_kind;                              // NONE and ADADP do nothing here
   if (k == D3P_OPT_SGD) {
     prm[j] = x - a.step_size * g;
   } else if (k == D3P_OPT_ADAM || k == D3P_OPT_CLIPPED_ADAM) {
     // jnp.clip (a NaN stays NaN); only the moments see the clipped value, grad_out got g already
     if (k == D3P_OPT_CLIPPED_ADAM) g = g < -a.clip ? -a.clip : (g > a.clip ? a.clip : g);
-    m = (1.0f - a.b1) * g + a.b1 * m;
-    v = (1.0f - a.b2) * (g * g) + a.b2 * v;
+    if (quad_adam && k == D3P_OPT_ADAM) {
+      m = __fmaf_rn(1.0f - a.b1, g, __fmul_rn(a.b1, m));
+      v = __fmaf_rn(1.0f - a.b2, __fmul_rn(g, g), __fmul_rn(a.b2, v));
+    } else {
+      m = (1.0f - a.b1) * g + a.b1 * m;
+      v = (1.0f - a.b2) * (g * g) + a.b2 * v;
+    }
     float mhat = m / bc1;
     float vhat = v / bc2;
     prm[j] = x - a.step_size * mhat / (sqrtf(vhat) + a.eps);
@@ -106,7 +111,121 @@ D3P_D void optim_element(const FinalizeArgs& a, float bc1, float bc2, uint32_t j
   }
 }
 
+// Adam's bias corrections of this step (bc1 / bc2 are left alone for the other kinds).
+D3P_D void adam_bias(const FinalizeArgs& a, float& bc1, float& bc2) {
+  if (a.opt_kind == D3P_OPT_ADAM || a.opt_kind == D3P_OPT_CLIPPED_ADAM) {
+    const float t = (float)(a.step + 1);
+    bc1 = 1.0f - powf(a.b1, t); bc2 = 1.0f - powf(a.b2, t);
+  }
+}
+
+// Fixed-order CTA sum of the partial rows' (count, loss) columns: rows strided over the NT threads, a shuffle tree per
+// warp, then thread 0 adds the warp sums in warp order into s_n / s_loss.  The caller synchronizes before reading them.
+template <int NT>
+D3P_D void reduce_count_loss(const FinalizeArgs& a, float (&red)[2][NT / 32], float& s_n, float& s_loss) {
+  const uint32_t stride = a.P + 2;
+  float cnt = 0.f, loss = 0.f;
+  for (uint32_t p = threadIdx.x; p < a.n_partials; p += NT) {
+    loss += a.partials[(size_t)p * stride + a.P];
+    cnt += a.partials[(size_t)p * stride + a.P + 1];
+  }
+  cnt = group_sum<32>(cnt);
+  loss = group_sum<32>(loss);
+  if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = cnt; red[1][threadIdx.x >> 5] = loss; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float c = 0.f, l = 0.f;
+#pragma unroll
+    for (int w = 0; w < NT / 32; ++w) { c += red[0][w]; l += red[1][w]; }
+    s_n = c; s_loss = l;
+  }
+}
+
+// One-shot all-reduce of the CTA's (n, loss) over NVLink peer memory (comm.cuh): thread 0 pushes them as tagged words
+// jn, jn + 1 to every peer, every thread polls its own window for the peers' copies and adds all copies in rank order
+// (identical on every rank).  Returns the start value of the caller's per-column sums: 0, or NaN when an earlier
+// time-out on this rank (sampler counts, a previous exchange) has poisoned everything from here on.  The caller pushes
+// its columns first and adds them in rank order after this.
+D3P_D float exchange_n_loss(const CommDev& comm, float& n, float& loss) {
+  const float my_n = n, my_loss = loss;
+  const size_t jn = comm.extra_off + 2 * (size_t)blockIdx.x;
+  if (threadIdx.x == 0) { ll_push(comm, jn, my_n); ll_push(comm, jn + 1, my_loss); }
+  const float zero = comm_poisoned(comm) ? __uint_as_float(0x7fc00000u) : 0.f;
+  n = 0.f; loss = zero;
+  for (int r = 0; r < comm.world; ++r) {
+    const bool me = r == comm.rank;
+    n += me ? my_n : ll_wait(comm, r, jn);
+    loss += me ? my_loss : ll_wait(comm, r, jn + 1);
+  }
+  return zero;
+}
+
 constexpr int kFinThreads = 512;   // 16 warps share the partial rows of a 32-column strip: the row loop is latency-bound
+
+// Fixed-order sum of column j over n_rows rows (kFinThreads threads, 32 columns per CTA): warp w adds rows w, w + 16,
+// ... in row order, four loads in flight, and warp 0 adds the 16 warp sums in warp order.  The result is warp 0's.
+D3P_D float column_sum(const float* __restrict__ rows, uint32_t n_rows, size_t stride, uint32_t j, bool live) {
+  constexpr uint32_t W = kFinThreads / 32;
+  __shared__ float colred[W][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float part = 0.f;
+  if (live) {
+    uint32_t p = warp;
+    for (; p + 3 * W < n_rows; p += 4 * W) {
+      float v0 = rows[p * stride + j];
+      float v1 = rows[(p + W) * stride + j];
+      float v2 = rows[(p + 2 * W) * stride + j];
+      float v3 = rows[(p + 3 * W) * stride + j];
+      part += v0; part += v1; part += v2; part += v3;
+    }
+    for (; p < n_rows; p += W) part += rows[p * stride + j];
+  }
+  colred[warp][lane] = part;
+  __syncthreads();
+  float sum = 0.f;
+  if (warp == 0)
+#pragma unroll
+    for (int w = 0; w < (int)W; ++w) sum += colred[w][lane];
+  return sum;
+}
+
+// The release scale of this step from the all-reduced (n, loss), and the loss / n / f statistics (thread 0 of CTA 0).
+struct Release { float Bf, f, sigma; };
+D3P_D Release release_scale(const FinalizeArgs& a, float n_all, float loss_all) {
+  const float n = a.use_override ? a.n_override : n_all;
+  const float Bf = (float)a.B;
+  const float f = a.use_override ? a.f_override : ((n == 0.f) ? 0.f : __fdiv_rn(Bf, n));   // svi.py:305
+  const float sigma = __fmul_rn(a.dp_scale, __fdiv_rn(a.C, n));        // svi.py:365-366 (inf when n == 0)
+  if (blockIdx.x == 0 && threadIdx.x == 0 && a.stats) {
+    a.stats[0] = __fmul_rn(__fdiv_rn(loss_all, Bf), f);                // svi.py:306,342
+    a.stats[1] = n;
+    a.stats[2] = f;
+  }
+  return {Bf, f, sigma};
+}
+
+// One released element: sum = its column sum over all ranks, xi = its Gaussian draw when `noisy`.
+D3P_D float release_element(const FinalizeArgs& a, const Release& r, uint32_t j, float sum, bool noisy, float xi) {
+  float g = __fdiv_rn(sum, r.Bf);                                      // mean over the padded batch size
+  if (noisy) g = __fadd_rn(g, __fmul_rn(xi, r.sigma));                // svi.py:485-486
+  g = __fmul_rn(__fmul_rn(g, a.obs_scale), r.f);                       // svi.py:374-375
+  if (a.grad_out) a.grad_out[j] = g;
+  return g;
+}
+
+// The optimizer update of element j from its released gradient g and old state x, m, v; ADADP adds its squared error
+// term to err2.
+D3P_D void update_element(const FinalizeArgs& a, float bc1, float bc2, float lr, uint32_t j, float g, float x, float m,
+                          float v, float& err2, bool quad_adam) {
+  optim_element(a, bc1, bc2, j, g, x, m, v, a.params, a.m, a.v, quad_adam);
+  if (a.opt_kind == D3P_OPT_ADADP) err2 += adadp_element(a, lr, j, x, g);
+}
+
+// A CTA's sum of the ADADP error terms (odd steps), for adadp_finish_kernel.
+D3P_D void store_err_partial(const FinalizeArgs& a, float e) {
+  a.err_ws[1 + blockIdx.x] = e;
+  if (blockIdx.x == 0) a.err_ws[0] = (float)gridDim.x;
+}
 
 // site states live in constant-bank kernel parameters next to the leaf table
 struct SiteStates { uint32_t w[D3P_MAX_LEAVES][16]; };
@@ -120,7 +239,6 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const __grid_cons
                                                                const __grid_constant__ CommDev comm) {
   __shared__ float red[2][kFinThreads / 32];
   __shared__ float s_n, s_loss;
-  const uint32_t stride = a.P + 2;
   // Launched as a programmatic dependent of the step kernel, this CTA is resident while that kernel is still running.
   // Everything that does not depend on its partial rows happens NOW, under the producer's tail instead of behind it:
   // the column's Gaussian draw (a ChaCha block: keys only), the Adam bias corrections and the loads of the parameter
@@ -152,94 +270,35 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const __grid_cons
       if (opt_uses_x(a.opt_kind)) x_pre = a.params[jp];
       if (opt_uses_m(a.opt_kind)) m_pre = a.m[jp];
       if (opt_uses_v(a.opt_kind)) v_pre = a.v[jp];
-      if (a.opt_kind == D3P_OPT_ADAM || a.opt_kind == D3P_OPT_CLIPPED_ADAM) {
-        const float t = (float)(a.step + 1);
-        bc1 = 1.0f - powf(a.b1, t); bc2 = 1.0f - powf(a.b2, t);
-      }
+      adam_bias(a, bc1, bc2);
     }
   }
   asm volatile("griddepcontrol.wait;" ::: "memory");    // no-op unless launched as a programmatic dependent
   // every CTA reduces the (count, loss) columns itself: n_partials is a few hundred at most
-  float cnt = 0.f, loss = 0.f;
-  for (uint32_t p = threadIdx.x; p < a.n_partials; p += kFinThreads) {
-    loss += a.partials[(size_t)p * stride + a.P];
-    cnt += a.partials[(size_t)p * stride + a.P + 1];
-  }
-  cnt = group_sum<32>(cnt);
-  loss = group_sum<32>(loss);
-  if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = cnt; red[1][threadIdx.x >> 5] = loss; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float c = 0.f, l = 0.f;
-#pragma unroll
-    for (int w = 0; w < kFinThreads / 32; ++w) { c += red[0][w]; l += red[1][w]; }
-    s_n = c; s_loss = l;
-  }
-  // 32 columns per CTA; warp w adds partials w, w+4, ... and warp 0 combines them in fixed order
-  __shared__ float colred[kFinThreads / 32][32];
+  reduce_count_loss<kFinThreads>(a, red, s_n, s_loss);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t j = blockIdx.x * 32 + lane;
-  float part = 0.f;
-  if (j < a.P) {
-    uint32_t p = warp;
-    for (; p + 3 * (kFinThreads / 32) < a.n_partials; p += 4 * (kFinThreads / 32)) {
-      float v0 = a.partials[(size_t)p * stride + j];
-      float v1 = a.partials[(size_t)(p + (kFinThreads / 32)) * stride + j];
-      float v2 = a.partials[(size_t)(p + 2 * (kFinThreads / 32)) * stride + j];
-      float v3 = a.partials[(size_t)(p + 3 * (kFinThreads / 32)) * stride + j];
-      part += v0; part += v1; part += v2; part += v3;
-    }
-    for (; p < a.n_partials; p += kFinThreads / 32) part += a.partials[(size_t)p * stride + j];
-  }
-  colred[warp][lane] = part;
-  __syncthreads();
-  if (warp != 0) return;
   const bool live = j < a.P;
-  float sum = 0.f;
-#pragma unroll
-  for (int w = 0; w < kFinThreads / 32; ++w) sum += colred[w][lane];
+  float sum = column_sum(a.partials, a.n_partials, a.P + 2, j, live);   // its barrier also publishes s_n / s_loss
+  if (warp != 0) return;
   float n_all = s_n, loss_all = s_loss;
   if (comm.world > 1) {
-    // one-shot all-reduce over NVLink peer memory (comm.cuh): push tagged words to every peer, poll my own
-    // window for theirs, add the G copies in rank order (identical on every rank)
-    const float mine = sum, my_n = s_n, my_loss = s_loss;
-    const size_t jn = comm.extra_off + 2 * (size_t)blockIdx.x;
+    const float mine = sum;
     if (live) ll_push(comm, j, mine);
-    if (lane == 0) { ll_push(comm, jn, my_n); ll_push(comm, jn + 1, my_loss); }
-    // an earlier time-out on this rank (sampler counts, a previous exchange) poisons everything from here on
-    sum = comm_poisoned(comm) ? __uint_as_float(0x7fc00000u) : 0.f;
-    n_all = 0.f; loss_all = sum;
-    for (int r = 0; r < comm.world; ++r) {
-      const bool me = r == comm.rank;
-      if (live) sum += me ? mine : ll_wait(comm, r, j);
-      n_all += me ? my_n : ll_wait(comm, r, jn);
-      loss_all += me ? my_loss : ll_wait(comm, r, jn + 1);
-    }
+    sum = exchange_n_loss(comm, n_all, loss_all);
+    for (int r = 0; r < comm.world; ++r)
+      if (live) sum += r == comm.rank ? mine : ll_wait(comm, r, j);
   }
-  const float n = a.use_override ? a.n_override : n_all;
-  const float Bf = (float)a.B;
-  const float f = a.use_override ? a.f_override : ((n == 0.f) ? 0.f : __fdiv_rn(Bf, n));   // svi.py:305
-  const float sigma = __fmul_rn(a.dp_scale, __fdiv_rn(a.C, n));        // svi.py:365-366 (inf when n == 0)
-  if (blockIdx.x == 0 && lane == 0 && a.stats) {
-    a.stats[0] = __fmul_rn(__fdiv_rn(loss_all, Bf), f);                // svi.py:306,342
-    a.stats[1] = n;
-    a.stats[2] = f;
-  }
+  const Release rel = release_scale(a, n_all, loss_all);
   float err2 = 0.f;
   if (live) {
-    float g = __fdiv_rn(sum, Bf);                                      // mean over the padded batch size
-    if (have_xi) g = __fadd_rn(g, __fmul_rn(xi_pre, sigma));          // svi.py:485-486 (drawn in the prologue)
-    g = __fmul_rn(__fmul_rn(g, a.obs_scale), f);                       // svi.py:374-375
-    if (a.grad_out) a.grad_out[j] = g;
-    optim_element(a, bc1, bc2, j, g, x_pre, m_pre, v_pre, a.params, a.m, a.v);
-    if (a.opt_kind == D3P_OPT_ADADP) err2 = adadp_element(a, *a.lr, j, a.params[j], g);
+    const bool adadp = a.opt_kind == D3P_OPT_ADADP;     // ADADP reads its parameter here, after griddepcontrol.wait
+    update_element(a, bc1, bc2, adadp ? *a.lr : 0.f, j, release_element(a, rel, j, sum, have_xi, xi_pre),
+                   adadp ? a.params[j] : x_pre, m_pre, v_pre, err2, false);
   }
   if (a.opt_kind == D3P_OPT_ADADP && (a.step & 1)) {
     err2 = group_sum<32>(err2);
-    if (lane == 0) {
-      a.err_ws[1 + blockIdx.x] = err2;
-      if (blockIdx.x == 0) a.err_ws[0] = (float)gridDim.x;
-    }
+    if (lane == 0) store_err_partial(a, err2);
   }
 }
 
@@ -247,7 +306,7 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(const __grid_cons
 // (~1000 instructions) for each of its 16 elements: fine at P ~ 2 k, 90 us at P ~ 650 k.  Here FOUR lanes
 // cooperate on one block, each holding one column of the 4 x 4 state (column round = local quarter round,
 // diagonal round = rotate rows 1-3 across the 4 lanes with shuffles), and then finalize the 4 elements whose
-// keystream words they hold.  Same arithmetic as finalize_kernel; partial rows are summed in row order.
+// keystream words they hold with finalize_kernel's release_element; partial rows are summed in row order.
 struct ChunkTable { uint32_t n_chunks; uint32_t chunk_start[D3P_MAX_LEAVES + 1]; };   // chunk = one 16-element block
 
 D3P_D void quad_qr(uint32_t& a, uint32_t& b, uint32_t& c, uint32_t& d) { D3P_QR(a, b, c, d) }
@@ -264,21 +323,7 @@ __global__ void __launch_bounds__(256) finalize_quad_kernel(const __grid_constan
   __shared__ float s_n, s_loss;
   const uint32_t stride = a.P + 2;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  float cnt = 0.f, loss = 0.f;
-  for (uint32_t p = threadIdx.x; p < a.n_partials; p += 256) {
-    loss += a.partials[(size_t)p * stride + a.P];
-    cnt += a.partials[(size_t)p * stride + a.P + 1];
-  }
-  cnt = group_sum<32>(cnt);
-  loss = group_sum<32>(loss);
-  if (lane == 0) { red[0][warp] = cnt; red[1][warp] = loss; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float c = 0.f, l = 0.f;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) { c += red[0][w]; l += red[1][w]; }
-    s_n = c; s_loss = l;
-  }
+  reduce_count_loss<256>(a, red, s_n, s_loss);
   __syncthreads();
   const uint32_t t = blockIdx.x * 256 + threadIdx.x;
   const uint32_t chunk = t >> 2, q = t & 3;
@@ -348,58 +393,27 @@ __global__ void __launch_bounds__(256) finalize_quad_kernel(const __grid_constan
 #pragma unroll
     for (int i = 0; i < 4; ++i) sum[i] += pre[p][i];
   float n_all = s_n, loss_all = s_loss;
-  if (comm.world > 1) {                                    // one-shot all-reduce over peer memory (comm.cuh)
-    const float my_n = s_n, my_loss = s_loss;
-    const size_t jn = comm.extra_off + 2 * (size_t)blockIdx.x;
+  if (comm.world > 1) {
     float mine[4];
-    const float zero = comm_poisoned(comm) ? __uint_as_float(0x7fc00000u) : 0.f;   // see finalize_kernel
 #pragma unroll
-    for (int i = 0; i < 4; ++i) { mine[i] = sum[i]; if (ok[i]) ll_push(comm, jj[i], mine[i]); sum[i] = zero; }
-    if (threadIdx.x == 0) { ll_push(comm, jn, my_n); ll_push(comm, jn + 1, my_loss); }
-    n_all = 0.f; loss_all = zero;
-    for (int r = 0; r < comm.world; ++r) {
-      const bool me = r == comm.rank;
+    for (int i = 0; i < 4; ++i) { mine[i] = sum[i]; if (ok[i]) ll_push(comm, jj[i], mine[i]); }
+    const float zero = exchange_n_loss(comm, n_all, loss_all);
 #pragma unroll
-      for (int i = 0; i < 4; ++i) if (ok[i]) sum[i] += me ? mine[i] : ll_wait(comm, r, jj[i]);
-      n_all += me ? my_n : ll_wait(comm, r, jn);
-      loss_all += me ? my_loss : ll_wait(comm, r, jn + 1);
-    }
+    for (int i = 0; i < 4; ++i) sum[i] = zero;
+    for (int r = 0; r < comm.world; ++r)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) if (ok[i]) sum[i] += r == comm.rank ? mine[i] : ll_wait(comm, r, jj[i]);
   }
-  const float n = a.use_override ? a.n_override : n_all;
-  const float Bf = (float)a.B;
-  const float f = a.use_override ? a.f_override : ((n == 0.f) ? 0.f : __fdiv_rn(Bf, n));
-  const float sigma = __fmul_rn(a.dp_scale, __fdiv_rn(a.C, n));
-  if (blockIdx.x == 0 && threadIdx.x == 0 && a.stats) {
-    a.stats[0] = __fmul_rn(__fdiv_rn(loss_all, Bf), f);
-    a.stats[1] = n;
-    a.stats[2] = f;
-  }
-  const float t1 = (float)(a.step + 1);
-  const float bc1 = 1.0f - powf(a.b1, t1), bc2 = 1.0f - powf(a.b2, t1);
+  const Release rel = release_scale(a, n_all, loss_all);
+  float bc1 = 1.f, bc2 = 1.f;
+  adam_bias(a, bc1, bc2);
   float err2 = 0.f;
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    if (!ok[i]) continue;
-    const uint32_t j = jj[i];
-    float g = __fdiv_rn(sum[i], Bf);
-    g = __fadd_rn(g, __fmul_rn(bits_to_normal<false>(ks[i]), sigma));
-    g = __fmul_rn(__fmul_rn(g, a.obs_scale), f);
-    if (a.grad_out) a.grad_out[j] = g;
-    if (a.opt_kind == D3P_OPT_SGD) {
-      prm[j] = x[i] - a.step_size * g;
-    } else if (a.opt_kind == D3P_OPT_ADAM) {
-      float m = (1.0f - a.b1) * g + a.b1 * m0[i];
-      float v = (1.0f - a.b2) * (g * g) + a.b2 * v0[i];
-      float mhat = m / bc1;
-      float vhat = v / bc2;
-      prm[j] = x[i] - a.step_size * mhat / (sqrtf(vhat) + a.eps);
-      pm[j] = m;
-      pv[j] = v;
-    } else {                                                     // the other kinds (and ADADP)
-      optim_element(a, bc1, bc2, j, g, x[i], m0[i], v0[i], prm, pm, pv);
-      if (a.opt_kind == D3P_OPT_ADADP) err2 += adadp_element(a, lr_adadp, j, x[i], g);
-    }
-  }
+  for (int i = 0; i < 4; ++i)
+    if (ok[i])
+      update_element(a, bc1, bc2, lr_adadp, jj[i],
+                     release_element(a, rel, jj[i], sum[i], true, bits_to_normal<false>(ks[i])), x[i], m0[i], v0[i],
+                     err2, true);
   if (adadp_odd) {                                              // fixed-order CTA sum of the error terms
     err2 = group_sum<32>(err2);
     if (lane == 0) red[0][warp] = err2;
@@ -408,8 +422,7 @@ __global__ void __launch_bounds__(256) finalize_quad_kernel(const __grid_constan
       float e = 0.f;
 #pragma unroll
       for (int w = 0; w < 8; ++w) e += red[0][w];
-      a.err_ws[1 + blockIdx.x] = e;
-      if (blockIdx.x == 0) a.err_ws[0] = (float)gridDim.x;
+      store_err_partial(a, e);
     }
   }
 }
@@ -441,24 +454,13 @@ __global__ void __launch_bounds__(256) adadp_finish_kernel(const float* __restri
   for (uint32_t j = blockIdx.x * 256 + threadIdx.x; j < P; j += gridDim.x * 256) params[j] = x_prev[j];
 }
 
-// out[j] = sum_p partials[p][j] for j < row_len, fixed order (warp w adds rows w, w+4, ...).
+// out[j] = sum_p partials[p][j] for j < row_len, in finalize_kernel's order.
 __global__ void __launch_bounds__(kFinThreads) reduce_partials_kernel(const float* __restrict__ partials,
                                                                       uint32_t n_partials, uint32_t row_len,
                                                                       float* __restrict__ out) {
-  __shared__ float colred[kFinThreads / 32][32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t j = blockIdx.x * 32 + lane;
-  float part = 0.f;
-  if (j < row_len)
-    for (uint32_t p = warp; p < n_partials; p += kFinThreads / 32) part += partials[(size_t)p * row_len + j];
-  colred[warp][lane] = part;
-  __syncthreads();
-  if (warp == 0 && j < row_len) {
-    float sum = 0.f;
-#pragma unroll
-    for (int w = 0; w < kFinThreads / 32; ++w) sum += colred[w][lane];
-    out[j] = sum;
-  }
+  const uint32_t j = blockIdx.x * 32 + (threadIdx.x & 31);
+  const float sum = column_sum(partials, n_partials, row_len, j, j < row_len);
+  if ((threadIdx.x >> 5) == 0 && j < row_len) out[j] = sum;
 }
 
 }  // namespace d3p
@@ -592,25 +594,22 @@ int32_t d3p::perturb_finalize_impl(const float* partials_d, uint32_t n_partials,
     }
     if (covered != P) return D3P_ERR_INVALID_ARGUMENT;
   }
-  // large parameter vectors with a leaf table that tiles [0, P): one thread per keystream block
-  if (add_noise && leaves_h && P >= 32768 && n_partials <= 64) {
+  // large parameter vectors (with noise, so the leaf table tiles [0, P) as checked above): four threads per keystream
+  // block
+  if (add_noise && P >= 32768 && n_partials <= 64) {
     ChunkTable ct;
     memset(&ct, 0, sizeof(ct));
-    uint64_t covered = 0;
     uint32_t nc = 0;
     for (uint32_t l = 0; l < lt.n_leaves; ++l) {
       ct.chunk_start[l] = nc;
       nc += (lt.len[l] + 15) / 16;
-      covered += lt.len[l];
     }
     ct.chunk_start[lt.n_leaves] = nc;
     ct.n_chunks = nc;
-    if (covered == P && nc > 0) {
-      const unsigned qgrid = (nc * 4 + 255) / 256;
-      if (comm) { const int32_t rc = comm_next(comm, P, qgrid, &cd); if (rc != D3P_OK) return rc; }
-      finalize_quad_kernel<<<qgrid, 256, 0, (cudaStream_t)stream>>>(a, lt, ss, site_states_d, ct, cd);
-      return check_launch();
-    }
+    const unsigned qgrid = (nc * 4 + 255) / 256;
+    if (comm) { const int32_t rc = comm_next(comm, P, qgrid, &cd); if (rc != D3P_OK) return rc; }
+    finalize_quad_kernel<<<qgrid, 256, 0, (cudaStream_t)stream>>>(a, lt, ss, site_states_d, ct, cd);
+    return check_launch();
   }
   unsigned grid = P ? (P + 31) / 32 : 1;
   if (comm) { const int32_t rc = comm_next(comm, P, grid, &cd); if (rc != D3P_OK) return rc; }
