@@ -14,7 +14,8 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "_lib")
 LIBNAME = "libd3p_b200.so"
 SOURCES = ["rng.cu", "samplers.cu", "clip.cu", "finalize.cu", "meanfield_step.cu", "meanfield_step_vec.cu",
-           "tc_gemm.cu", "vae.cu", "gmm_step.cu", "evaluate.cu", "epoch.cu", "comm.cu", "jrandom.cu", "gmm_dist.cu"]
+           "tc_gemm.cu", "vae.cu", "gmm_step.cu", "evaluate.cu", "epoch.cu", "comm.cu", "jrandom.cu", "gmm_dist.cu",
+           "autodiag.cu"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -41,6 +41,11 @@ class GmmDesc(C.Structure):
                 ("mus_off", C.c_uint32), ("num_obs_total", C.c_float)]
 
 
+class AutodiagDesc(C.Structure):
+    _fields_ = [("latent_dim", C.c_uint32), ("n_params", C.c_uint32), ("loc_off", C.c_uint32),
+                ("scale_off", C.c_uint32), ("num_obs_total", C.c_float)]
+
+
 class LeafTable(C.Structure):
     _fields_ = [("n_leaves", C.c_uint32), ("leaf_off", C.c_uint32 * MAX_LEAVES),
                 ("leaf_len", C.c_uint32 * MAX_LEAVES), ("site_state", (C.c_uint32 * 16) * MAX_LEAVES)]
@@ -99,6 +104,12 @@ _SIGNATURES = {
     "d3p_dpsvi_step_meanfield": (C.c_int32, [C.POINTER(MeanfieldDesc), _vp, _vp, C.c_size_t, _vp, _vp, _vp, _vp,
                                              C.c_uint32, C.c_uint32, C.c_uint32, _u32p, C.c_float, C.c_float,
                                              _vp, _vp, _vp, _vp, C.c_size_t, _vp]),  # norms, grads, loss, ws
+    "d3p_autodiag_draw_f32": (C.c_int32, [C.POINTER(AutodiagDesc), _vp, _u32p, C.c_uint32, C.c_uint32, C.c_uint32,
+                                          _vp, _vp, C.c_size_t, _vp]),
+    "d3p_autodiag_workspace_bytes": (C.c_size_t, [C.POINTER(AutodiagDesc), C.c_uint32, _u32p]),
+    "d3p_dpsvi_step_autodiag": (C.c_int32, [C.POINTER(AutodiagDesc), _vp, _vp, _vp, C.c_size_t, _vp, _vp, _vp,
+                                            C.c_uint32, C.c_uint32, C.c_uint32, C.c_float, C.c_float,
+                                            _vp, _vp, _vp, _vp, C.c_size_t, _vp]),  # norms, grads, loss, ws
     "d3p_perturb_finalize_f32": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(LeafTable),
                                              C.c_float, C.c_float, C.c_float, C.c_int32, _vp,
                                              C.POINTER(OptimDesc), _vp, _vp, _vp, _vp,
@@ -162,6 +173,8 @@ _SIGNATURES = {
     "d3p_dpsvi_step_meanfield_dk": (C.c_int32, [C.POINTER(MeanfieldDesc), _vp, _vp, C.c_size_t, _vp, _vp, _vp, _vp,
                                                 C.c_uint32, C.c_uint32, C.c_uint32, _vp, C.c_float, C.c_float,
                                                 _vp, _vp, _vp, _vp, C.c_size_t, _vp]),
+    "d3p_autodiag_draw_f32_dk": (C.c_int32, [C.POINTER(AutodiagDesc), _vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32,
+                                             _vp, _vp, C.c_size_t, _vp]),
     "d3p_dpsvi_step_vae_dk": (C.c_int32, [C.POINTER(VaeDesc), _vp, _vp, C.c_size_t, _vp, _vp, _vp, C.c_uint32, C.c_uint32,
                                           C.c_uint32, _vp, C.c_float, C.c_float, _vp, _vp, _vp, C.c_size_t,
                                           C.POINTER(C.c_void_p), _vp, _vp]),

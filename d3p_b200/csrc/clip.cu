@@ -4,25 +4,11 @@
 // caller already holds (the path the reference's own tests drive, tests/test_dpsvi.py:146-191).
 #include "common.cuh"
 #include "launch.cuh"
+#include "reduce.cuh"
 
 namespace d3p {
 
 constexpr int kClipThreads = 256;
-
-D3P_D float block_sum(float v, float* smem /* >= 32 floats */) {
-  v = group_sum<32>(v);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  __syncthreads();
-  if (lane == 0) smem[warp] = v;
-  __syncthreads();
-  float t = (threadIdx.x < (blockDim.x >> 5)) ? smem[threadIdx.x] : 0.f;
-  if (warp == 0) {
-    t = group_sum<32>(t);
-    if (lane == 0) smem[0] = t;
-  }
-  __syncthreads();
-  return smem[0];
-}
 
 D3P_D float row_sq_norm(const float* __restrict__ row, uint32_t P, float* smem) {
   float acc = 0.f;
@@ -39,9 +25,6 @@ D3P_D float row_sq_norm(const float* __restrict__ row, uint32_t P, float* smem) 
   }
   return block_sum(acc, smem);
 }
-
-// clip factor exactly as clip_gradient: 1 / max(1, norm / C)
-D3P_D float clip_factor(float norm, float C) { return 1.0f / fmaxf(1.0f, norm / C); }
 
 __global__ void __launch_bounds__(kClipThreads) clip_rows_kernel(float* __restrict__ g, uint32_t B, uint32_t P, float C,
                                                                  float* __restrict__ norms) {

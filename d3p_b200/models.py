@@ -11,14 +11,20 @@ model/guide pair:
 
 Parameters are the *unconstrained* variational parameters, stored as one flat float32 vector
 whose leaf order is the jax pytree order of the reference's param dict (sorted site names).
-Arbitrary models go through the materialised-gradient stage methods of ``DPSVI``.
+A user model with real-valued latents trains under an AutoDiagonalNormal guide through
+``AutoDiagonalNormalModel``; any other model goes through the materialised-gradient stage methods
+of ``DPSVI``.
 """
 import ctypes as C
+import inspect
+import math
 
 import numpy as np
 import torch
 
 from . import _native as _n
+from .minibatch import BatchView, LocalRows
+from .util import example_count
 
 
 class Trace_ELBO:
@@ -49,6 +55,7 @@ class Family:
     # DPSVI.run_epoch has a C driver with device keys / for a batch sharded over NVLink peers (else: step by step)
     epoch_device_keys = True
     epoch_sharded = True
+    epoch_driver = True             # False: the family has no C epoch driver at all (DPSVI.run_epoch steps)
 
     def layout(self):
         """[(name, offset, shape)] in pytree (sorted-name) order."""
@@ -424,3 +431,201 @@ class GaussianMixture(Family):
     def _epoch(self, device_keys, desc, sampler, x, stride, y, batch_key, rng_key, rest):
         _n.check(_n.lib().d3p_dpsvi_run_epoch_gmm(C.byref(desc), C.byref(sampler), x, stride, batch_key, rng_key, *rest),
                  "run_epoch_gmm")
+
+
+_LOG_SQRT_2PI = math.log(math.sqrt(2 * math.pi))
+
+
+def std_normal_log_prior(latents):
+    """The default prior of ``AutoDiagonalNormalModel``: N(0, 1) on every latent element, with its normaliser."""
+    out = 0.
+    for v in latents.values():
+        out = out + (-0.5 * v * v - _LOG_SQRT_2PI).reshape(v.shape[0], -1).sum(1)
+    return out
+
+
+class AutoDiagonalNormalModel(Family):
+    """A user model under numpyro's ``AutoDiagonalNormal`` guide (d3p's README and ``tests/test_dpsvi.py:65-70``):
+
+        fam = AutoDiagonalNormalModel([("w", (d,)), ("b", ())], log_likelihood)
+        svi = DPSVI(fam.model, fam.guide, Adam(1e-3), Trace_ELBO(), clipping_threshold=1., dp_scale=1.,
+                    num_obs_total=N)
+
+    ``sites`` is ``[(name, shape), ...]`` in model order; their ravelled concatenation is the guide's single
+    ``_auto_latent`` site of D elements, and the parameters are ``auto_loc[D]`` and ``auto_scale[D]`` (softplus link).
+
+    ``log_likelihood(latents, *batch) -> [B]`` is ``log p(x_i | theta_i)`` of every example and
+    ``log_prior(latents) -> [B]`` is ``log p(theta_i)`` (default: N(0, 1) on every element, normaliser included);
+    ``latents`` maps each site name to a ``[B, *shape]`` tensor and ``batch`` holds the rows of the batch arrays
+    passed to ``update``.  Both are torch functions: a step evaluates the potential
+    ``U_i = -log_prior - num_obs_total * log_likelihood`` for all examples at once and takes ``h_i = dU_i / dtheta_i``
+    with ONE ``torch.autograd.grad`` of ``U.sum()``.  That is exact only if the model is separable: example i's
+    outputs may depend on row i of ``latents`` and of ``batch`` alone (no batch statistics, no cross-row reductions).
+
+    Latents have real support.  For a constrained latent, such as a noise scale ``sigma = exp(tau)``, declare the
+    unconstrained ``tau`` and write its density with the Jacobian, ``log p_sigma(exp(tau)) + tau``, which is what
+    numpyro's ``biject_to`` does for a constrained site.
+
+    The guide draws, the per-example norms, the clipping and the clipped sums run in the library's CUDA kernels
+    (``d3p_autodiag_draw_f32``, ``d3p_dpsvi_step_autodiag``), with the key plumbing and arithmetic of the fused
+    ``guide="auto"`` families: a model that restates ``LogisticRegression`` reproduces ``LogisticRegression(d,
+    guide="auto")``.  ``run_epoch`` steps through ``update`` (the likelihood is a Python callable); ``LocalRows``
+    batches are not supported.
+    """
+    epoch_driver = False
+
+    def __init__(self, sites, log_likelihood, log_prior=None, init_scale=0.1):
+        self.sites = [(str(name), tuple(int(n) for n in shape)) for name, shape in sites]
+        if not self.sites:
+            raise ValueError("AutoDiagonalNormalModel needs at least one latent site")
+        if len({name for name, _ in self.sites}) != len(self.sites):
+            raise ValueError("latent site names must be unique")
+        self.latent_dim = sum(math.prod(shape) for _, shape in self.sites)
+        if self.latent_dim == 0:
+            raise ValueError("the latent sites have no elements")
+        if not callable(log_likelihood) or (log_prior is not None and not callable(log_prior)):
+            raise TypeError("log_likelihood and log_prior must be callables")
+        self.log_likelihood = log_likelihood
+        self.log_prior = std_normal_log_prior if log_prior is None else log_prior
+        self.init_scale = float(init_scale)
+        self.model, self.guide = _Handle(self, "model"), _Handle(self, "guide")
+        self._bufs = {}
+
+    def param_shapes(self):
+        return {"auto_loc": (self.latent_dim,), "auto_scale": (self.latent_dim,)}
+
+    def init_params(self):
+        """loc 0, scale ``init_scale`` (numpyro draws auto_loc with init_to_uniform: pass ``params=`` to
+        ``DPSVI.init`` to start from specific values)."""
+        D = self.latent_dim
+        return {"auto_loc": np.zeros(D, np.float32), "auto_scale": np.full(D, softplus_inv(self.init_scale), np.float32)}
+
+    def constrain(self, name, value):
+        if name == "auto_scale":
+            return torch.nn.functional.softplus(value)
+        return value
+
+    def desc(self, num_obs_total):
+        o = self.offsets()
+        return _n.AutodiagDesc(self.latent_dim, self.n_params, o["auto_loc"], o["auto_scale"], float(num_obs_total))
+
+    def check_args(self, args):
+        if len(args) == 0:
+            raise ValueError("AutoDiagonalNormalModel expects the batch arrays of log_likelihood")
+        if any(isinstance(a, LocalRows) for a in args):
+            raise ValueError("AutoDiagonalNormalModel takes whole batches: LocalRows is not supported")
+        counts = {example_count(a) for a in args}
+        if len(counts) != 1 or any(len(getattr(a, "shape", np.shape(a))) == 0 for a in args):
+            raise ValueError("every batch array must have the same leading (example) axis")
+        try:
+            sig = inspect.signature(self.log_likelihood)
+        except (TypeError, ValueError):         # a callable without a signature: checked when called
+            return
+        try:
+            sig.bind({}, *args)
+        except TypeError as e:
+            raise ValueError(f"log_likelihood(latents, *batch) does not take the {len(args)} batch arrays: {e}") from None
+
+    def latents(self, theta):
+        """[n, D] -> {site: [n, *shape]} views of the ravelled ``_auto_latent`` rows."""
+        n, out, o = theta.shape[0], {}, 0
+        for name, shape in self.sites:
+            k = math.prod(shape)
+            out[name] = theta[:, o:o + k].reshape((n,) + shape)
+            o += k
+        return out
+
+    def potential_and_grad(self, theta, rows, num_obs_total):
+        """``U = -log_prior - N * log_likelihood`` of the [n, D] draws ``theta`` on the batch rows ``rows`` and
+        ``h = dU_i / dtheta_i`` -> (U [n], h [n, D]), both float32 and contiguous."""
+        n = theta.shape[0]
+        th = theta.detach().requires_grad_(True)
+        with torch.enable_grad():
+            lat = self.latents(th)
+            lp, ll = self.log_prior(lat), self.log_likelihood(lat, *rows)
+            for what, v in (("log_prior", lp), ("log_likelihood", ll)):
+                if not isinstance(v, torch.Tensor) or tuple(v.shape) != (n,):
+                    raise ValueError(f"{what} returned shape {tuple(getattr(v, 'shape', ()))}, expected ({n},): "
+                                     "it must return one value per example")
+            U = -lp - float(num_obs_total) * ll
+            (h,) = torch.autograd.grad(U.sum(), th, materialize_grads=True)
+        return U.detach().float().contiguous(), h.float().contiguous()
+
+    @staticmethod
+    def _rows(args, pos_begin, pos_end):
+        """Rows [pos_begin, pos_end) of the batch arrays on the device (a BatchView through its gather, with the
+        padding rows of a Poisson batch zero-filled)."""
+        dev = torch.device("cuda", torch.cuda.current_device())
+        out = []
+        for a in args:
+            if isinstance(a, BatchView):
+                t = a.tensor()
+            else:
+                t = a if isinstance(a, torch.Tensor) else torch.as_tensor(np.asarray(a))
+                t = t.to(dev)
+            if t.is_floating_point() and t.dtype != torch.float32:
+                t = t.float()
+            out.append(t[pos_begin:pos_end])
+        return out
+
+    def _draw(self, desc, params, tf_key, B, pos_begin, pos_end):
+        """Guide draws into this object's cached buffers -> (theta, eps), [n, D] each (n = 1 when B == 0)."""
+        n, D = (pos_end - pos_begin) if B else 1, self.latent_dim
+        dev = torch.cuda.current_device()
+        buf = self._bufs.get(dev)
+        if buf is None or buf.shape[1] < n:
+            buf = self._bufs[dev] = torch.empty((2, max(n, 1), D), dtype=torch.float32, device=torch.device("cuda", dev))
+        theta, eps = buf[0, :n], buf[1, :n]
+        if n:
+            _n.check(_n.lib().d3p_autodiag_draw_f32(C.byref(desc), params, tf_key, B, pos_begin, pos_end,
+                                                    _n.ptr(theta), _n.ptr(eps), D, _n.stream_ptr()), "autodiag_draw")
+        return theta, eps
+
+    def run_step(self, svi, state, tf_key, args, mask, pos_begin, pos_end, px_norms, px_grads, px_loss):
+        self.check_args(args)
+        if isinstance(mask, LocalRows):
+            raise ValueError("AutoDiagonalNormalModel takes whole batches: LocalRows is not supported")
+        B = example_count(args[0])
+        desc = self.desc(svi._num_obs_total())
+        params = _n.ptr(state.optim_state.flat)
+        mask_t, _ = svi._mask_arg(mask, B)
+        num_valid = args[0].num_valid if isinstance(args[0], BatchView) else None
+        rows = pos_end - pos_begin
+        key = tf_key.ctypes.data_as(C.POINTER(C.c_uint32))
+        U = h = eps = None
+        if rows:
+            theta, eps = self._draw(desc, params, key, B, pos_begin, pos_end)
+            U, h = self.potential_and_grad(theta, self._rows(args, pos_begin, pos_end), desc.num_obs_total)
+        n_part = C.c_uint32(0)
+        lib = _n.lib()
+        need = lib.d3p_autodiag_workspace_bytes(C.byref(desc), rows, C.byref(n_part))
+        ws = svi._workspace(need)
+        if svi.event_hook is not None:
+            svi.event_hook("step_begin")
+        _n.check(lib.d3p_dpsvi_step_autodiag(
+            C.byref(desc), params, _n.ptr(eps), _n.ptr(h), self.latent_dim, _n.ptr(U), _n.ptr(mask_t),
+            _n.ptr(num_valid), B, pos_begin, pos_end, float(state.observation_scale), float(svi._clipping_threshold),
+            _n.ptr(px_norms), _n.ptr(px_grads), _n.ptr(px_loss), _n.ptr(ws), need, _n.stream_ptr()),
+            "dpsvi_step_autodiag")
+        if svi.event_hook is not None:
+            svi.event_hook("step_end")
+        return ws, n_part.value, B, desc.n_params
+
+    def _evaluate(self, svi, desc, flat, args, key, loss):
+        """``-(log p(theta) + (N / B) sum_i log p(x_i | theta) - log q(theta))`` with ONE draw for the whole batch
+        (the ``B == 0`` draw from ``key``).  Unlike the fused families this takes the parameter tensor ``flat`` and
+        the batch arrays ``args`` themselves: the likelihood is evaluated in torch."""
+        self.check_args(args)
+        B, D = example_count(args[0]), self.latent_dim
+        theta, eps = self._draw(desc, _n.ptr(flat), key, 0, 0, 0)
+        rows = self._rows(args, 0, B)
+        with torch.no_grad():
+            lat1 = self.latents(theta)
+            ll = self.log_likelihood({k: v.expand((B,) + tuple(v.shape[1:])) for k, v in lat1.items()}, *rows)
+            if not isinstance(ll, torch.Tensor) or tuple(ll.shape) != (B,):
+                raise ValueError(f"log_likelihood returned shape {tuple(getattr(ll, 'shape', ()))}, expected ({B},): "
+                                 "it must return one value per example")
+            s = torch.nn.functional.softplus(flat[desc.scale_off:desc.scale_off + D])
+            log_q = (-0.5 * eps[0] * eps[0] - torch.log(s) - _LOG_SQRT_2PI).sum()
+            val = -(self.log_prior(lat1).reshape(-1)[0] + (desc.num_obs_total / B) * ll.sum() - log_q)
+        loss.copy_(val.reshape(1).float())

@@ -435,7 +435,8 @@ class DPSVI:
         For the model families fed by ``poisson_batchify_data`` / ``subsample_batchify_data`` /
         ``split_batchify_data`` the whole loop runs inside the family's ``d3p_dpsvi_run_epoch_*`` driver (no
         interpreter between launches); the result is bit-identical to the step-by-step calls, which remain the path for
-        everything else (NCCL-backend sharded runs, custom batchifiers, the key modes or sharded runs a family has
+        everything else (NCCL-backend sharded runs, custom batchifiers, a family without a driver
+        (``Family.epoch_driver``: ``AutoDiagonalNormalModel``), the key modes or sharded runs a family has
         no driver for: ``Family.epoch_device_keys`` / ``Family.epoch_sharded``, and an optimizer whose step size is a
         Python callable other than the named schedules of ``d3p_b200.optimizers``, which the C driver cannot call).
         Either way a schedule is evaluated at the optimizer's own step counter, not at ``first_step``.
@@ -447,7 +448,7 @@ class DPSVI:
         fam = self.family
         spec = getattr(get_batch, "spec", None)
         is_split = spec is not None and spec["kind"] == _n.SAMPLER_SPLIT
-        fused = (spec is not None and fam is not None and (fam.epoch_device_keys or not device_keys)
+        fused = (spec is not None and fam is not None and fam.epoch_driver and (fam.epoch_device_keys or not device_keys)
                  and (self.shard is None or (fam.epoch_sharded and self.shard[2] is None))
                  and self._rng_suite is strong_rng and spec["rng_suite"] is strong_rng and self.event_hook is None
                  and getattr(self.optim, "fused_epoch", True) and num_steps > 0)

@@ -181,6 +181,50 @@ int32_t d3p_dpsvi_step_meanfield(const d3p_meanfield_desc* desc, const float* pa
                                  void* ws_d, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * AutoDiagonalNormal guide over a user model (d3p_b200.models.AutoDiagonalNormalModel): one
+ * `_auto_latent` site of D real-valued elements, parameters auto_loc[D] and auto_scale[D]
+ * (softplus link).  Everything but the model's log density runs here: the caller draws
+ * theta_i = loc + softplus(rho) * eps_i with d3p_autodiag_draw_f32, evaluates the potential
+ *     U_i = -log p(theta_i) - N log p(x_i | theta_i)
+ * and its gradient h_i = dU_i / dtheta_i itself (autodiff of the model), and d3p_dpsvi_step_autodiag
+ * forms (with S = obs_scale, s = softplus(rho), a = sigmoid(rho))
+ *     gl_i = h_i / S ,   gs_i = gl_i * eps_i * a - (1/S) a / s
+ *     S * loss_i = U_i - |eps_i|^2 / 2 - sum_e log s_e - D log sqrt(2 pi)
+ * and clips and sums them as d3p_dpsvi_step_meanfield does.  Row r of theta_d / eps_d / grad_d /
+ * potential_d belongs to batch position pos_begin + r; rows are `ld` floats apart.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct {
+  uint32_t latent_dim;  /* D: elements of the `_auto_latent` site                         */
+  uint32_t n_params;    /* P: length of the flat parameter vector                          */
+  uint32_t loc_off;     /* offset of auto_loc[D] in the flat vector                        */
+  uint32_t scale_off;   /* offset of auto_scale[D] (unconstrained: scale = softplus)        */
+  float num_obs_total;  /* plate size N, the factor of the log-likelihood inside U          */
+} d3p_autodiag_desc;
+
+/* The guide draws of batch positions [pos_begin, pos_end): eps_d / theta_d row r receive the
+ * draw of key_p = jax.random.split(threefry_key, B)[pos_begin + r] through the seed-handler
+ * plumbing of the fused AutoDiagonalNormal families ((model_seed, guide_seed) = split(key_p),
+ * one site split; Threefry call j yields elements j and j + ceil(D/2)), with the step kernels'
+ * normal transform.  Every position of the range is drawn (no mask).  B == 0: ONE draw from
+ * threefry_key itself (no example split, pos_begin / pos_end ignored) with the exact transform of
+ * d3p_elbo_evaluate_meanfield — SVI.evaluate's draw. */
+int32_t d3p_autodiag_draw_f32(const d3p_autodiag_desc* desc, const float* params_d, const uint32_t threefry_key_h[2],
+                              uint32_t B, uint32_t pos_begin, uint32_t pos_end, float* theta_d, float* eps_d,
+                              size_t ld, void* stream);
+/* Workspace of a step over `rows` batch rows; its first n_partials * (P + 2) floats are the
+ * partial rows that d3p_perturb_finalize_* reduce. */
+size_t d3p_autodiag_workspace_bytes(const d3p_autodiag_desc* desc, uint32_t rows, uint32_t* n_partials_out);
+/* Partial rows { sum c_i gl_i | sum c_i gs_i | sum S loss_i | count } over the positions p of
+ * [pos_begin, pos_end) with (mask_d == NULL || mask_d[p]) and (num_valid_d == NULL || p < *num_valid_d),
+ * c_i = 1 / max(1, |(gl_i, gs_i)| / C); the other rows of eps_d / grad_d / potential_d are not
+ * read.  px_norms_d[B], px_grads_d[B, P], px_loss_d[B] (may be NULL) as in d3p_dpsvi_step_meanfield. */
+int32_t d3p_dpsvi_step_autodiag(const d3p_autodiag_desc* desc, const float* params_d, const float* eps_d,
+                                const float* grad_d, size_t ld, const float* potential_d, const uint8_t* mask_d,
+                                const int32_t* num_valid_d, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
+                                float obs_scale, float C, float* px_norms_d, float* px_grads_d, float* px_loss_d,
+                                void* ws_d, size_t ws_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Reduce + perturb + rescale (+ optimizer) — replaces d3p/svi.py:327-393,470-498.
  * ------------------------------------------------------------------------------------------ */
 #define D3P_OPT_NONE 0
@@ -557,6 +601,10 @@ int32_t d3p_chacha_normal_f32_dk(const uint32_t* state_d, uint64_t first_block, 
  * site_states_out_d[n_leaves][16] = split(k_noise, n_leaves). */
 int32_t d3p_dpsvi_keys_dk(uint32_t* rng_key_io_d, uint32_t n_leaves, uint32_t* threefry_key_out_d,
                           uint32_t* site_states_out_d, void* stream);
+/* d3p_autodiag_draw_f32 with the Threefry key (2 words) in device memory. */
+int32_t d3p_autodiag_draw_f32_dk(const d3p_autodiag_desc* desc, const float* params_d,
+                                 const uint32_t* threefry_key_d, uint32_t B, uint32_t pos_begin, uint32_t pos_end,
+                                 float* theta_d, float* eps_d, size_t ld, void* stream);
 /* Samplers.  rc_out_d / rc_d: 30 words (32 allocated is fine). */
 int32_t d3p_feistel_round_constants_dk(const uint32_t* state_d, uint32_t* rc_out_d, void* stream);
 int32_t d3p_feistel_sample_dk(const uint32_t* rc_d, uint32_t capacity, uint32_t first_pos, uint32_t n, int32_t* idx_d,
