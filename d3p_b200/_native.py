@@ -67,7 +67,7 @@ class SamplerDesc(C.Structure):
                 ("suppress", C.c_int32), ("perm_d", C.c_void_p)]
 
 
-SAMPLER_POISSON, SAMPLER_SUBSAMPLE, SAMPLER_SPLIT = 0, 1, 2
+SAMPLER_POISSON, SAMPLER_SUBSAMPLE, SAMPLER_SPLIT, SAMPLER_SUBSAMPLE_REPLACE = 0, 1, 2, 3
 
 _u32p = C.POINTER(C.c_uint32)
 _vp = C.c_void_p
@@ -90,6 +90,8 @@ _SIGNATURES = {
     "d3p_randint_finish_i32": (C.c_int32, [_vp, C.c_int32, _vp, C.c_size_t, _vp]),
     "d3p_chacha_randint_round": (C.c_int32, [_u32p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, _vp, C.c_size_t, _vp, _vp]),
     "d3p_randint_finish": (C.c_int32, [_vp, C.c_int32, C.c_uint32, _vp, C.c_size_t, _vp]),
+    "d3p_chacha_randint": (C.c_int32, [_u32p, C.c_uint32, C.c_int64, C.c_int64, _vp, C.c_size_t, _vp]),
+    "d3p_randint_bitmask": (C.c_uint32, [C.c_uint32, C.c_uint32]),
     "d3p_feistel_round_constants_h": (C.c_int32, [_u32p, _u32p]),
     "d3p_feistel_sample": (C.c_int32, [_u32p, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp]),
     "d3p_poisson_workspace_bytes": (C.c_size_t, [C.c_uint32]),
@@ -163,6 +165,7 @@ _SIGNATURES = {
     "d3p_chacha_random_bits_dk": (C.c_int32, [_vp, C.c_uint64, _vp, C.c_size_t, _vp]),
     "d3p_chacha_uniform_f32_dk": (C.c_int32, [_vp, C.c_uint64, C.c_float, C.c_float, _vp, C.c_size_t, _vp]),
     "d3p_chacha_normal_f32_dk": (C.c_int32, [_vp, C.c_uint64, _vp, C.c_size_t, _vp]),
+    "d3p_chacha_randint_dk": (C.c_int32, [_vp, C.c_uint32, C.c_int64, C.c_int64, _vp, C.c_size_t, _vp]),
     "d3p_dpsvi_keys_dk": (C.c_int32, [_vp, C.c_uint32, _vp, _vp, _vp]),
     "d3p_feistel_round_constants_dk": (C.c_int32, [_vp, _vp, _vp]),
     "d3p_feistel_sample_dk": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp]),

@@ -70,6 +70,7 @@ bool sampler_ok(const d3p_sampler_desc* s) {
   if (s->kind == D3P_SAMPLER_POISSON) return s->q >= 0.f && s->q <= 1.f;
   if (s->kind == D3P_SAMPLER_SUBSAMPLE) return s->batch <= s->n_records;
   if (s->kind == D3P_SAMPLER_SPLIT) return s->batch <= s->n_records && s->perm_d != nullptr;
+  if (s->kind == D3P_SAMPLER_SUBSAMPLE_REPLACE) return true;
   return false;
 }
 
@@ -240,6 +241,7 @@ int32_t run_epoch(const StepLauncher& fam, const d3p_sampler_desc* sampler, cons
   auto queue_sampler = [&](uint32_t s) -> int32_t {
     const int b = s & 1;
     const bool poisson = sampler->kind == D3P_SAMPLER_POISSON;
+    const bool feistel = sampler->kind == D3P_SAMPLER_SUBSAMPLE;
     uint32_t bkey[16], rcs[30];
     int32_t r = D3P_OK;
     if (!dk && (r = d3p_chacha_fold_in_h(batch_key_h, first_step + s, bkey)) != D3P_OK) return r;
@@ -247,8 +249,8 @@ int32_t run_epoch(const StepLauncher& fam, const d3p_sampler_desc* sampler, cons
     if (dk) {
       // the same keys made by one-block kernels, into the buffers of parity b (free once step s - 2 has consumed them)
       if ((r = d3p_chacha_fold_in_dk(batch_key_d, nullptr, first_step + s, w.bkey[b], samp_s)) != D3P_OK) return r;
-      if (!poisson && (r = d3p_feistel_round_constants_dk(w.bkey[b], w.rc[b], samp_s)) != D3P_OK) return r;
-    } else if (!poisson && (r = d3p_feistel_round_constants_h(bkey, rcs)) != D3P_OK) {
+      if (feistel && (r = d3p_feistel_round_constants_dk(w.bkey[b], w.rc[b], samp_s)) != D3P_OK) return r;
+    } else if (feistel && (r = d3p_feistel_round_constants_h(bkey, rcs)) != D3P_OK) {
       return r;
     }
     const uint32_t* key_h = dk ? nullptr : bkey;
@@ -262,8 +264,10 @@ int32_t run_epoch(const StepLauncher& fam, const d3p_sampler_desc* sampler, cons
       if (r == D3P_ERR_UNSUPPORTED)            // same decision on every rank (window size, tiles >= ranks)
         r = poisson_sample_impl(key_h, key_d, sampler->q, sampler->n_records, B, sampler->suppress, w.idx[b], w.counts[b],
                                 w.mask[b], w.poisson, w.poisson_bytes, samp_s);
-    } else {
+    } else if (feistel) {
       r = feistel_sample_impl(dk ? nullptr : rcs, dk ? w.rc[b] : nullptr, sampler->n_records, 0, B, w.idx[b], samp_s);
+    } else {                                   // randint(batch_key, (B,), 0, N): every rank draws all B indices
+      r = randint_impl(key_h, key_d, 32, 0, sampler->n_records, w.idx[b], B, samp_s);
     }
     if (r == D3P_OK && fork && cudaEventRecord(ev_sampled[b], samp_s) != cudaSuccess) r = D3P_ERR_CUDA;
     return r;

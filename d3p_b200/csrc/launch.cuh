@@ -45,6 +45,8 @@ int32_t step_vae_impl(const d3p_vae_desc* desc, const float* params_d, const flo
                       void* const* profile_events_h, d3p_vae_ctx* ctx, void* stream, float* eval_loss_d = nullptr);
 int32_t feistel_sample_impl(const uint32_t* rc_h, const uint32_t* rc_d, uint32_t capacity, uint32_t first_pos, uint32_t n,
                             int32_t* idx_d, void* stream);
+int32_t randint_impl(const uint32_t* key_h, const uint32_t* key_d, uint32_t nbits, int64_t minval, int64_t maxval,
+                     void* out_d, size_t n, void* stream);
 int32_t poisson_sample_impl(const uint32_t* state_h, const uint32_t* state_d, float q, uint32_t n_records, uint32_t max_b,
                             int32_t suppress, int32_t* idx_d, int32_t* counts_d, uint8_t* mask_d, void* ws_d,
                             size_t ws_bytes, void* stream);

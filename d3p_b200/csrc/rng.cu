@@ -1,6 +1,10 @@
 // K1: ChaCha20 keystream kernels (+ uniform / normal transforms, randint round) and the
 // host-side key plumbing of the rng suite.  Replaces jax-chacha-prng behind
 // d3p/random/__init__.py:28-155.
+#include <math.h>
+
+#include <type_traits>
+
 #include "common.cuh"
 #include "launch.cuh"
 
@@ -78,6 +82,78 @@ __global__ void randint_finish_kernel(const uint32_t* vals, int32_t minval, T* o
     out[i] = (T)(uint32_t)(vals[i] + (uint32_t)minval);
 }
 
+// The whole rejection loop of rng_suite.randint (d3p/random/__init__.py:84-146) in one launch.  A thread owns one ChaCha
+// block of outputs (kPerBlock elements) and walks the round-key chain (key, round_key) = split(key, 2) by itself,
+// drawing bit field e of round_key_r's block b until every element of its block has been accepted: element e keeps the
+// draw of the first round r with bits(round_key_r)[e] & bitmask <= delta, which is what the per-round loop keeps.
+// There is no round cap.  Accepted fields are packed into `acc` exactly as the keystream packs them, so the block's
+// 64 output bytes are written as four 16-byte vectors.
+template <int NBITS>
+__global__ void __launch_bounds__(256) randint_kernel(ChaChaArg key, uint32_t bitmask, uint32_t delta, uint32_t minval,
+                                                      void* out, size_t n) {
+  constexpr int kPerWord = 32 / NBITS, kPerBlock = 16 * kPerWord;
+  constexpr uint32_t kFieldMask = NBITS == 32 ? 0xFFFFFFFFu : ((1u << (NBITS & 31)) - 1u);
+  ChaChaState k0;
+  load_chacha(key, k0);
+  const size_t n_blocks = (n + kPerBlock - 1) / kPerBlock;
+  for (size_t b = (size_t)blockIdx.x * blockDim.x + threadIdx.x; b < n_blocks;
+       b += (size_t)gridDim.x * blockDim.x) {
+    const size_t base = b * kPerBlock;
+    const int valid = n - base < (size_t)kPerBlock ? (int)(n - base) : kPerBlock;
+    using Mask = typename std::conditional<kPerBlock == 64, uint64_t, uint32_t>::type;
+    // elements of this block not yet accepted (bit i = element i; kPerBlock may be narrower than Mask)
+    Mask pending = valid == (int)(8 * sizeof(Mask)) ? ~(Mask)0 : (((Mask)1 << valid) - 1);
+    uint32_t acc[16];
+#pragma unroll
+    for (int w = 0; w < 16; ++w) acc[w] = 0;
+    uint32_t chain[16];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) chain[i] = k0.w[i];
+    while (pending) {
+      uint32_t rk[16], next[16], ks[16];
+      chacha_derive_key(chain, 1u, D3P_DERIVE_SPLIT, rk);
+      chacha_derive_key(chain, 0u, D3P_DERIVE_SPLIT, next);
+#pragma unroll
+      for (int i = 0; i < 16; ++i) chain[i] = next[i];
+      chacha20_block(rk, rk[12] + (uint32_t)b, ks);
+#pragma unroll
+      for (int i = 0; i < kPerBlock; ++i) {
+        const int sh = (i % kPerWord) * NBITS;
+        const uint32_t v = ((ks[i / kPerWord] >> sh) & kFieldMask) & bitmask;
+        if (((pending >> i) & 1) && v <= delta) {
+          acc[i / kPerWord] |= v << sh;
+          pending &= ~((Mask)1 << i);
+        }
+      }
+    }
+    // + minval in the arithmetic of the result type (wraps like vdtype(uvals) + minval, d3p/random/__init__.py:145)
+#pragma unroll
+    for (int w = 0; w < 16; ++w) {
+      uint32_t r = 0;
+#pragma unroll
+      for (int j = 0; j < kPerWord; ++j)
+        r |= ((((acc[w] >> (j * NBITS)) & kFieldMask) + minval) & kFieldMask) << (j * NBITS);
+      acc[w] = r;
+    }
+    uint8_t* o = static_cast<uint8_t*>(out) + base * (NBITS / 8);
+    if (valid == kPerBlock && (reinterpret_cast<uintptr_t>(o) & 15) == 0) {
+      uint4* o4 = reinterpret_cast<uint4*>(o);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) o4[i] = make_uint4(acc[4 * i], acc[4 * i + 1], acc[4 * i + 2], acc[4 * i + 3]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < kPerBlock; ++i) {
+        if (i < valid) {
+          const uint32_t v = (acc[i / kPerWord] >> ((i % kPerWord) * NBITS)) & kFieldMask;
+          if (NBITS == 8) o[i] = (uint8_t)v;
+          else if (NBITS == 16) reinterpret_cast<uint16_t*>(o)[i] = (uint16_t)v;
+          else reinterpret_cast<uint32_t*>(o)[i] = v;
+        }
+      }
+    }
+  }
+}
+
 // ---- device-resident keys (the *_dk entry points) -------------------------------------------------------------------
 // The reference runs get_batch + update as the body of a jitted fori_loop with TRACED keys
 // (examples/logistic_regression.py:149-160, d3p/random/__init__.py:28-32): a key there is a device value no host ever
@@ -153,6 +229,30 @@ static int32_t launch_stream(const uint32_t* state_h, const uint32_t* state_d, u
   if (grid > (size_t)sm_count() * 16) grid = (size_t)sm_count() * 16;
   chacha_stream_kernel<kMode><<<(unsigned)grid, threads, 0, (cudaStream_t)stream>>>(
       chacha_arg(state_h, state_d), (uint32_t)first_block, out_d, n, lo, hi);
+  return check_launch();
+}
+
+int32_t randint_impl(const uint32_t* key_h, const uint32_t* key_d, uint32_t nbits, int64_t minval, int64_t maxval,
+                     void* out_d, size_t n, void* stream) {
+  if (nbits != 8 && nbits != 16 && nbits != 32) return D3P_ERR_UNSUPPORTED;
+  if (n == 0) return D3P_OK;
+  if ((!key_h && !key_d) || !out_d) return D3P_ERR_INVALID_ARGUMENT;
+  // delta = (maxval - 1 - minval) mod 2^nbits; the arithmetic is done unsigned so that it wraps without overflow
+  const uint32_t full = nbits == 32 ? 0xFFFFFFFFu : (1u << nbits) - 1u;
+  const uint32_t delta = (uint32_t)((uint64_t)maxval - 1u - (uint64_t)minval) & full;
+  const uint32_t bitmask = d3p_randint_bitmask(nbits, delta);
+  const size_t per_block = 512 / nbits;
+  const size_t n_blocks = (n + per_block - 1) / per_block;
+  size_t grid = (n_blocks + 255) / 256;
+  if (grid > (size_t)sm_count() * 16) grid = (size_t)sm_count() * 16;
+  const ChaChaArg key = chacha_arg(key_h, key_d);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (nbits == 8)
+    randint_kernel<8><<<(unsigned)grid, 256, 0, s>>>(key, bitmask, delta, (uint32_t)minval, out_d, n);
+  else if (nbits == 16)
+    randint_kernel<16><<<(unsigned)grid, 256, 0, s>>>(key, bitmask, delta, (uint32_t)minval, out_d, n);
+  else
+    randint_kernel<32><<<(unsigned)grid, 256, 0, s>>>(key, bitmask, delta, (uint32_t)minval, out_d, n);
   return check_launch();
 }
 
@@ -302,6 +402,27 @@ int32_t d3p_randint_finish_i32(const uint32_t* vals_d, int32_t minval, int32_t* 
   return d3p_randint_finish(vals_d, minval, 32, out_d, n, stream);
 }
 
+// log_po2 = min(int(float32(log2(float32(delta))) + 1), nbits) of randint (d3p/random/__init__.py:84-146).  Rounding delta and
+// its log2 to float32 widens the mask by one bit just below powers of two (delta = 2^25 - 1 rounds to 2^25, and
+// log2(2^24 - 1) rounds to 24); the reference does this, so it is kept.  log2 is taken in double and rounded once to float32, i.e. a correctly rounded
+// log2f: near an integer the float32 result is far from a rounding tie, so every faithful log2f agrees with it.
+uint32_t d3p_randint_bitmask(uint32_t nbits, uint32_t delta) {
+  if (nbits == 0) return 0;
+  if (nbits > 32) nbits = 32;
+  uint32_t log_po2 = 0;
+  if (delta > 0) {
+    const float l = (float)log2((double)(float)delta);
+    log_po2 = (uint32_t)(l + 1.0f);
+  }
+  if (log_po2 > nbits) log_po2 = nbits;
+  return log_po2 >= 32 ? 0xFFFFFFFFu : (1u << log_po2) - 1u;
+}
+
+int32_t d3p_chacha_randint(const uint32_t key_h[16], uint32_t nbits, int64_t minval, int64_t maxval, void* out_d,
+                           size_t n, void* stream) {
+  return randint_impl(key_h, nullptr, nbits, minval, maxval, out_d, n, stream);
+}
+
 
 // ---- device-key forms (keys never leave the device) ------------------------------------------------------------------
 int32_t d3p_chacha_split_dk(const uint32_t* in_d, int32_t num, uint32_t* out_d, void* stream) {
@@ -331,6 +452,11 @@ int32_t d3p_chacha_uniform_f32_dk(const uint32_t* state_d, uint64_t first_block,
 
 int32_t d3p_chacha_normal_f32_dk(const uint32_t* state_d, uint64_t first_block, float* out_d, size_t n, void* stream) {
   return launch_stream<kNormal>(nullptr, state_d, first_block, out_d, n, 0.f, 1.f, stream);
+}
+
+int32_t d3p_chacha_randint_dk(const uint32_t* key_d, uint32_t nbits, int64_t minval, int64_t maxval, void* out_d,
+                              size_t n, void* stream) {
+  return randint_impl(nullptr, key_d, nbits, minval, maxval, out_d, n, stream);
 }
 
 int32_t d3p_dpsvi_keys_dk(uint32_t* rng_key_io_d, uint32_t n_leaves, uint32_t* threefry_key_out_d,

@@ -214,9 +214,9 @@ def subsample_batchify_data(dataset, batch_size=None, q=None, with_replacement=F
             return batch, torch.ones(batch_size, dtype=torch.bool, device=ret_idx.device)
         return batch
 
-    if not with_replacement:
-        get_batch.spec = dict(kind=_n.SAMPLER_SUBSAMPLE, q=0.0, n_records=num_records, batch=int(batch_size),
-                              suppress=False, dataset=dataset, rng_suite=rng_suite)
+    get_batch.spec = dict(kind=_n.SAMPLER_SUBSAMPLE_REPLACE if with_replacement else _n.SAMPLER_SUBSAMPLE, q=0.0,
+                          n_records=num_records, batch=int(batch_size), suppress=False, dataset=dataset,
+                          rng_suite=rng_suite)
     return init, get_batch
 
 

@@ -139,8 +139,8 @@ _INT_DTYPES = {torch.int8: (8, torch.int8), np.int8: (8, torch.int8), "int8": (8
 
 def randint(key: PRNGState, shape: Sequence[int], minval, maxval, dtype=torch.int32) -> torch.Tensor:
     """``d3p/random/__init__.py:84-146``: power-of-two mask + rejection on ``random_bits(round_key, nbits, shape)`` with
-    nbits the width of the result type, one fresh key pair per round.  The loop condition needs one 4-byte
-    device->host read per round."""
+    nbits the width of the result type, one fresh key pair per round.  The whole rejection loop is one launch
+    (``d3p_chacha_randint``), so the call never synchronises with the host and can be captured in a CUDA graph."""
     try:
         np_dt = np.dtype(dtype) if not isinstance(dtype, torch.dtype) else None
     except TypeError:
@@ -148,28 +148,13 @@ def randint(key: PRNGState, shape: Sequence[int], minval, maxval, dtype=torch.in
     if dtype not in _INT_DTYPES and not (np_dt is not None and np_dt.type in _INT_DTYPES):
         raise TypeError(f"dtype argument to `randint` must be an integer dtype, got {dtype}")
     nbits, out_dtype = _INT_DTYPES[dtype] if dtype in _INT_DTYPES else _INT_DTYPES[np_dt.type]
-    full = (1 << nbits) - 1
     shape = _shape(shape)
     size = int(np.prod(shape)) if len(shape) else 1
-    delta = (int(maxval) - 1 - int(minval)) & full
-    log_po2 = min(int(np.float32(np.log2(np.float32(delta))) + np.float32(1)) if delta > 0 else 0, nbits)
-    bitmask = ((1 << log_po2) - 1) & full
-    dev = _device()
-    vals = torch.empty(max(size, 1), dtype=torch.int32, device=dev)
-    pending = torch.zeros(1, dtype=torch.int32, device=dev)
-    first = 1
-    while True:
-        ks = split(key, 2)
-        key, round_key = ks[0], ks[1]
-        a, p = _state(round_key)
-        _n.check(_n.lib().d3p_chacha_randint_round(p, nbits, bitmask, delta, first, _n.ptr(vals), size, _n.ptr(pending),
-                                                   _n.stream_ptr()), "randint")
-        first = 0
-        if int(pending.item()) == 0:
-            break
-    out = torch.empty(max(size, 1), dtype=out_dtype, device=dev)
-    minval32 = ((int(minval) + (1 << 31)) & 0xFFFFFFFF) - (1 << 31)      # the addition wraps in the result type
-    _n.check(_n.lib().d3p_randint_finish(_n.ptr(vals), minval32, nbits, _n.ptr(out), size, _n.stream_ptr()), "randint")
+    # only the low nbits of the bounds matter (the arithmetic wraps in the result type); int64 carries them to C
+    lo, hi = (((int(v) + (1 << 63)) & ((1 << 64) - 1)) - (1 << 63) for v in (minval, maxval))
+    a, p = _state(key)
+    out = torch.empty(max(size, 1), dtype=out_dtype, device=_device())
+    _n.check(_n.lib().d3p_chacha_randint(p, nbits, lo, hi, _n.ptr(out), size, _n.stream_ptr()), "randint")
     return out[:size].reshape(shape)
 
 

@@ -432,8 +432,8 @@ class DPSVI:
         (``examples/logistic_regression.py:149-160``): returns ``(new_state, stats)`` where
         ``stats[num_steps, 3]`` holds ``(loss, n, f)`` per step on the device.
 
-        For the model families fed by ``poisson_batchify_data`` / ``subsample_batchify_data`` /
-        ``split_batchify_data`` the whole loop runs inside the family's ``d3p_dpsvi_run_epoch_*`` driver (no
+        For the model families fed by ``poisson_batchify_data`` / ``subsample_batchify_data`` (with or without
+        replacement) / ``split_batchify_data`` the whole loop runs inside the family's ``d3p_dpsvi_run_epoch_*`` driver (no
         interpreter between launches); the result is bit-identical to the step-by-step calls, which remain the path for
         everything else (NCCL-backend sharded runs, custom batchifiers, a family without a driver
         (``Family.epoch_driver``: ``AutoDiagonalNormalModel``), the key modes or sharded runs a family has

@@ -87,6 +87,16 @@ int32_t d3p_randint_finish_i32(const uint32_t* vals_d, int32_t minval, int32_t* 
 int32_t d3p_chacha_randint_round(const uint32_t round_state_h[16], uint32_t nbits, uint32_t bitmask, uint32_t delta,
                                  int32_t first, uint32_t* vals_d, size_t n, int32_t* pending_d, void* stream);
 int32_t d3p_randint_finish(const uint32_t* vals_d, int32_t minval, uint32_t nbits, void* out_d, size_t n, void* stream);
+/* The whole of d3p.random.randint(key, (n,), minval, maxval, int{nbits}) (d3p/random/__init__.py:84-146) in one launch,
+ * with no host synchronisation: key_h is the key randint receives (the kernel does the first split itself); out_d is
+ * int8 / int16 / int32 for nbits = 8, 16, 32 and gets the values of the per-round loop above bit for bit.
+ * nbits outside {8, 16, 32}: D3P_ERR_UNSUPPORTED; n == 0: D3P_OK without a launch; a null pointer with n > 0:
+ * D3P_ERR_INVALID_ARGUMENT.  Both refusals come before any launch. */
+int32_t d3p_chacha_randint(const uint32_t key_h[16], uint32_t nbits, int64_t minval, int64_t maxval, void* out_d,
+                           size_t n, void* stream);
+/* randint's rejection mask for delta = (maxval - 1 - minval) mod 2^nbits: 2^log_po2 - 1 with
+ * log_po2 = min(int(float32(log2(float32(delta))) + 1), nbits) and 0 for delta == 0 (host only, no device work). */
+uint32_t d3p_randint_bitmask(uint32_t nbits, uint32_t delta);
 
 /* ------------------------------------------------------------------------------------------
  * Minibatch samplers — replace d3p/util.py:216-301 and d3p/minibatch.py:29-39,103-131,217-237.
@@ -318,6 +328,8 @@ int32_t d3p_adadp_finish_f32(const d3p_optim_desc* optim_h, uint32_t P, float* p
 #define D3P_SAMPLER_SPLIT 2     /* split_batchify_data (d3p/minibatch.py:242-312): step i takes records
                                    perm_d[i * batch, (i + 1) * batch) of the epoch's shuffle; no sampler kernel, the batch
                                    key is unused */
+#define D3P_SAMPLER_SUBSAMPLE_REPLACE 3 /* subsample_batchify_data(with_replacement=True): batch indices drawn with
+                                           d3p_chacha_randint(fold_in(batch_key, i), 32, 0, n_records) */
 
 typedef struct {
   int32_t kind;          /* D3P_SAMPLER_*                                            */
@@ -596,6 +608,9 @@ int32_t d3p_chacha_random_bits_dk(const uint32_t* state_d, uint64_t first_block,
 int32_t d3p_chacha_uniform_f32_dk(const uint32_t* state_d, uint64_t first_block, float lo, float hi, float* out_d,
                                   size_t n, void* stream);
 int32_t d3p_chacha_normal_f32_dk(const uint32_t* state_d, uint64_t first_block, float* out_d, size_t n, void* stream);
+/* d3p_chacha_randint with the key in device memory. */
+int32_t d3p_chacha_randint_dk(const uint32_t* key_d, uint32_t nbits, int64_t minval, int64_t maxval, void* out_d,
+                              size_t n, void* stream);
 /* The keys of one DPSVI.update (d3p/svi.py:208-211,413-414,490-491) from the state key, which is advanced in place:
  * (carry, k_grad, k_noise) = split(key, 3); key := carry; threefry_key_out_d[2] = convert_to_jax_rng_key(k_grad);
  * site_states_out_d[n_leaves][16] = split(k_noise, n_leaves). */
