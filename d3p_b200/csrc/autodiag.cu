@@ -1,8 +1,8 @@
 // AutoDiagonalNormal guide over a user model: the guide draw and the per-example gradient / clip / clipped sum of
 // a DP-VI step, around a model log density that the caller differentiates itself (see include/d3p_b200.h).
 //
-// The draw restates the fused families' joint-site plumbing (meanfield_step.cu, evaluate.cu) on the common.cuh
-// Threefry functions.  The step is two passes over the caller's [rows, ld] arrays h (= dU/dtheta) and eps:
+// The draw is the fused families' joint-site draw: the guide_rng / next_site key chain of common.cuh, then one
+// normal per element.  The step is two passes over the caller's [rows, ld] arrays h (= dU/dtheta) and eps:
 //   pass 1 (autodiag_rows_kernel): one CTA per row; norm of (gl, gs), |eps|^2 -> c_i and S * loss_i;
 //   pass 2 (autodiag_colsum_kernel): column tiles x example splits; sum_i c_i (gl_i, gs_i), sum S loss_i, count.
 // gl and gs are formed on the fly from (h, eps) and the per-element constants a = s' and (1/S) a / s of a small
@@ -33,10 +33,8 @@ template <bool kEval>
 __global__ void __launch_bounds__(kAdThreads) autodiag_draw_kernel(DrawArgs a) {
   const TfKey K = tf_key_arg(a.k0, a.k1, a.key_d);
   for (uint32_t r = blockIdx.x; r < a.rows; r += gridDim.x) {
-    const TfKey kp = kEval ? K : tf_example_key(K, a.B, a.pos_begin + r);   // jax.random.split(key, B)[p]
-    TfKey model_seed, guide_seed, rng, k_site;
-    tf_split2(kp, model_seed, guide_seed);             // Trace_ELBO: model_seed, guide_seed
-    tf_split2(guide_seed, rng, k_site);                // seed handler: the `_auto_latent` site
+    TfKey rng = guide_rng(kEval ? K : tf_example_key(K, a.B, a.pos_begin + r));   // jax.random.split(key, B)[p]
+    const TfKey k_site = next_site(rng);               // the `_auto_latent` site
     float* th = a.theta + (size_t)r * a.ld;
     float* ep = a.eps + (size_t)r * a.ld;
     for (uint32_t j = threadIdx.x; j < a.half; j += kAdThreads) {

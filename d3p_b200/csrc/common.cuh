@@ -141,6 +141,23 @@ D3P_HD TfKey tf_example_key(const TfKey& K, uint32_t B, uint32_t p) {
   return TfKey(tf_split_word(K, B, 2u * p), tf_split_word(K, B, 2u * p + 1u));
 }
 
+// numpyro's seed-handler plumbing under Trace_ELBO: (model_seed, guide_seed) = split(kp); the guide's handler then
+// takes one split per latent site, in the order the guide samples them:
+//   rng = guide_rng(kp); k_site0 = next_site(rng); k_site1 = next_site(rng); ...
+D3P_HD TfKey guide_rng(const TfKey& kp) {
+  TfKey model_seed, guide_seed;
+  tf_split2(kp, model_seed, guide_seed);
+  return guide_seed;
+}
+
+// (rng, site) = split(rng); returns site
+D3P_HD TfKey next_site(TfKey& rng) {
+  TfKey next, site;
+  tf_split2(rng, next, site);
+  rng = next;
+  return site;
+}
+
 // ---- bits -> uniform -> normal (jax.random._uniform / _normal_real) -------------------------
 D3P_HD float bits_to_unit_float(uint32_t bits) {
 #ifdef __CUDA_ARCH__

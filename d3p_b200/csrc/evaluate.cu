@@ -28,9 +28,8 @@ __global__ void __launch_bounds__(kEvalThreads) meanfield_eval_kernel(EvalArgs a
   __shared__ float red[kEvalThreads / 32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const TfKey K = tf_key_arg(a.k0, a.k1, a.key_d);
-  TfKey model_seed, guide_seed, rng, k_main;
-  tf_split2(K, model_seed, guide_seed);
-  tf_split2(guide_seed, rng, k_main);
+  TfKey rng = guide_rng(K);
+  const TfKey k_main = next_site(rng);
   float pq = 0.f;                           // log p(theta) - log q(theta), accumulated by every CTA, used from CTA 0
   const float kLogSqrt2Pi = 0.918938533f;
   for (uint32_t c = threadIdx.x; c < a.half; c += kEvalThreads) {
@@ -51,8 +50,7 @@ __global__ void __launch_bounds__(kEvalThreads) meanfield_eval_kernel(EvalArgs a
   }
   float th_b = 0.f;
   if (a.has_b) {
-    TfKey rng2, k_b;
-    tf_split2(rng, rng2, k_b);
+    const TfKey k_b = next_site(rng);
     uint32_t y0, y1;
     threefry2x32(k_b, 0u, 0u, y0, y1);
     const float eps = bits_to_normal<false>(y0);
@@ -71,13 +69,10 @@ __global__ void __launch_bounds__(kEvalThreads) meanfield_eval_kernel(EvalArgs a
     float s = 0.f;
     if (a.family == D3P_FAMILY_LOGREG) {
       for (uint32_t j = lane; j < a.d; j += 32) s = fmaf(xr[j], th[j], s);
-      s = group_sum<32>(s);
-      const float z = s + th_b, yv = (float)a.y[row];
-      s = -(fmaxf(z, 0.f) + log1pf(expf(-fabsf(z))) - z * yv);
+      s = row_loglik<D3P_FAMILY_LOGREG>(group_sum<32>(s), th_b, (float)a.y[row], a.d, a.inv_var, a.log_norm_lik);
     } else {
       for (uint32_t j = lane; j < a.d; j += 32) { const float q = xr[j] - th[j]; s = fmaf(q, q, s); }
-      s = group_sum<32>(s);
-      s = -0.5f * s * a.inv_var - (float)a.d * a.log_norm_lik;
+      s = row_loglik<D3P_FAMILY_GAUSS>(group_sum<32>(s), th_b, 0.f, a.d, a.inv_var, a.log_norm_lik);
     }
     ll += s;                                  // identical on every lane
   }
@@ -124,22 +119,15 @@ extern "C" int32_t d3p_elbo_evaluate_meanfield(const d3p_meanfield_desc* desc, c
   if (desc->family != D3P_FAMILY_LOGREG && desc->family != D3P_FAMILY_GAUSS) return D3P_ERR_UNSUPPORTED;
   if (desc->family == D3P_FAMILY_LOGREG && !y_d) return D3P_ERR_INVALID_ARGUMENT;
   if (ws_bytes < d3p_elbo_evaluate_workspace_bytes()) return D3P_ERR_WORKSPACE;
+  MeanfieldSite site;
+  if (!meanfield_site(desc, x_row_stride, site)) return D3P_ERR_INVALID_ARGUMENT;
   EvalArgs a;
   a.params = params_d; a.x = x_d; a.x_stride = x_row_stride; a.y = y_d; a.idx = idx_d; a.B = B;
   a.k0 = threefry_key_h[0]; a.k1 = threefry_key_h[1]; a.key_d = nullptr;
-  a.d = desc->d;
-  a.n_main = (desc->joint_site && desc->family == D3P_FAMILY_LOGREG) ? desc->d + 1 : desc->d;
-  a.half = (a.n_main + 1) / 2;
+  a.d = desc->d; a.n_main = site.n_main; a.half = site.half;
   a.loc_off = desc->loc_off; a.rho_off = desc->rho_off; a.b_loc_off = desc->b_loc_off; a.b_rho_off = desc->b_rho_off;
-  a.family = desc->family; a.link = desc->link;
-  a.has_b = (desc->family == D3P_FAMILY_LOGREG && !desc->joint_site) ? 1 : 0;
-  a.N = desc->num_obs_total;
-  a.inv_var = 0.f; a.log_norm_lik = 0.f;
-  if (desc->family == D3P_FAMILY_GAUSS) {
-    if (!(desc->lik_scale > 0.f)) return D3P_ERR_INVALID_ARGUMENT;
-    a.inv_var = 1.0f / (desc->lik_scale * desc->lik_scale);
-    a.log_norm_lik = logf(2.50662827463f * desc->lik_scale);
-  }
+  a.family = desc->family; a.link = desc->link; a.has_b = site.has_b;
+  a.N = desc->num_obs_total; a.inv_var = site.inv_var; a.log_norm_lik = site.log_norm_lik;
   a.partials = static_cast<float*>(ws_d);
   a.loss = loss_d;
   const size_t smem = (size_t)(a.n_main + 1) * sizeof(float);

@@ -168,12 +168,8 @@ __global__ void __launch_bounds__(kGmmThreads, 2) gmm_step_kernel(GmmArgs a) {
     const uint32_t row = a.idx ? (uint32_t)a.idx[p] : p;
     for (uint32_t j = tid; j < d; j += kGmmThreads) xs[j] = a.x[(size_t)row * a.x_stride + j];
     // per-example keys: key_p -> (_, guide_seed) -> site keys of pis, mus, sigs (one split each)
-    TfKey kp = tf_example_key(Kk, a.B, p);
-    TfKey model_seed, guide_seed, rng1, k_pis, rng2, k_mus, rng3, k_sigs;
-    tf_split2(kp, model_seed, guide_seed);
-    tf_split2(guide_seed, rng1, k_pis);
-    tf_split2(rng1, rng2, k_mus);
-    tf_split2(rng2, rng3, k_sigs);
+    TfKey rng = guide_rng(tf_example_key(Kk, a.B, p));
+    const TfKey k_pis = next_site(rng), k_mus = next_site(rng), k_sigs = next_site(rng);
 
     // ---- A1: sigs[m] = 1 / gamma(split(k_sigs, n)[m], 1); lane-level work queue ---------------------------
     {
@@ -359,12 +355,8 @@ __global__ void __launch_bounds__(kGmmThreads) gmm_eval_draw_kernel(GmmEvalArgs 
   const float lgam_sum = block_sum<NW>(lgam_part, red, lane, warp);
   const float log_norm_q_pis = lgammaf(alpha_sum) - lgam_sum;
   __syncthreads();
-  const TfKey Ke(a.k0, a.k1);
-  TfKey model_seed, guide_seed, rng1, k_pis, rng2, k_mus, rng3, k_sigs;
-  tf_split2(Ke, model_seed, guide_seed);
-  tf_split2(guide_seed, rng1, k_pis);
-  tf_split2(rng1, rng2, k_mus);
-  tf_split2(rng2, rng3, k_sigs);
+  TfKey rng = guide_rng(TfKey(a.k0, a.k1));
+  const TfKey k_pis = next_site(rng), k_mus = next_site(rng), k_sigs = next_site(rng);
   {   // sigs[m] = 1 / gamma(split(k_sigs, n)[m], 1): lane-level work queue (see gmm_step_kernel A1)
     const float dd = 1.0f - 1.0f / 3.0f, cc = (1.0f / 3.0f) / sqrtf(dd);
     uint32_t m = tid;

@@ -24,6 +24,16 @@ inline int32_t check_launch() { return cudaGetLastError() == cudaSuccess ? D3P_O
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// What the mean-field step and evaluate kernels derive from a descriptor.  meanfield_site returns false when the
+// descriptor is malformed (an unknown family or link, d == 0, a site that does not fit n_params, a missing intercept
+// offset), the Gaussian scale is not positive or rows are shorter than d.
+struct MeanfieldSite {
+  uint32_t n_main, half;      // main latent site: d elements, + 1 for a logreg intercept in the joint site
+  int has_b;                  // logreg with the intercept as a separate site
+  float inv_var, log_norm_lik;  // Gaussian: 1 / scale^2, log(sqrt(2 pi) scale); else 0
+};
+bool meanfield_site(const d3p_meanfield_desc* d, size_t x_row_stride, MeanfieldSite& site);
+
 // Bodies of the public entry points that come as a host-key / device-key pair (d3p_x and d3p_x_dk): each takes its key
 // as a (key_h, key_d) pair of which one is non-null, so a caller that serves both key modes (the epoch drivers) makes
 // one call.  Arguments as in include/d3p_b200.h.

@@ -49,5 +49,43 @@ D3P_D float gsum(float v, unsigned m) {
   return v;
 }
 
+struct InterceptGuide { float loc, s, a, bt; };   // the separate intercept site: loc, s, s', (1/S) s'/s (link_terms)
+
+// log p(x_i | theta) of one example.  Bernoulli-logit (numpyro BernoulliLogits.log_prob): r = x . theta of the main
+// site, th_b the intercept; Gaussian: r = sum (x - theta)^2 over the n elements of the row.
+template <int FAMILY>
+D3P_D float row_loglik(float r, float th_b, float y, uint32_t n, float inv_var, float log_norm_lik) {
+  if (FAMILY == D3P_FAMILY_LOGREG) {
+    const float z = r + th_b;
+    return -(fmaxf(z, 0.f) + log1pf(expf(-fabsf(z))) - z * y);
+  }
+  return -0.5f * r * inv_var - (float)n * log_norm_lik;
+}
+
+// Per-example ELBO terms of the step kernels from the group-reduced sums (r as in row_loglik, |theta|^2, |eps|^2
+// of the main site over its n elements): the intercept's draw th_b = loc + eb s joins the sums, then
+//   S * loss_i = -(log p(theta) - log q(theta)) - N * loglik     (the sqrt(2 pi) terms cancel; returned)
+//   Lr = L (sigmoid(z) - y)                                       (logreg; 0 for the Gaussian family)
+template <int FAMILY>
+D3P_D float example_loss(const StepArgs& a, const InterceptGuide& b, float eb, float y, float r, float s_th2,
+                         float s_e2, float sum_log_s, uint32_t n, float& th_b, float& Lr) {
+  th_b = 0.f; Lr = 0.f;
+  if (a.has_b) { th_b = fmaf(eb, b.s, b.loc); s_th2 = fmaf(th_b, th_b, s_th2); s_e2 = fmaf(eb, eb, s_e2); }
+  const float loglik = row_loglik<FAMILY>(r, th_b, y, n, a.inv_var, a.log_norm_lik);
+  if (FAMILY == D3P_FAMILY_LOGREG) Lr = a.L * (sigmoid_f(r + th_b) - y);
+  return 0.5f * s_th2 - 0.5f * s_e2 - sum_log_s - a.N * loglik;
+}
+
+// The intercept's gradient (glb wrt its loc, gsb wrt its rho; 0 without one); returns nrm plus their squares.
+D3P_D float intercept_grad(const StepArgs& a, const InterceptGuide& b, float th_b, float eb, float Lr, float nrm,
+                           float& glb, float& gsb) {
+  glb = 0.f; gsb = 0.f;
+  if (a.has_b) {
+    glb = fmaf(th_b, a.inv_S, Lr);
+    gsb = fmaf(glb, eb * b.a, -b.bt);
+    nrm = fmaf(glb, glb, fmaf(gsb, gsb, nrm));
+  }
+  return nrm;
+}
 
 }  // namespace d3p

@@ -68,6 +68,7 @@ __global__ void __launch_bounds__(kStepThreads, 1) meanfield_step_kernel(StepArg
   float sum_log_s = 0.f;
 #pragma unroll
   for (int w = 0; w < kStepWarps; ++w) sum_log_s += s_red[w];
+  const InterceptGuide b{b_loc, b_s, b_a, b_bt};
 
   // validity of the lane's slots
   using mask_t = typename std::conditional<(NS > 32), uint64_t, uint32_t>::type;
@@ -99,14 +100,11 @@ __global__ void __launch_bounds__(kStepThreads, 1) meanfield_step_kernel(StepArg
     uint32_t my_k0 = 0, my_k1 = 0, my_row = 0;
     float my_eb = 0.f, my_y = 0.f;
     if (my_valid) {
-      TfKey kp = tf_example_key(K, a.B, my_p);          // jax.random.split(key, B)[p]
-      TfKey model_seed, guide_seed, rng, k_main;
-      tf_split2(kp, model_seed, guide_seed);             // Trace_ELBO: model_seed, guide_seed
-      tf_split2(guide_seed, rng, k_main);                // seed handler, first latent site
+      TfKey rng = guide_rng(tf_example_key(K, a.B, my_p));   // jax.random.split(key, B)[p]
+      const TfKey k_main = next_site(rng);
       my_k0 = k_main.k0; my_k1 = k_main.k1;
       if (a.has_b) {
-        TfKey rng2, k_b;
-        tf_split2(rng, rng2, k_b);                       // second latent site (intercept)
+        const TfKey k_b = next_site(rng);                // second latent site (intercept)
         uint32_t y0, y1;
         threefry2x32(k_b, 0u, 0u, y0, y1);               // random_bits(k, 32, ()) -> counts [0, pad 0]
         my_eb = bits_to_normal_fast(y0);
@@ -164,18 +162,9 @@ __global__ void __launch_bounds__(kStepThreads, 1) meanfield_step_kernel(StepArg
       s_th2 = gsum<G>(s_th2, gm);
       s_e2 = gsum<G>(s_e2, gm);
 
-      float th_b = 0.f, Lr = 0.f, loglik;
-      if (a.has_b) { th_b = fmaf(eb, b_s, b_loc); s_th2 = fmaf(th_b, th_b, s_th2); s_e2 = fmaf(eb, eb, s_e2); }
-      if (FAMILY == D3P_FAMILY_LOGREG) {
-        const float z = zdot + th_b;
-        const float sp = fmaxf(z, 0.f) + log1pf(expf(-fabsf(z)));   // numpyro BernoulliLogits.log_prob
-        loglik = -(sp - z * yv);
-        Lr = a.L * (sigmoid_f(z) - yv);
-      } else {
-        loglik = -0.5f * s_res2 * a.inv_var - (float)a.n_main * a.log_norm_lik;
-      }
-      // S * loss_i = -(log p(theta) - log q(theta)) - N * loglik ; the sqrt(2 pi) terms cancel
-      const float loss_i = 0.5f * s_th2 - 0.5f * s_e2 - sum_log_s - a.N * loglik;
+      float th_b, Lr;
+      const float loss_i = example_loss<FAMILY>(a, b, eb, yv, FAMILY == D3P_FAMILY_LOGREG ? zdot : s_res2, s_th2, s_e2,
+                                                sum_log_s, a.n_main, th_b, Lr);
 
       // ---- pass 2: gradient wrt loc (kept in xv), norm -----------------------------------------
       float nrm = 0.f;
@@ -200,13 +189,8 @@ __global__ void __launch_bounds__(kStepThreads, 1) meanfield_step_kernel(StepArg
           }
         }
       }
-      nrm = gsum<G>(nrm, gm);
-      float glb = 0.f, gsb = 0.f;
-      if (a.has_b) {
-        glb = fmaf(th_b, a.inv_S, Lr);
-        gsb = fmaf(glb, eb * b_a, -b_bt);
-        nrm = fmaf(glb, glb, fmaf(gsb, gsb, nrm));
-      }
+      float glb, gsb;
+      nrm = intercept_grad(a, b, th_b, eb, Lr, gsum<G>(nrm, gm), glb, gsb);
       const float norm = sqrtf(nrm);
       const float c = 1.0f / fmaxf(1.0f, norm / a.C);      // clip_gradient, d3p/svi.py:121-122
 
@@ -309,6 +293,20 @@ static bool desc_ok(const d3p_meanfield_desc* d) {
   return true;
 }
 
+bool meanfield_site(const d3p_meanfield_desc* d, size_t x_row_stride, MeanfieldSite& site) {
+  if (!desc_ok(d) || x_row_stride < d->d) return false;
+  if (d->family == D3P_FAMILY_GAUSS && !(d->lik_scale > 0.f)) return false;
+  site.n_main = main_site_len(d);
+  site.half = (site.n_main + 1) / 2;
+  site.has_b = (d->family == D3P_FAMILY_LOGREG && !d->joint_site) ? 1 : 0;
+  site.inv_var = 0.f; site.log_norm_lik = 0.f;
+  if (d->family == D3P_FAMILY_GAUSS) {
+    site.inv_var = 1.0f / (d->lik_scale * d->lik_scale);
+    site.log_norm_lik = logf(2.50662827463f * d->lik_scale);   // log(sqrt(2 pi) * scale)
+  }
+  return true;
+}
+
 template <int FAMILY, int LINK, int G, int NQ>
 static int32_t launch_one(const StepArgs& a, size_t smem, unsigned grid, cudaStream_t s) {
   auto kern = meanfield_step_kernel<FAMILY, LINK, G, NQ>;
@@ -349,11 +347,11 @@ int32_t d3p::step_meanfield_impl(const d3p_meanfield_desc* desc, const float* pa
                                  uint32_t pos_begin, uint32_t pos_end, const uint32_t* threefry_key_h,
                                  const uint32_t* threefry_key_d, float obs_scale, float C, float* px_norms_d,
                                  float* px_grads_d, float* px_loss_d, void* ws_d, size_t ws_bytes, void* stream) {
-  if (!desc_ok(desc) || !params_d || !x_d || (!threefry_key_h && !threefry_key_d) || !ws_d) return D3P_ERR_INVALID_ARGUMENT;
-  if (desc->family == D3P_FAMILY_LOGREG && !y_d) return D3P_ERR_INVALID_ARGUMENT;
-  if (C == 0.f || obs_scale == 0.f || B == 0 || pos_begin > pos_end || pos_end > B || x_row_stride < desc->d)
+  MeanfieldSite site;
+  if (!meanfield_site(desc, x_row_stride, site) || !params_d || !x_d || (!threefry_key_h && !threefry_key_d) || !ws_d)
     return D3P_ERR_INVALID_ARGUMENT;
-  if (desc->family == D3P_FAMILY_GAUSS && !(desc->lik_scale > 0.f)) return D3P_ERR_INVALID_ARGUMENT;
+  if (desc->family == D3P_FAMILY_LOGREG && !y_d) return D3P_ERR_INVALID_ARGUMENT;
+  if (C == 0.f || obs_scale == 0.f || B == 0 || pos_begin > pos_end || pos_end > B) return D3P_ERR_INVALID_ARGUMENT;
   uint32_t n_partials = 0;
   size_t need = d3p_meanfield_workspace_bytes(desc, &n_partials);
   if (ws_bytes < need) return D3P_ERR_WORKSPACE;
@@ -363,14 +361,10 @@ int32_t d3p::step_meanfield_impl(const d3p_meanfield_desc* desc, const float* pa
   a.k0 = threefry_key_h ? threefry_key_h[0] : 0u; a.k1 = threefry_key_h ? threefry_key_h[1] : 0u;
   a.key_d = threefry_key_d;
   a.inv_S = 1.0f / obs_scale; a.L = desc->num_obs_total / obs_scale; a.C = C; a.N = desc->num_obs_total;
-  a.inv_var = 0.f; a.log_norm_lik = 0.f;
-  if (desc->family == D3P_FAMILY_GAUSS) {
-    a.inv_var = 1.0f / (desc->lik_scale * desc->lik_scale);
-    a.log_norm_lik = logf(2.50662827463f * desc->lik_scale);   // log(sqrt(2 pi) * scale)
-  }
-  a.d = desc->d; a.n_main = main_site_len(desc); a.half = (a.n_main + 1) / 2; a.P = desc->n_params;
+  a.inv_var = site.inv_var; a.log_norm_lik = site.log_norm_lik;
+  a.d = desc->d; a.n_main = site.n_main; a.half = site.half; a.P = desc->n_params;
   a.loc_off = desc->loc_off; a.rho_off = desc->rho_off; a.b_loc_off = desc->b_loc_off; a.b_rho_off = desc->b_rho_off;
-  a.has_b = (desc->family == D3P_FAMILY_LOGREG && !desc->joint_site) ? 1 : 0;
+  a.has_b = site.has_b;
   a.px_norms = px_norms_d; a.px_grads = px_grads_d; a.px_loss = px_loss_d; a.partials = reinterpret_cast<float*>(ws_d);
   {
     int32_t rc = launch_meanfield_vec(desc->family, desc->link, a, n_partials, (cudaStream_t)stream);

@@ -1,7 +1,8 @@
 // K5a/K5b fast path: the fused mean-field step for "full" shapes d = 64 * NQ (256, 512, 1024),
 // one warp per example, 4 consecutive latent elements per lane and float4 everywhere
 // (LDG.128 row loads, LDS.128 parameter reads).  Same math and same random streams as the generic
-// kernel in meanfield_step.cu (that file documents the algebra); this one removes the per-slot
+// kernel in meanfield_step.cu (that file documents the algebra), and the same per-example ELBO terms
+// (meanfield_common.cuh); this one removes the per-slot
 // predicates, keeps the Gaussian transform branch-free (one warp-uniform tail fix-up per 4
 // variates) and exposes 4-8 independent Threefry / erf_inv chains per lane to the scheduler.
 #include "common.cuh"
@@ -92,14 +93,15 @@ __global__ void __launch_bounds__(kStepThreads, 2) meanfield_step_vec_kernel(Ste
     link_terms<LINK>(a.params[a.rho_off + e], a.inv_S, s, aa, bt, ls);
     s_loc[e] = a.params[a.loc_off + e];
     s_scl[e] = s;
-    if (!kExp) { s_a[e] = aa; s_sa[e] = s / aa; s_bt[e] = bt; }
+    // s' underflows to 0 below rho ~ -88.7 while s stays a denormal: theta = loc there, as in the generic kernel
+    if (!kExp) { s_a[e] = aa; s_sa[e] = (aa != 0.f) ? s / aa : 0.f; s_bt[e] = bt; }
     log_s_part += ls;
   }
-  float b_loc = 0.f, b_s = 0.f, b_a = 0.f, b_bt = 0.f;
+  InterceptGuide b{0.f, 0.f, 0.f, 0.f};
   if (a.has_b) {
     float ls;
-    b_loc = a.params[a.b_loc_off];
-    link_terms<LINK>(a.params[a.b_rho_off], a.inv_S, b_s, b_a, b_bt, ls);
+    b.loc = a.params[a.b_loc_off];
+    link_terms<LINK>(a.params[a.b_rho_off], a.inv_S, b.s, b.a, b.bt, ls);
     if (threadIdx.x == 0) log_s_part += ls;
   }
   log_s_part = gsum<32>(log_s_part, 0xffffffffu);
@@ -137,10 +139,11 @@ __global__ void __launch_bounds__(kStepThreads, 2) meanfield_step_vec_kernel(Ste
     uint32_t my_k0, my_k1, my_row = 0;
     float my_eb = 0.f, my_y = 0.f;
     {
-      // Key chain of example base + (lane & 15): split(K,B)[p] -> split -> guide_seed -> split ->
-      // (rng, k_main) [-> split(rng) -> k_b -> eps_b].  Every level is two independent Threefry
-      // calls ((0,2) and (1,3)); the lower / upper half-warp take one each and swap by shuffle,
-      // so the chain costs 3 (5 with an intercept) calls per tile of 16 examples instead of 6 (9) per example.
+      // Key chain of example base + (lane & 15); it must equal the guide_rng / next_site chain of common.cuh
+      // that the generic kernel runs: split(K,B)[p] -> split -> guide_seed -> split -> (rng, k_main)
+      // [-> split(rng) -> k_b -> eps_b].  Every level is two independent Threefry calls ((0,2) and (1,3)); the
+      // lower / upper half-warp take one each and swap by shuffle, so the chain costs 3 (5 with an intercept)
+      // calls per tile of 16 examples instead of 6 (9) per example.
       const uint32_t tl = lane & 15u, part = lane >> 4;
       const uint32_t w = tf_split_word(K, a.B, 2u * (base + tl) + part);
       TfKey kk(__shfl_sync(0xffffffffu, w, tl), __shfl_sync(0xffffffffu, w, tl + 16u));
@@ -230,17 +233,9 @@ __global__ void __launch_bounds__(kStepThreads, 2) meanfield_step_vec_kernel(Ste
       s_th2 = gsum<LPE>(s_th2, 0xffffffffu);
       s_e2 = gsum<LPE>(s_e2, 0xffffffffu);
 
-      float th_b = 0.f, Lr = 0.f, loglik;
-      if (a.has_b) { th_b = fmaf(eb, b_s, b_loc); s_th2 = fmaf(th_b, th_b, s_th2); s_e2 = fmaf(eb, eb, s_e2); }
-      if (FAMILY == D3P_FAMILY_LOGREG) {
-        const float z = zdot + th_b;
-        const float sp = fmaxf(z, 0.f) + log1pf(expf(-fabsf(z)));
-        loglik = -(sp - z * yv);
-        Lr = a.L * (sigmoid_f(z) - yv);
-      } else {
-        loglik = -0.5f * s_res2 * a.inv_var - (float)D * a.log_norm_lik;
-      }
-      const float loss_i = 0.5f * s_th2 - 0.5f * s_e2 - sum_log_s - a.N * loglik;
+      float th_b, Lr;
+      const float loss_i = example_loss<FAMILY>(a, b, eb, yv, FAMILY == D3P_FAMILY_LOGREG ? zdot : s_res2, s_th2, s_e2,
+                                                sum_log_s, D, th_b, Lr);
 
       // ---- loop B (logreg: needs the logit first): gradients (g_loc overwrites x, g_rho overwrites u), norm ----
 #pragma unroll 2
@@ -276,13 +271,8 @@ __global__ void __launch_bounds__(kStepThreads, 2) meanfield_step_vec_kernel(Ste
 #undef D3P_PG
         }
       }
-      nrm = gsum<LPE>(nrm, 0xffffffffu);
-      float glb = 0.f, gsb = 0.f;
-      if (a.has_b) {
-        glb = fmaf(th_b, a.inv_S, Lr);
-        gsb = fmaf(glb, eb * b_a, -b_bt);
-        nrm = fmaf(glb, glb, fmaf(gsb, gsb, nrm));
-      }
+      float glb, gsb;
+      nrm = intercept_grad(a, b, th_b, eb, Lr, gsum<LPE>(nrm, 0xffffffffu), glb, gsb);
       const float norm = sqrtf(nrm);
       const float c = act ? 1.0f / fmaxf(1.0f, norm / a.C) : 0.f;
 
