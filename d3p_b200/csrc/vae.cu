@@ -8,11 +8,11 @@
 // Pipeline (one stream, no host sync; GEMMs = 3xTF32 tcgen05 kernels of tc_gemm_kernel.cuh):
 //   split W1, W5 -> hi/lo | prep X (gather, hi/lo, ||x||^2, ones column)
 //   G1  pre1 = X W1          epilogue: + b1, softplus -> H1 hi/lo, ||h1||^2
-//   S1  heads z_loc, log z_std (K = H, N = 2Z), eps (Threefry), z, KL part, pre4 = z W4, H2 hi/lo
+//   S1  heads z_loc, log z_std (K = H, N = 2Z), eps (Threefry), z, KL part, pre4 = z W4, H2
 //   G5  logits = H2 W5       epilogue: + b5, sigmoid, Bernoulli loss, delta5 hi/lo, ||delta5||^2
 //   G5b dh2 = delta5 W5^T    epilogue: * softplus'(pre4) -> delta4, ||delta4||^2
-//   S2  delta_z, delta2/3, delta1, ghost norm, c_i; writes c*delta1 hi/lo, c*delta4, c*[delta2|delta3],
-//       [c*h2 | c] hi/lo
+//   S2  delta_z, delta2/3, delta1, ghost norm, c_i; writes c*delta1, c*delta4 hi/lo, c*[delta2|delta3] hi/lo,
+//       [c*h2 | c]
 //   GW1 [X | 1]^T (c delta1)        -> dW1, db1  (split over the batch, partial rows)
 //   GW5 delta5^T [c h2 | c]         -> dW5^T, db5
 //   GW23 [H1 | 1]^T (c [delta2|delta3]) -> dW2, dW3, db2, db3;  GW4 (c delta4)^T [z | 1] -> dW4^T, db4
@@ -30,9 +30,6 @@ namespace d3p {
 constexpr int kVaeBN = 224;            // N tile of the GEMMs with N = D (784 -> 4 tiles x 32 M tiles = 128 CTAs)
 constexpr int kVaeBNH = 128;           // N tile of the forward/backward GEMMs with N = H: 400 -> 4 tiles = 128 CTAs
                                        // (224 gave 2 tiles = 64 CTAs on 148 SMs: measured 36 / 58 us for G1 / G5b)
-constexpr int kMidWarps = 16;
-constexpr int kMidE = 2;               // examples per warp iteration in the SIMT "middle" kernels (the kernels are
-                                       // latency-bound: 16 warps x 2 examples hide more than 8 x 4 did)
 constexpr float kF32Tiny = 1.17549435e-38f;
 constexpr float kF32OneMinusEps = 0.99999988079071044921875f;   // 1 - 2^-23
 
@@ -114,7 +111,7 @@ struct EpiFwd5 {   // p = sigmoid(acc + b5); Bernoulli(probs) log-lik (numpyro c
 };
 
 struct EpiBwd5 {   // delta4 = acc * softplus'(pre4) = acc * (1 - exp(-h2))
-  struct Args { const float* h_hi; const float* h_lo; size_t ld; float* d4; float* rowsq; uint32_t rows_ld; };
+  struct Args { const float* h_hi; size_t ld; float* d4; float* rowsq; uint32_t rows_ld; };
   struct RowState { float sq; };
   __device__ static void begin(const Args&, const tc::GemmShape&, uint32_t, uint32_t, uint32_t, RowState& rs) { rs.sq = 0.f; }
   __device__ static void tile(const Args& a, const tc::GemmShape& g, uint32_t row, uint32_t col0, uint32_t,
@@ -190,7 +187,7 @@ struct EpiGrad {   // clipped-sum tile -> partial row `split`: weight block(s) +
   }
 };
 
-// ---- SIMT kernels ------------------------------------------------------------------------------------
+// ---- kernels -----------------------------------------------------------------------------------------
 struct VaeArgs {
   uint32_t D, H, Z, B, Bl, pos_begin;
   size_t ldx, ldh, ldz, ld23;         // D + 4, H + 4, roundup(Z + 1, 4), roundup(2 Z, 4)
@@ -205,7 +202,7 @@ struct VaeArgs {
   uint32_t S;                         // partial rows
   // workspace
   float *x_hi, *x_lo; int* x_lo_flag;
-  float *h1_hi, *h1_lo, *h2_hi, *h2_lo, *ch2_hi, *ch2_lo, *d5_hi, *d5_lo, *d4, *cd4_hi, *cd4_lo, *cd1_hi, *cd1_lo;
+  float *h1_hi, *h1_lo, *h2_hi, *ch2_hi, *d5_hi, *d5_lo, *d4, *cd4_hi, *cd4_lo, *cd1_hi;
   float *z_hi, *z_lo, *u, *cd23_hi, *cd23_lo;
   float *sq_x, *sq_h1, *sq_h2, *sq_z, *sq_d5, *loss_rec, *sq_d4, *loss_kl, *lossv, *cnt;
   float* partials;
@@ -278,382 +275,18 @@ D3P_D float vae_eval_eps(const TfKey& K_eval, uint32_t B, uint32_t Z, uint32_t p
   return bits_to_normal<false>(y1);
 }
 
-// S1: encoder heads, guide sample, KL part of the loss, decoder hidden layer.  The three thin weight
-// matrices are staged in shared memory once per CTA; each warp walks groups of kMidE examples.
-__global__ void __launch_bounds__(kMidWarps * 32) vae_mid_fwd_kernel(VaeArgs a) {
-  extern __shared__ float smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t H = a.H, Z = a.Z, Z2 = 2 * a.Z;
-  float* w23s = smem;                                   // [H][2Z]: row k = (W2[k, :], W3[k, :])
-  float* w4s = w23s + (size_t)H * Z2;                   // [Z][H]
-  float* b23s = w4s + (size_t)Z * H;                    // [2Z]
-  float* b4s = b23s + 64;                               // [H]
-  float* wsm = b4s + H + (size_t)warp * kMidE * (H + 3 * 64);
-  float* h1s = wsm;                                     // [E][H]
-  float* zs = h1s + kMidE * H;                          // [E][64]  (z_loc | log z_std)
-  float* es = zs + kMidE * 64;                          // [E][64]  eps
-  float* zz = es + kMidE * 64;                          // [E][64]  z
-  for (uint32_t i0 = threadIdx.x; i0 < H * Z; i0 += 4 * blockDim.x) {     // 12 independent loads in flight
-    float v2[4], v3[4], v4[4];
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const uint32_t i = i0 + t * blockDim.x;
-      const bool ok = i < H * Z;
-      v2[t] = ok ? __ldg(a.params + a.off_w2 + i) : 0.f;
-      v3[t] = ok ? __ldg(a.params + a.off_w3 + i) : 0.f;
-      v4[t] = ok ? __ldg(a.params + a.off_w4 + i) : 0.f;
-    }
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const uint32_t i = i0 + t * blockDim.x;
-      if (i >= H * Z) break;
-      const uint32_t k = i / Z, j = i - k * Z;
-      w23s[k * Z2 + j] = v2[t];
-      w23s[k * Z2 + Z + j] = v3[t];
-      w4s[i] = v4[t];
-    }
-  }
-  for (uint32_t i = threadIdx.x; i < Z; i += blockDim.x) { b23s[i] = a.params[a.off_b2 + i]; b23s[Z + i] = a.params[a.off_b3 + i]; }
-  for (uint32_t i = threadIdx.x; i < H; i += blockDim.x) b4s[i] = a.params[a.off_b4 + i];
-  __syncthreads();
-  const TfKey K = tf_key_arg(a.k0, a.k1, a.key_d);
-  const uint32_t half = (Z + 1) / 2;
-  const uint32_t groups = (a.Bl + kMidE - 1) / kMidE;
-  for (uint32_t gidx = blockIdx.x * kMidWarps + warp; gidx < groups; gidx += gridDim.x * kMidWarps) {
-    const uint32_t r0 = gidx * kMidE;
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      const uint32_t r = r0 + e;
-      {
-        const float* __restrict__ ph = a.h1_hi + (size_t)r * a.ldh;
-        const float* __restrict__ pl = a.h1_lo + (size_t)r * a.ldh;
-        for (uint32_t k0 = 0; k0 < H; k0 += 128) {          // 8 independent loads in flight per lane
-          float vh[4], vl[4];
-#pragma unroll
-          for (int t = 0; t < 4; ++t) {
-            const uint32_t k = k0 + 32 * t + lane;
-            const bool ok = r < a.Bl && k < H;
-            vh[t] = ok ? __ldg(ph + k) : 0.f;
-            vl[t] = ok ? __ldg(pl + k) : 0.f;
-          }
-#pragma unroll
-          for (int t = 0; t < 4; ++t) {
-            const uint32_t k = k0 + 32 * t + lane;
-            if (k < H) h1s[e * H + k] = vh[t] + vl[t];
-          }
-        }
-      }
-      // guide noise: key_p -> (_, guide_seed) -> (rng, k_plate) -> (_, k_z); eps = normal(k_z, (Z,))
-      if (r < a.Bl && a.eval_mode) {
-        for (uint32_t j = lane; j < Z; j += 32) es[e * 64 + j] = vae_eval_eps(K, a.B, Z, a.pos_begin + r, j);
-      } else if (r < a.Bl) {
-        TfKey kp = tf_example_key(K, a.B, a.pos_begin + r);
-        TfKey model_seed, guide_seed, rng, k_plate, rng2, k_z;
-        tf_split2(kp, model_seed, guide_seed);
-        tf_split2(guide_seed, rng, k_plate);
-        tf_split2(rng, rng2, k_z);
-        for (uint32_t j = lane; j < half; j += 32) {
-          uint32_t y0, y1;
-          const uint32_t c1 = (j + half < Z) ? j + half : 0u;
-          threefry2x32(k_z, j, c1, y0, y1);
-          es[e * 64 + j] = bits_to_normal<false>(y0);
-          if (j + half < Z) es[e * 64 + j + half] = bits_to_normal<false>(y1);
-        }
-      }
-      if (r < a.Bl) {
-        if (lane < 4) {     // ones column of [H1 | 1] (bias row of the dW2 / dW3 clipped-sum GEMM)
-          a.h1_hi[(size_t)r * a.ldh + H + lane] = lane == 0 ? 1.0f : 0.f;
-          a.h1_lo[(size_t)r * a.ldh + H + lane] = 0.f;
-        }
-      }
-    }
-    __syncwarp();
-    // heads: output j < Z is z_loc_j (W2), Z <= j < 2Z is log z_std (W3); lane owns j = lane, lane + 32
-    float acc[kMidE][2];
-    const uint32_t j0 = lane, j1 = lane + 32;
-    const bool v0 = j0 < Z2, v1 = j1 < Z2;
-    const uint32_t jj0 = v0 ? j0 : 0, jj1 = v1 ? j1 : 0;
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) { acc[e][0] = 0.f; acc[e][1] = 0.f; }
-#pragma unroll 4
-    for (uint32_t k = 0; k < H; ++k) {
-      const float w0 = w23s[k * Z2 + jj0];
-      const float w1 = w23s[k * Z2 + jj1];
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) {
-        const float h = h1s[e * H + k];
-        acc[e][0] = fmaf(h, w0, acc[e][0]);
-        acc[e][1] = fmaf(h, w1, acc[e][1]);
-      }
-    }
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      if (v0) zs[e * 64 + j0] = acc[e][0] + b23s[j0];
-      if (v1) zs[e * 64 + j1] = acc[e][1] + b23s[j1];
-    }
-    __syncwarp();
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      const uint32_t r = r0 + e;
-      float kl = 0.f, sqz = 0.f;
-      for (uint32_t j = lane; j < Z; j += 32) {
-        const float zl = zs[e * 64 + j], sr = zs[e * 64 + Z + j], eps = es[e * 64 + j];
-        const float u = expf(sr) * eps;
-        const float z = zl + u;
-        zz[e * 64 + j] = z;
-        if (r < a.Bl) {
-          const float hi = tc::tf32_hi(z);
-          a.z_hi[(size_t)r * a.ldz + j] = hi;
-          a.z_lo[(size_t)r * a.ldz + j] = z - hi;
-          a.u[(size_t)r * Z + j] = u;
-        }
-        kl += 0.5f * z * z - 0.5f * eps * eps - sr;       // -log N(z;0,1) + log N(z; z_loc, z_std), constants cancel
-        sqz = fmaf(z, z, sqz);
-      }
-      if (r < a.Bl)
-        for (uint32_t j = Z + lane; j < a.ldz; j += 32) {   // ones column of [z | 1] (db4 of the dW4 GEMM) + padding
-          a.z_hi[(size_t)r * a.ldz + j] = j == Z ? 1.0f : 0.f;
-          a.z_lo[(size_t)r * a.ldz + j] = 0.f;
-        }
-      kl = group_sum<32>(kl);
-      sqz = group_sum<32>(sqz);
-      if (lane == 0 && r < a.Bl) { a.loss_kl[r] = kl; a.sq_z[r] = sqz; }
-    }
-    __syncwarp();
-    // decoder hidden layer: h2 = softplus(z W4 + b4)
-    float sq2[kMidE];
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) sq2[e] = 0.f;
-    for (uint32_t h = lane; h < H; h += 32) {
-      float s[kMidE];
-      const float b = b4s[h];
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) s[e] = b;
-#pragma unroll 4
-      for (uint32_t j = 0; j < Z; ++j) {
-        const float w = w4s[j * H + h];
-#pragma unroll
-        for (int e = 0; e < kMidE; ++e) s[e] = fmaf(zz[e * 64 + j], w, s[e]);
-      }
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) {
-        const uint32_t r = r0 + e;
-        const float h2 = softplus_f(s[e]);
-        sq2[e] = fmaf(h2, h2, sq2[e]);
-        if (r < a.Bl) {
-          const float hi = tc::tf32_hi(h2);
-          a.h2_hi[(size_t)r * H + h] = h2;          // unmasked (kind::tf32 truncates; consumers read h2 from here)
-          a.h2_lo[(size_t)r * H + h] = h2 - hi;
-        }
-      }
-    }
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      const float s = group_sum<32>(sq2[e]);
-      if (lane == 0 && r0 + e < a.Bl) a.sq_h2[r0 + e] = s;
-    }
-    __syncwarp();
-  }
-}
-
-// S2: back-propagation through the z layer and the encoder heads, ghost norm, clip factor, scaled
-// operands of the clipped-sum GEMMs.  W4, W2^T, W3^T staged in shared memory.
-__global__ void __launch_bounds__(kMidWarps * 32) vae_mid_bwd_kernel(VaeArgs a) {
-  extern __shared__ float smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const uint32_t H = a.H, Z = a.Z;
-  float* w4s = smem;                                    // [Z][H]
-  float* w2t = w4s + (size_t)Z * H;                     // [Z][H] = W2^T
-  float* w3t = w2t + (size_t)Z * H;                     // [Z][H] = W3^T
-  float* wsm = w3t + (size_t)Z * H + (size_t)warp * kMidE * (H + 128);
-  float* d4s = wsm;                                     // [E][H]
-  float* d23 = d4s + kMidE * H;                         // [E][128]: delta2 at [0,64), delta3 at [64,128)
-  for (uint32_t i0 = threadIdx.x; i0 < H * Z; i0 += 4 * blockDim.x) {     // 12 independent loads in flight
-    float v2[4], v3[4], v4[4];
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const uint32_t i = i0 + t * blockDim.x;
-      const bool ok = i < H * Z;
-      v2[t] = ok ? __ldg(a.params + a.off_w2 + i) : 0.f;
-      v3[t] = ok ? __ldg(a.params + a.off_w3 + i) : 0.f;
-      v4[t] = ok ? __ldg(a.params + a.off_w4 + i) : 0.f;
-    }
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const uint32_t i = i0 + t * blockDim.x;
-      if (i >= H * Z) break;
-      const uint32_t h = i / Z, j = i - h * Z;
-      w4s[i] = v4[t];
-      w2t[j * H + h] = v2[t];
-      w3t[j * H + h] = v3[t];
-    }
-  }
-  __syncthreads();
-  const uint32_t nv = a.num_valid ? (uint32_t)max(*a.num_valid, 0) : 0xffffffffu;
-  const float ratio = a.site_scale * a.inv_S;                   // (1 / obs_scale) * site scale
-  const uint32_t groups = (a.Bl + kMidE - 1) / kMidE;
-  for (uint32_t gidx = blockIdx.x * kMidWarps + warp; gidx < groups; gidx += gridDim.x * kMidWarps) {
-    const uint32_t r0 = gidx * kMidE;
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      const uint32_t r = r0 + e;
-      for (uint32_t h0 = 0; h0 < H; h0 += 128) {
-        float v[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const uint32_t h = h0 + 32 * t + lane;
-          v[t] = (r < a.Bl && h < H) ? __ldg(a.d4 + (size_t)r * H + h) : 0.f;
-        }
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const uint32_t h = h0 + 32 * t + lane;
-          if (h < H) d4s[e * H + h] = v[t];
-        }
-      }
-    }
-    __syncwarp();
-    // delta_z_j = z_j + sum_h delta4_h W4[j, h]; lane j keeps z_j and u_j of every example of the group
-    float sq23[kMidE], zreg[kMidE], ureg[kMidE];
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      const uint32_t r = r0 + e;
-      const bool ok = r < a.Bl && (uint32_t)lane < Z;
-      sq23[e] = 0.f;
-      zreg[e] = ok ? a.z_hi[(size_t)r * a.ldz + lane] + a.z_lo[(size_t)r * a.ldz + lane] : 0.f;
-      ureg[e] = ok ? a.u[(size_t)r * Z + lane] : 0.f;
-    }
-    for (uint32_t j = 0; j < Z; ++j) {
-      float part[kMidE];
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) part[e] = 0.f;
-#pragma unroll 4
-      for (uint32_t h = lane; h < H; h += 32) {
-        const float w = w4s[j * H + h];
-#pragma unroll
-        for (int e = 0; e < kMidE; ++e) part[e] = fmaf(d4s[e * H + h], w, part[e]);
-      }
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) {
-        const float s = group_sum<32>(part[e]);
-        if ((uint32_t)lane == j) {
-          const float dz = s + zreg[e];
-          const float d3 = fmaf(dz, ureg[e], -1.0f);
-          d23[e * 128 + j] = dz;
-          d23[e * 128 + 64 + j] = d3;
-          sq23[e] = fmaf(dz, dz, d3 * d3);
-        }
-      }
-    }
-    __syncwarp();
-    // delta_h1 = delta2 W2^T + delta3 W3^T ; delta1 = delta_h1 * softplus'(pre1); raw delta1 parked in cd1_hi
-    float sq1[kMidE];
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) sq1[e] = 0.f;
-    for (uint32_t h = lane; h < H; h += 32) {
-      float s[kMidE];
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) s[e] = 0.f;
-#pragma unroll 4
-      for (uint32_t j = 0; j < Z; ++j) {
-        const float w2 = w2t[j * H + h], w3 = w3t[j * H + h];
-#pragma unroll
-        for (int e = 0; e < kMidE; ++e) s[e] = fmaf(d23[e * 128 + j], w2, fmaf(d23[e * 128 + 64 + j], w3, s[e]));
-      }
-      float h1v[kMidE];
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) {
-        const uint32_t r = r0 + e;
-        h1v[e] = r < a.Bl ? __ldg(a.h1_hi + (size_t)r * a.ldh + h) + __ldg(a.h1_lo + (size_t)r * a.ldh + h) : 0.f;
-      }
-#pragma unroll
-      for (int e = 0; e < kMidE; ++e) {
-        const uint32_t r = r0 + e;
-        if (r < a.Bl) {
-          const float d1 = s[e] * (-expm1f(-h1v[e]));
-          a.cd1_hi[(size_t)r * H + h] = d1;
-          sq1[e] = fmaf(d1, d1, sq1[e]);
-        }
-      }
-    }
-    __syncwarp();
-#pragma unroll
-    for (int e = 0; e < kMidE; ++e) {
-      const uint32_t r = r0 + e;
-      if (r >= a.Bl) continue;                     // warp-uniform
-      const float s1 = group_sum<32>(sq1[e]);
-      const float s23 = group_sum<32>(sq23[e]);
-      // row-reduction slots of the GEMM epilogues: lane t reads slot t, fixed shuffle-tree order
-      float sq_h1 = 0.f, sq_d4 = 0.f, sq_d5 = 0.f, lrec = 0.f;
-      for (uint32_t t = lane; t < a.ns_h; t += 32) { sq_h1 += a.sq_h1[(size_t)t * a.Bl + r]; sq_d4 += a.sq_d4[(size_t)t * a.Bl + r]; }
-      for (uint32_t t = lane; t < a.ns_d; t += 32) { sq_d5 += a.sq_d5[(size_t)t * a.Bl + r]; lrec += a.loss_rec[(size_t)t * a.Bl + r]; }
-      sq_h1 = group_sum<32>(sq_h1); sq_d4 = group_sum<32>(sq_d4);
-      sq_d5 = group_sum<32>(sq_d5); lrec = group_sum<32>(lrec);
-      const float n2 = (a.sq_h2[r] + 1.0f) * sq_d5 + (a.sq_z[r] + 1.0f) * sq_d4 + (sq_h1 + 1.0f) * s23 +
-                       (a.sq_x[r] + 1.0f) * s1;
-      const float norm = fabsf(ratio) * sqrtf(n2);
-      const uint32_t p = a.pos_begin + r;
-      const bool valid = (p < nv) && (!a.mask || a.mask[p]);
-      const float c = valid ? 1.0f / fmaxf(1.0f, norm / a.C) : 0.f;
-      const float cc = c * ratio;
-      const float loss_s = valid ? a.site_scale * (a.loss_kl[r] + lrec) : 0.f;   // = obs_scale * loss_i
-      if (lane == 0) {
-        a.lossv[r] = loss_s;
-        a.cnt[r] = valid ? 1.0f : 0.f;
-        if (a.px_norms) a.px_norms[p] = valid ? norm : 0.f;
-        if (a.px_loss) a.px_loss[p] = loss_s;
-      }
-      for (uint32_t h0 = 0; h0 < H; h0 += 128) {             // batched loads: 12 in flight per lane
-        float d1v[4], h2h[4], h2l[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const uint32_t h = h0 + 32 * t + lane;
-          const bool ok = h < H;
-          d1v[t] = ok ? a.cd1_hi[(size_t)r * H + h] : 0.f;
-          h2h[t] = ok ? __ldg(a.h2_hi + (size_t)r * H + h) : 0.f;      // h2, unmasked
-          h2l[t] = 0.f;
-        }
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const uint32_t h = h0 + 32 * t + lane;
-          if (h >= H) continue;
-          const float v1 = cc * d1v[t];
-          a.cd1_hi[(size_t)r * H + h] = v1;          // unmasked: split by the dW1 GEMM itself (tc_gemm_kernel.cuh)
-          a.cd1_lo[(size_t)r * H + h] = v1 - tc::tf32_hi(v1);
-          const float v4 = cc * d4s[e * H + h];
-          const float hi4 = tc::tf32_hi(v4);
-          a.cd4_hi[(size_t)r * H + h] = hi4;
-          a.cd4_lo[(size_t)r * H + h] = v4 - hi4;
-          const float v2 = cc * (h2h[t] + h2l[t]);
-          a.ch2_hi[(size_t)r * a.ldh + h] = v2;      // unmasked, as above (dW5 GEMM)
-          a.ch2_lo[(size_t)r * a.ldh + h] = v2 - tc::tf32_hi(v2);
-        }
-      }
-      if (lane < 4) {
-        const float v = lane == 0 ? cc : 0.f;
-        a.ch2_hi[(size_t)r * a.ldh + H + lane] = v;
-        a.ch2_lo[(size_t)r * a.ldh + H + lane] = v - tc::tf32_hi(v);
-      }
-      for (uint32_t j = lane; j < a.ld23; j += 32) {
-        const float v = j < 2 * Z ? cc * (j < Z ? d23[e * 128 + j] : d23[e * 128 + 64 + j - Z]) : 0.f;
-        const float hi = tc::tf32_hi(v);
-        a.cd23_hi[(size_t)r * a.ld23 + j] = hi;
-        a.cd23_lo[(size_t)r * a.ld23 + j] = v - hi;
-      }
-    }
-    __syncwarp();
-  }
-}
-
-
 // ---- thin layers on warp-level tensor-core MMA ------------------------------------------------------------
 // The encoder heads (K = H, N = 2Z), the decoder hidden layer (K = Z, N = H) and their transposes in the backward
 // pass are far too thin for a 128-row tcgen05 tile (N = 40, K = 20) and were SIMT loops that re-read the weights
-// from shared memory per warp (47 + 55 us of the 0.40 ms step).  Here a CTA of 4 warps owns 16 examples = one
+// from shared memory per warp (47 + 55 us of the 0.40 ms step).  Here a CTA of 8 warps owns 16 examples = one
 // mma.sync m16n8k8 row block; products are 3xTF32 (a_hi b_hi + a_lo b_hi + a_hi b_lo, fp32 accumulate) like the
 // tcgen05 GEMMs.  B operands come from global memory in fragment order (one LDG.128 per lane per 8x8 block:
 // {hi(b0), hi(b1), lo(b0), lo(b1)}), written once per step by vae_prep_mid_kernel.  The reduction index is
 // permuted so that a lane's two k slots (t, t + 4) are adjacent columns (2t, 2t + 1) in memory: A rows are read
-// as 8-byte pairs.  Shapes: H % 8 == 0, Z % 4 == 0, Z <= 32; other shapes keep the SIMT kernels above.
+// as 8-byte pairs.  Every shape (H % 4 == 0, 1 <= Z <= 32) is padded to whole 8 x 8 blocks: the B fragments are
+// zero outside the matrices, the A operands are zero past K (never whatever the workspace holds there: 0 * NaN is
+// NaN), and columns past N are neither stored nor summed.  H is even, so a lane's column pair (n, n + 1) is
+// either inside or outside H.
 constexpr int kMmaRows = 16;
 constexpr int kMmaWarps = 8;              // the kernels are latency-bound (16 rows per CTA): 8 warps split K / N
 constexpr int kMmaThreads = kMmaWarps * 32;
@@ -693,15 +326,16 @@ D3P_D void split_a(const float2 v0, const float2 v1, uint32_t (&ah)[4], uint32_t
 struct MidFragDims {
   uint32_t ks23, nt23, ks4, nt4, ks4t, nt4t, ks23t, nt23t;
   __host__ __device__ MidFragDims(uint32_t H, uint32_t Z)
-      : ks23(H / 8), nt23(2 * Z / 8), ks4((Z + 7) / 8), nt4(H / 8), ks4t(H / 8), nt4t((Z + 7) / 8), ks23t(2 * Z / 8),
-        nt23t(H / 8) {}
+      : ks23((H + 7) / 8), nt23((2 * Z + 7) / 8), ks4((Z + 7) / 8), nt4((H + 7) / 8), ks4t((H + 7) / 8),
+        nt4t((Z + 7) / 8), ks23t((2 * Z + 7) / 8), nt23t((H + 7) / 8) {}
   __host__ __device__ size_t n23() const { return (size_t)ks23 * nt23 * 32; }
   __host__ __device__ size_t n4() const { return (size_t)ks4 * nt4 * 32; }
   __host__ __device__ size_t n4t() const { return (size_t)ks4t * nt4t * 32; }
   __host__ __device__ size_t n23t() const { return (size_t)ks23t * nt23t * 32; }
 };
 
-// One thread per float4: entry (ks, nt, lane) of matrix m holds rows k = 8 ks + 2t, k + 1 of column n = 8 nt + g.
+// One thread per float4: entry (ks, nt, lane) of matrix m holds rows k = 8 ks + 2t, k + 1 of column n = 8 nt + g;
+// zero outside the K x N matrix.
 __global__ void vae_prep_mid_kernel(VaeArgs a) {
   const uint32_t H = a.H, Z = a.Z;
   const MidFragDims fd(H, Z);
@@ -710,11 +344,11 @@ __global__ void vae_prep_mid_kernel(VaeArgs a) {
   const float* __restrict__ W3 = a.params + a.off_w3;
   const float* __restrict__ W4 = a.params + a.off_w4;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n3; i += (size_t)gridDim.x * blockDim.x) {
-    int m; size_t loc; uint32_t nt_count;
-    if (i < n0) { m = 0; loc = i; nt_count = fd.nt23; }
-    else if (i < n1) { m = 1; loc = i - n0; nt_count = fd.nt4; }
-    else if (i < n2) { m = 2; loc = i - n1; nt_count = fd.nt4t; }
-    else { m = 3; loc = i - n2; nt_count = fd.nt23t; }
+    int m; size_t loc; uint32_t nt_count, K, N;
+    if (i < n0) { m = 0; loc = i; nt_count = fd.nt23; K = H; N = 2 * Z; }
+    else if (i < n1) { m = 1; loc = i - n0; nt_count = fd.nt4; K = Z; N = H; }
+    else if (i < n2) { m = 2; loc = i - n1; nt_count = fd.nt4t; K = H; N = Z; }
+    else { m = 3; loc = i - n2; nt_count = fd.nt23t; K = 2 * Z; N = H; }
     const uint32_t lane = (uint32_t)(loc & 31), blk = (uint32_t)(loc >> 5);
     const uint32_t ks = blk / nt_count, nt = blk - ks * nt_count;
     const uint32_t k = 8 * ks + 2 * (lane & 3), n = 8 * nt + (lane >> 2);
@@ -722,11 +356,13 @@ __global__ void vae_prep_mid_kernel(VaeArgs a) {
 #pragma unroll
     for (int q = 0; q < 2; ++q) {
       const uint32_t kk = k + q;
-      float x;
-      if (m == 0) x = n < Z ? W2[(size_t)kk * Z + n] : W3[(size_t)kk * Z + n - Z];            // [h][j]
-      else if (m == 1) x = kk < Z ? W4[(size_t)kk * H + n] : 0.f;                                // [j][h]
-      else if (m == 2) x = n < Z ? W4[(size_t)n * H + kk] : 0.f;                                 // [h][j] = W4[j][h]
-      else x = kk < Z ? W2[(size_t)n * Z + kk] : W3[(size_t)n * Z + kk - Z];                     // [j'][h]
+      float x = 0.f;
+      if (kk < K && n < N) {
+        if (m == 0) x = n < Z ? W2[(size_t)kk * Z + n] : W3[(size_t)kk * Z + n - Z];          // [h][j]
+        else if (m == 1) x = W4[(size_t)kk * H + n];                                            // [j][h]
+        else if (m == 2) x = W4[(size_t)n * H + kk];                                            // [h][j] = W4[j][h]
+        else x = kk < Z ? W2[(size_t)n * Z + kk] : W3[(size_t)n * Z + kk - Z];                   // [j'][h]
+      }
       v[q] = x;
     }
     const float h0 = tc::tf32_hi(v[0]), h1 = tc::tf32_hi(v[1]);
@@ -780,9 +416,12 @@ __global__ void __launch_bounds__(kMmaThreads) vae_mid_fwd_mma_kernel(VaeArgs a)
     const float* pl1 = a.h1_lo + (size_t)rg8 * a.ldh;
 #pragma unroll 4
     for (uint32_t ks = warp; ks < fd.ks23; ks += kMmaWarps) {
-      uint32_t ah[4], al[4];
-      load_a_pair(ph0, ph1, 8 * ks + 2 * t, ah);
-      load_a_pair(pl0, pl1, 8 * ks + 2 * t, al);
+      uint32_t ah[4] = {0u, 0u, 0u, 0u}, al[4] = {0u, 0u, 0u, 0u};
+      const uint32_t k = 8 * ks + 2 * t;
+      if (k < H) {                    // columns H.. hold the ones column of [H1 | 1], written only in phase 2
+        load_a_pair(ph0, ph1, k, ah);
+        load_a_pair(pl0, pl1, k, al);
+      }
       const float4* bf = a.wf23 + (size_t)ks * fd.nt23 * 32 + lane;
 #pragma unroll
       for (int nt = 0; nt < 8; ++nt)
@@ -852,19 +491,15 @@ __global__ void __launch_bounds__(kMmaThreads) vae_mid_fwd_mma_kernel(VaeArgs a)
       for (int ks = 0; ks < 4; ++ks)
         if ((uint32_t)ks < fd.ks4) mma3(acc, zh[ks], zl[ks], __ldg(a.wf4 + ((size_t)ks * fd.nt4 + nt) * 32 + lane));
       const uint32_t n = 8 * nt + 2 * t;
-      const float2 b = make_float2(a.params[a.off_b4 + n], a.params[a.off_b4 + n + 1]);
-      const float v00 = softplus_f(acc[0] + b.x), v01 = softplus_f(acc[1] + b.y);
-      const float v10 = softplus_f(acc[2] + b.x), v11 = softplus_f(acc[3] + b.y);
-      sq0 = fmaf(v00, v00, fmaf(v01, v01, sq0));
-      sq1 = fmaf(v10, v10, fmaf(v11, v11, sq1));
-      const float h00 = tc::tf32_hi(v00), h01 = tc::tf32_hi(v01), h10 = tc::tf32_hi(v10), h11 = tc::tf32_hi(v11);
-      if (live0) {
-        *reinterpret_cast<float2*>(a.h2_hi + (size_t)(r0 + g) * H + n) = make_float2(v00, v01);     // unmasked
-        *reinterpret_cast<float2*>(a.h2_lo + (size_t)(r0 + g) * H + n) = make_float2(v00 - h00, v01 - h01);
-      }
-      if (live1) {
-        *reinterpret_cast<float2*>(a.h2_hi + (size_t)(r0 + g + 8) * H + n) = make_float2(v10, v11);
-        *reinterpret_cast<float2*>(a.h2_lo + (size_t)(r0 + g + 8) * H + n) = make_float2(v10 - h10, v11 - h11);
+      if (n < H) {
+        const float2 b = make_float2(a.params[a.off_b4 + n], a.params[a.off_b4 + n + 1]);
+        const float v00 = softplus_f(acc[0] + b.x), v01 = softplus_f(acc[1] + b.y);
+        const float v10 = softplus_f(acc[2] + b.x), v11 = softplus_f(acc[3] + b.y);
+        sq0 = fmaf(v00, v00, fmaf(v01, v01, sq0));
+        sq1 = fmaf(v10, v10, fmaf(v11, v11, sq1));
+        // unmasked and unsplit: the G5 GEMM splits its operand itself (GemmOperand::split)
+        if (live0) *reinterpret_cast<float2*>(a.h2_hi + (size_t)(r0 + g) * H + n) = make_float2(v00, v01);
+        if (live1) *reinterpret_cast<float2*>(a.h2_hi + (size_t)(r0 + g + 8) * H + n) = make_float2(v10, v11);
       }
     }
     sq0 += __shfl_xor_sync(0xffffffffu, sq0, 1); sq0 += __shfl_xor_sync(0xffffffffu, sq0, 2);
@@ -903,7 +538,9 @@ __global__ void __launch_bounds__(kMmaThreads) vae_mid_bwd_mma_kernel(VaeArgs a)
     for (uint32_t ks = warp; ks < fd.ks4t; ks += kMmaWarps) {
       uint32_t ah[4], al[4];
       const uint32_t k = 8 * ks + 2 * t;
-      split_a(*reinterpret_cast<const float2*>(p0 + k), *reinterpret_cast<const float2*>(p1 + k), ah, al);
+      const float2 zero = make_float2(0.f, 0.f);       // d4 rows are H wide: columns H.. are the next row or buffer
+      split_a(k < H ? *reinterpret_cast<const float2*>(p0 + k) : zero,
+              k < H ? *reinterpret_cast<const float2*>(p1 + k) : zero, ah, al);
       const float4* bf = a.wf4t + (size_t)ks * fd.nt4t * 32 + lane;
 #pragma unroll
       for (int nt = 0; nt < 4; ++nt)
@@ -936,6 +573,7 @@ __global__ void __launch_bounds__(kMmaThreads) vae_mid_bwd_mma_kernel(VaeArgs a)
       s_dh[0][e8][Z + j] = h3; s_dh[1][e8][Z + j] = d3 - h3;
       sq23 = fmaf(dz, dz, fmaf(d3, d3, sq23));
     }
+    for (uint32_t j = Z2 + j8; j < 8 * fd.ks23t; j += kMmaTpe) { s_dh[0][e8][j] = 0.f; s_dh[1][e8][j] = 0.f; }  // k padding
 #pragma unroll
     for (int o = 1; o < kMmaTpe; o <<= 1) sq23 += __shfl_xor_sync(0xffffffffu, sq23, o);
     if (j8 == 0) s_sq23[e8] = sq23;
@@ -961,14 +599,16 @@ __global__ void __launch_bounds__(kMmaThreads) vae_mid_bwd_mma_kernel(VaeArgs a)
         load_a_pair(&s_dh[1][g][0], &s_dh[1][g + 8][0], 8 * ks + 2 * t, al);
         mma3(acc, ah, al, __ldg(a.wf23t + ((size_t)ks * fd.nt23t + nt) * 32 + lane));
       }
-      const float d00 = live0 ? acc[0] * (-expm1f(-(hh0.x + hl0.x))) : 0.f;
-      const float d01 = live0 ? acc[1] * (-expm1f(-(hh0.y + hl0.y))) : 0.f;
-      const float d10 = live1 ? acc[2] * (-expm1f(-(hh1.x + hl1.x))) : 0.f;
-      const float d11 = live1 ? acc[3] * (-expm1f(-(hh1.y + hl1.y))) : 0.f;
-      sq0 = fmaf(d00, d00, fmaf(d01, d01, sq0));
-      sq1 = fmaf(d10, d10, fmaf(d11, d11, sq1));
-      *reinterpret_cast<float2*>(s_d1 + (size_t)g * H + n) = make_float2(d00, d01);
-      *reinterpret_cast<float2*>(s_d1 + (size_t)(g + 8) * H + n) = make_float2(d10, d11);
+      if (n < H) {                    // (h1 rows are H + 4 wide: the loads above stay inside the row)
+        const float d00 = live0 ? acc[0] * (-expm1f(-(hh0.x + hl0.x))) : 0.f;
+        const float d01 = live0 ? acc[1] * (-expm1f(-(hh0.y + hl0.y))) : 0.f;
+        const float d10 = live1 ? acc[2] * (-expm1f(-(hh1.x + hl1.x))) : 0.f;
+        const float d11 = live1 ? acc[3] * (-expm1f(-(hh1.y + hl1.y))) : 0.f;
+        sq0 = fmaf(d00, d00, fmaf(d01, d01, sq0));
+        sq1 = fmaf(d10, d10, fmaf(d11, d11, sq1));
+        *reinterpret_cast<float2*>(s_d1 + (size_t)g * H + n) = make_float2(d00, d01);
+        *reinterpret_cast<float2*>(s_d1 + (size_t)(g + 8) * H + n) = make_float2(d10, d11);
+      }
     }
     sq0 += __shfl_xor_sync(0xffffffffu, sq0, 1); sq0 += __shfl_xor_sync(0xffffffffu, sq0, 2);
     sq1 += __shfl_xor_sync(0xffffffffu, sq1, 1); sq1 += __shfl_xor_sync(0xffffffffu, sq1, 2);
@@ -1042,8 +682,7 @@ __global__ void __launch_bounds__(kMmaThreads) vae_mid_bwd_mma_kernel(VaeArgs a)
       const float cc = s_cc[e8];
       if (j8 < 4) {
         const float v = j8 == 0 ? cc : 0.f;
-        a.ch2_hi[(size_t)r * a.ldh + H + j8] = v;          // unmasked; the dW5 GEMM never reads ch2_lo
-
+        a.ch2_hi[(size_t)r * a.ldh + H + j8] = v;          // unmasked and unsplit, as above
       }
       for (uint32_t j = j8; j < a.ld23; j += kMmaTpe) {
         const float v = j < Z2 ? cc * s_d23[e8][j] : 0.f;
@@ -1101,9 +740,9 @@ constexpr int kThinBN = 64;            // N tile of the two thin clipped-sum GEM
 
 struct VaeLayout {
   size_t total;
-  size_t partials, w1_hi, w1_lo, w5_hi, w5_lo, x_hi, x_lo, flag, h1_hi, h1_lo, h2_hi, h2_lo, ch2_hi, ch2_lo, d5_hi, d5_lo,
-      d4, cd4_hi, cd4_lo, cd1_hi, cd1_lo, z_hi, z_lo, u, cd23_hi, cd23_lo, sq_x, sq_h1, sq_h2, sq_z, sq_d5, loss_rec, sq_d4,
-      loss_kl, lossv, cnt, wf23, wf4, wf4t, wf23t;
+  size_t partials, w1_hi, w1_lo, w5_hi, w5_lo, x_hi, x_lo, flag, h1_hi, h1_lo, h2_hi, ch2_hi, d5_hi, d5_lo, d4, cd4_hi,
+      cd4_lo, cd1_hi, z_hi, z_lo, u, cd23_hi, cd23_lo, sq_x, sq_h1, sq_h2, sq_z, sq_d5, loss_rec, sq_d4, loss_kl, lossv, cnt,
+      wf23, wf4, wf4t, wf23t;
   uint32_t S, ns_h, ns_d;
   size_t ldx, ldh, ldz, ld23;
 };
@@ -1137,11 +776,10 @@ static VaeLayout vae_layout(const d3p_vae_desc* d, uint32_t Bl) {
   L.w1_hi = take(D * H); L.w1_lo = take(D * H); L.w5_hi = take(H * D); L.w5_lo = take(H * D);
   L.x_hi = take((size_t)Bl * L.ldx); L.x_lo = take((size_t)Bl * L.ldx); L.flag = take(4);
   L.h1_hi = take((size_t)Bl * L.ldh); L.h1_lo = take((size_t)Bl * L.ldh);
-  L.h2_hi = take((size_t)Bl * H); L.h2_lo = take((size_t)Bl * H);
-  L.ch2_hi = take((size_t)Bl * L.ldh); L.ch2_lo = take((size_t)Bl * L.ldh);
+  L.h2_hi = take((size_t)Bl * H); L.ch2_hi = take((size_t)Bl * L.ldh);
   L.d5_hi = take((size_t)Bl * D); L.d5_lo = take((size_t)Bl * D);
   L.d4 = take((size_t)Bl * H); L.cd4_hi = take((size_t)Bl * H); L.cd4_lo = take((size_t)Bl * H);
-  L.cd1_hi = take((size_t)Bl * H); L.cd1_lo = take((size_t)Bl * H);
+  L.cd1_hi = take((size_t)Bl * H);
   L.z_hi = take((size_t)Bl * L.ldz); L.z_lo = take((size_t)Bl * L.ldz); L.u = take((size_t)Bl * Z);
   L.cd23_hi = take((size_t)Bl * L.ld23); L.cd23_lo = take((size_t)Bl * L.ld23);
   L.sq_x = take(Bl); L.sq_h1 = take((size_t)L.ns_h * Bl); L.sq_h2 = take(Bl); L.sq_z = take(Bl);
@@ -1155,12 +793,8 @@ static VaeLayout vae_layout(const d3p_vae_desc* d, uint32_t Bl) {
   return L;
 }
 
-static size_t mid_fwd_smem_bytes(uint32_t H, uint32_t Z) {
-  return ((size_t)H * 2 * Z + (size_t)Z * H + 64 + H + (size_t)kMidWarps * kMidE * (H + 3 * 64)) * sizeof(float);
-}
-static size_t mid_bwd_smem_bytes(uint32_t H, uint32_t Z) {
-  return (3 * (size_t)Z * H + (size_t)kMidWarps * kMidE * (H + 128)) * sizeof(float);
-}
+// Dynamic shared memory of vae_mid_bwd_mma_kernel: raw delta1 of its 16 rows
+static size_t mid_bwd_dyn_smem(uint32_t H) { return (size_t)kMmaRows * H * sizeof(float); }
 
 }  // namespace d3p
 
@@ -1176,10 +810,19 @@ struct d3p_vae_ctx {
 namespace d3p {
 using VaeSideStreams = d3p_vae_ctx;
 
+// H is bounded by the backward thin-layer kernel: its static shared memory and 16 rows of H floats fit one block's
+// opt-in maximum (227 KB on B200: H <= 3156)
 static bool vae_supported(const d3p_vae_desc* d) {
-  return d && d->out_dim >= 4 && d->hidden_dim >= 4 && d->z_dim >= 1 && d->z_dim <= 32 && (d->out_dim % 4) == 0 &&
-         (d->hidden_dim % 4) == 0 && mid_fwd_smem_bytes(d->hidden_dim, d->z_dim) <= 220 * 1024 &&
-         mid_bwd_smem_bytes(d->hidden_dim, d->z_dim) <= 220 * 1024;
+  if (!d || d->out_dim < 4 || d->hidden_dim < 4 || d->z_dim < 1 || d->z_dim > 32 || (d->out_dim % 4) != 0 ||
+      (d->hidden_dim % 4) != 0)
+    return false;
+  int dev = 0, optin = 0;
+  cudaFuncAttributes fa;
+  if (cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+      cudaFuncGetAttributes(&fa, vae_mid_bwd_mma_kernel) != cudaSuccess)
+    return false;
+  return fa.sharedSizeBytes + mid_bwd_dyn_smem(d->hidden_dim) <= (size_t)optin;
 }
 
 }  // namespace d3p
@@ -1255,9 +898,9 @@ int32_t d3p::step_vae_impl(const d3p_vae_desc* desc, const float* params_d, cons
   a.site_scale = desc->site_scale; a.inv_S = 1.0f / obs_scale; a.C = C;
   a.ns_h = L.ns_h; a.ns_d = L.ns_d; a.S = L.S;
   a.x_hi = F(L.x_hi); a.x_lo = F(L.x_lo); a.x_lo_flag = reinterpret_cast<int*>(ws + L.flag);
-  a.h1_hi = F(L.h1_hi); a.h1_lo = F(L.h1_lo); a.h2_hi = F(L.h2_hi); a.h2_lo = F(L.h2_lo);
-  a.ch2_hi = F(L.ch2_hi); a.ch2_lo = F(L.ch2_lo); a.d5_hi = F(L.d5_hi); a.d5_lo = F(L.d5_lo);
-  a.d4 = F(L.d4); a.cd4_hi = F(L.cd4_hi); a.cd4_lo = F(L.cd4_lo); a.cd1_hi = F(L.cd1_hi); a.cd1_lo = F(L.cd1_lo);
+  a.h1_hi = F(L.h1_hi); a.h1_lo = F(L.h1_lo); a.h2_hi = F(L.h2_hi); a.ch2_hi = F(L.ch2_hi);
+  a.d5_hi = F(L.d5_hi); a.d5_lo = F(L.d5_lo); a.d4 = F(L.d4); a.cd4_hi = F(L.cd4_hi); a.cd4_lo = F(L.cd4_lo);
+  a.cd1_hi = F(L.cd1_hi);
   a.z_hi = F(L.z_hi); a.z_lo = F(L.z_lo); a.u = F(L.u); a.cd23_hi = F(L.cd23_hi); a.cd23_lo = F(L.cd23_lo);
   a.sq_x = F(L.sq_x); a.sq_h1 = F(L.sq_h1); a.sq_h2 = F(L.sq_h2); a.sq_z = F(L.sq_z); a.sq_d5 = F(L.sq_d5);
   a.loss_rec = F(L.loss_rec); a.sq_d4 = F(L.sq_d4); a.loss_kl = F(L.loss_kl); a.lossv = F(L.lossv); a.cnt = F(L.cnt);
@@ -1265,8 +908,6 @@ int32_t d3p::step_vae_impl(const d3p_vae_desc* desc, const float* params_d, cons
   a.px_norms = px_norms_d; a.px_loss = px_loss_d;
   a.wf23 = reinterpret_cast<float4*>(ws + L.wf23); a.wf4 = reinterpret_cast<float4*>(ws + L.wf4);
   a.wf4t = reinterpret_cast<float4*>(ws + L.wf4t); a.wf23t = reinterpret_cast<float4*>(ws + L.wf23t);
-  // thin layers: warp-MMA kernels for the shapes they tile (H % 8 == 0, Z % 4 == 0), SIMT kernels otherwise
-  const bool mid_mma = (H % 8) == 0 && (Z % 4) == 0 && Z <= 32;
   float* w1_hi = F(L.w1_hi); float* w1_lo = F(L.w1_lo); float* w5_hi = F(L.w5_hi); float* w5_lo = F(L.w5_lo);
 
   const int sms = sm_count();
@@ -1286,7 +927,7 @@ int32_t d3p::step_vae_impl(const d3p_vae_desc* desc, const float* params_d, cons
     }
     if ((rc = d3p_split_tf32(params_d + a.off_w1, nullptr, 0, w1_hi, w1_lo, (size_t)D * H, sw)) != D3P_OK) return rc;
     if ((rc = d3p_split_tf32(params_d + a.off_w5, nullptr, 0, w5_hi, w5_lo, (size_t)H * D, sw)) != D3P_OK) return rc;
-    if (mid_mma) {
+    {
       const MidFragDims fd(H, Z);
       const size_t n = fd.n23() + fd.n4() + fd.n4t() + fd.n23t();
       vae_prep_mid_kernel<<<(unsigned)((n + 255) / 256), 256, 0, sm>>>(a);
@@ -1310,19 +951,9 @@ int32_t d3p::step_vae_impl(const d3p_vae_desc* desc, const float* params_d, cons
     if ((rc = tc::launch_tc_gemm<false, true, kVaeBNH, EpiFwd1, kHeavyEW>(A, Bo, Bl, H, D, 1, ea, s, a.x_lo_flag)) != D3P_OK)
       return rc;
   }
-  const size_t mid_fwd_smem = mid_fwd_smem_bytes(H, Z), mid_bwd_smem = mid_bwd_smem_bytes(H, Z);
-  unsigned mid_grid = ((Bl + kMidE - 1) / kMidE + kMidWarps - 1) / kMidWarps;
-  if (mid_grid > (unsigned)sms) mid_grid = sms;
   const unsigned mma_grid = (Bl + kMmaRows - 1) / kMmaRows;
-  if (mid_mma) {
-    vae_mid_fwd_mma_kernel<<<mma_grid, kMmaThreads, 0, s>>>(a);
-    if ((rc = check_launch()) != D3P_OK) return rc;
-  } else {
-    if (cudaFuncSetAttribute(vae_mid_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mid_fwd_smem) != cudaSuccess)
-      return D3P_ERR_CUDA;
-    vae_mid_fwd_kernel<<<mid_grid, kMidWarps * 32, mid_fwd_smem, s>>>(a);
-    if ((rc = check_launch()) != D3P_OK) return rc;
-  }
+  vae_mid_fwd_mma_kernel<<<mma_grid, kMmaThreads, 0, s>>>(a);
+  if ((rc = check_launch()) != D3P_OK) return rc;
   // G5: logits = H2 W5  (B = W5 stored [K = H, N = D])
   {
     tc::GemmOperand A{a.h2_hi, nullptr, 0, H, 1}, Bo{params_d + a.off_w5, nullptr, 1, D, 1};   // both split in the kernel
@@ -1337,21 +968,16 @@ int32_t d3p::step_vae_impl(const d3p_vae_desc* desc, const float* params_d, cons
   // G5b: dh2 = delta5 W5^T  (B[n = h, k = d] = W5[h, d]: K-major)
   {
     tc::GemmOperand A{a.d5_hi, a.d5_lo, 0, D}, Bo{w5_hi, w5_lo, 0, D};     // pre-split: the in-kernel split measured slower here
-    EpiBwd5::Args ea{a.h2_hi, a.h2_lo, H, a.d4, a.sq_d4, Bl};
+    EpiBwd5::Args ea{a.h2_hi, H, a.d4, a.sq_d4, Bl};
     if ((rc = tc::launch_tc_gemm<false, false, kVaeBNH, EpiBwd5, kHeavyEW>(A, Bo, Bl, H, D, 1, ea, s, nullptr)) != D3P_OK)
       return rc;
   }
-  if (mid_mma) {
-    const size_t smem = (size_t)kMmaRows * H * sizeof(float);
-    if (smem > 24 * 1024 &&
-        cudaFuncSetAttribute(vae_mid_bwd_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+  {
+    // static + dynamic shared memory over 48 KB needs the opt-in: set it on every step rather than track the static part
+    const size_t smem = mid_bwd_dyn_smem(H);
+    if (cudaFuncSetAttribute(vae_mid_bwd_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
       return D3P_ERR_CUDA;
     vae_mid_bwd_mma_kernel<<<mma_grid, kMmaThreads, smem, s>>>(a);
-    if ((rc = check_launch()) != D3P_OK) return rc;
-  } else {
-    if (cudaFuncSetAttribute(vae_mid_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mid_bwd_smem) != cudaSuccess)
-      return D3P_ERR_CUDA;
-    vae_mid_bwd_kernel<<<mid_grid, kMidWarps * 32, mid_bwd_smem, s>>>(a);
     if ((rc = check_launch()) != D3P_OK) return rc;
   }
   // The four clipped-sum GEMMs are independent: GW1 stays on the caller's stream, GW5 / GW23 / GW4 run on side streams

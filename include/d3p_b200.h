@@ -477,7 +477,7 @@ int32_t d3p_gemm_f32x3(const float* a_d, int32_t a_mn_major, size_t lda, const f
  * W4 [Z,H], b4 [H], W5 [H,D], b5 [D], W1 [D,H], b1 [H], W2 [H,Z], b2 [Z], W3 [H,Z], b3 [Z].
  * ------------------------------------------------------------------------------------------ */
 typedef struct {
-  uint32_t out_dim, hidden_dim, z_dim; /* D, H (multiples of 4), Z <= 32 */
+  uint32_t out_dim, hidden_dim, z_dim; /* D, H (multiples of 4; H <= 3156 on B200), 1 <= Z <= 32 */
   uint32_t n_params;
   uint32_t off_w4, off_b4, off_w5, off_b5, off_w1, off_b1, off_w2, off_b2, off_w3, off_b3;
   float site_scale; /* plate scale N / 1 times the scale handler's 1 / N (examples/vae.py:193-194) */

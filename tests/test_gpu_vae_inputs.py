@@ -59,8 +59,8 @@ def batch_mask(B):
 def setup(D, H, Z, X, C, N=60000, seed=0, init_std=None, params=None):
     """Oracle and CUDA DPSVI with SGD(1) and dp_scale = 0 on the same float32 parameters (test_gpu_vae.make's
     initialisation unless ``params`` is given)."""
-    if init_std is None:
-        init_std = 0.1 if D <= 64 else 0.03
+    if init_std is None:                     # as test_gpu_vae.make
+        init_std = 0.1 if D <= 64 and H <= 400 else 0.03
     ofam = ovae.VAE(D, H, Z, N)
     p0 = ofam.init_params(seed, init_std) if params is None else params
     o = osvi.DPSVI(ofam, None, osvi.SGD(1.0), None, C, 0.0)
@@ -150,10 +150,10 @@ def check_step(tag, o, ost, s, st, X, Xd, mask, check_update=True):
 
 
 # ---- 1. real-valued X -----------------------------------------------------------------------------------------------
-# (D, H, Z, B, kind, layout): (36, 20, 3) runs the SIMT thin-layer kernels, the others the warp-MMA ones; D + 1 = 129 /
-# 257 leaves GW1's last 128-row M tile with the bias row alone; B is never a multiple of 16 (the warp-MMA CTA) or of
-# 32 (the GEMM k-block).  Layout "c": aligned contiguous rows (vae_prep_x_kernel<true>); "b": a column slice
-# 4 bytes past a 16-byte boundary with an odd row stride (vae_prep_x_kernel<false>).
+# (D, H, Z, B, kind, layout): the thin-layer shapes of tests/test_gpu_vae.py, padded (H % 8 == 4, 2Z % 8 != 0, Z = 32)
+# and not; D + 1 = 129 / 257 leaves GW1's last 128-row M tile with the bias row alone; B is never a multiple of 16 (the
+# warp-MMA CTA) or of 32 (the GEMM k-block).  Layout "c": aligned contiguous rows (vae_prep_x_kernel<true>); "b": a
+# column slice 4 bytes past a 16-byte boundary with an odd row stride (vae_prep_x_kernel<false>).
 REAL_CASES = [
     (36, 20, 3, 19, "k255", "c"), (36, 20, 3, 45, "uniform", "b"),
     (36, 24, 4, 21, "uniform", "c"), (36, 24, 4, 19, "k255", "b"),
@@ -161,6 +161,8 @@ REAL_CASES = [
     (128, 40, 8, 45, "k255", "c"), (128, 40, 8, 61, "uniform", "b"),
     (256, 64, 8, 77, "uniform", "c"), (256, 64, 8, 33, "k255", "b"),
     (784, 400, 20, 300, "k255", "c"), (784, 400, 20, 300, "uniform", "b"),
+    (36, 20, 4, 21, "uniform", "c"), (36, 24, 3, 19, "k255", "b"), (36, 20, 1, 23, "k255", "c"),
+    (64, 44, 30, 37, "uniform", "b"), (64, 44, 32, 29, "k255", "c"), (64, 416, 32, 45, "uniform", "b"),
 ]
 
 
